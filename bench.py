@@ -2,6 +2,7 @@
 """Benchmark of the log-mel hot path (BASELINE.json metric: log-mel audio-seconds/second).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c3|c4] [--no-extras]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic PCM.  The headline workload is
 BASELINE.json configs[1] (C2: whisper-small 80-mel, batch 256 x 30 s, device-resident PCM, one
@@ -18,6 +19,11 @@ in the same run with the same rules:
     cpu_baseline / cpu_baseline_numpy   the reference's CPU paths on this box's host cores (N = 1)
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for how every field is derived.
+
+--dump-outputs DIR writes what the headline workload's last timed step computed, as the caller of the device path
+receives it: DIR/input_features.npy, float32 [K, n_mels, 3000], the features of K clips of rank 0's batch drawn with
+numpy's default_rng(0) (every clip while the batch fits in 60 MB, else as many as fit).  The PCM is generated from fixed
+seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -32,10 +38,12 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from
 
 N_SAMPLES = 480000
 N_FRAMES = 3000
 CLIP_SECONDS = 30.0
+DUMP_BYTES = 60_000_000
 
 WORKLOADS = {
     "c2": dict(n_mels=80, batch=256, strong=False, profile="c2_80mel",
@@ -369,9 +377,18 @@ def make_workload(cx: Ctx, wl):
     return w
 
 
-def measure(cx: Ctx, w, steps, warmup, e2e=True, e2e_extra=False):
+def dump_sample(B, n_mels):
+    """Sorted clip indices of the --dump-outputs sample: all B clips, or a seeded draw of as many as fit in DUMP_BYTES."""
+    import numpy as np
+
+    k = min(B, DUMP_BYTES // (n_mels * N_FRAMES * 4))
+    return np.sort(np.random.default_rng(0).choice(B, size=k, replace=False))
+
+
+def measure(cx: Ctx, w, steps, warmup, e2e=True, e2e_extra=False, sample=None):
     """Device-resident and end-to-end timing of one workload on this rank; returns the fields of its JSON object
-    (max over ranks applied)."""
+    (max over ranks applied).  With `sample` (clip indices), res["_outputs"] holds those clips' features from the last
+    timed step."""
     torch = cx.torch
     fe = cx.fe(w["n_mels"])
     B, n_mels, out = w["B"], w["n_mels"], w["out"]
@@ -398,8 +415,11 @@ def measure(cx: Ctx, w, steps, warmup, e2e=True, e2e_extra=False):
     dev_ms = t0.elapsed_time(t1)
     launch_ms = dev_ms / steps        # back-to-back launches between two events on the launch stream: the average step
 
-    # ---- end to end: pinned host PCM -> H2D -> kernels -> D2H of one float per clip --------------
     res = {}
+    if sample is not None:          # copied now: the end-to-end legs below write into `out` again
+        res["_outputs"] = {"input_features": out[torch.from_numpy(sample).to(cx.dev)].cpu().numpy()}
+
+    # ---- end to end: pinned host PCM -> H2D -> kernels -> D2H of one float per clip --------------
     e2e_steps = max(2, min(steps, 5))
     gmax_host = torch.empty((max(B, 1),), dtype=torch.float32).pin_memory()
     clips = w["clips"]
@@ -700,7 +720,15 @@ def run_ours(args, wl_name, rank, world, local_rank):
     cx = Ctx(rank, world, local_rank)
     wl = WORKLOADS[wl_name]
     w = make_workload(cx, wl)
-    res = measure(cx, w, args.steps, args.warmup, e2e=not args.no_e2e, e2e_extra=not args.no_e2e and not wl.get("variable"))
+    sample = dump_sample(w["B"], wl["n_mels"]) if args.dump_outputs and rank == 0 else None
+    res = measure(cx, w, args.steps, args.warmup, e2e=not args.no_e2e, e2e_extra=not args.no_e2e and not wl.get("variable"),
+                  sample=sample)
+    if sample is not None:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in res.pop("_outputs").items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     line = {
         "metric": "log-mel audio-seconds/second", "value": res["value"], "unit": "audio-s/s",
         "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
@@ -779,7 +807,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host end-to-end legs (profiling runs)")
     ap.add_argument("--no-extras", action="store_true", help="only the headline workload (no c3/c4/c1/sustained/hf_cuda objects)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the features of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

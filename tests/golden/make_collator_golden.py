@@ -2,7 +2,7 @@
 `DataCollatorSpeechSeq2SeqWithPadding` (REF/data_utils/data_collator.py:27-127), imported here through
 an offline shim (its module body calls `from_pretrained`, which needs the network).
 
-Build container only:   python tests/golden/make_collator_golden.py
+Usage:                  python tests/golden/make_collator_golden.py REFERENCE_CHECKOUT
 Output:                 tests/golden/collator_golden.npz
 """
 import importlib.util
@@ -14,7 +14,6 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-REF = "/root/reference"
 
 
 def _bytes_to_unicode():
@@ -43,22 +42,22 @@ def synthetic_tokenizer():
     return tok
 
 
-def import_reference_collator(tok):
+def import_reference_collator(ref, tok):
     from transformers import WhisperFeatureExtractor, WhisperTokenizer
 
     WhisperFeatureExtractor.from_pretrained = classmethod(lambda cls, *a, **k: cls())
     WhisperTokenizer.from_pretrained = classmethod(lambda cls, *a, **k: tok)
-    spec = importlib.util.spec_from_file_location("ref_data_collator", os.path.join(REF, "data_utils", "data_collator.py"))
+    spec = importlib.util.spec_from_file_location("ref_data_collator", os.path.join(ref, "data_utils", "data_collator.py"))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     return mod
 
 
-def main():
+def main(ref):
     from transformers import WhisperFeatureExtractor, WhisperProcessor
 
     tok = synthetic_tokenizer()
-    mod = import_reference_collator(tok)
+    mod = import_reference_collator(ref, tok)
     proc = WhisperProcessor(WhisperFeatureExtractor(), tok)
     sot = tok.convert_tokens_to_ids("<|startoftranscript|>")
     prev = tok.convert_tokens_to_ids("<|startofprev|>")
@@ -96,4 +95,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

@@ -7,7 +7,7 @@ Rows 0..11 of REF/data/medical-united-syn-med-test-jsonl/test.jsonl, all four pr
 (no random perturbation).  Stored: labels and bias_spans of every item, the sha256 of the PCM the reference extractor was
 given, and a frame-subsampled copy of the features the reference item carried.
 
-Build container only:   python tests/golden/make_dataset_golden.py
+Usage:                  python tests/golden/make_dataset_golden.py REFERENCE_CHECKOUT
 Output:                 tests/golden/dataset_golden.npz  (+ dataset_golden_rows.jsonl, the 12 metadata rows)
 """
 import hashlib
@@ -22,7 +22,6 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 STRATEGIES = {"desc": dict(prompt=True, bias_list=False), "bias": dict(prompt=False, bias_list=True, bias_nums=4),
               "desc_bias": dict(prompt=True, bias_list=True, bias_nums=4), "none": dict(prompt=False, bias_list=False)}
 
@@ -36,7 +35,7 @@ def synth_audio_for(path, sr=16000):
     return O.synth_clip("speech", n, seed % 100000), sr
 
 
-def import_reference_dataset():
+def import_reference_dataset(ref):
     """The reference module with stubs for the imports that are missing offline (SURVEY 8c)."""
     import importlib.machinery
 
@@ -50,7 +49,7 @@ def import_reference_dataset():
             stubs[name] = sys.modules[name] = m
     sys.modules["librosa"].load = lambda path, sr=16000: synth_audio_for(path, sr)
     try:
-        spec = importlib.util.spec_from_file_location("ref_data_loader", os.path.join(REF, "data_utils", "data_loader.py"))
+        spec = importlib.util.spec_from_file_location("ref_data_loader", os.path.join(ref, "data_utils", "data_loader.py"))
         mod = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(mod)
     finally:
@@ -59,7 +58,7 @@ def import_reference_dataset():
     return mod
 
 
-def main():
+def main(ref):
     import random
 
     import torch
@@ -67,9 +66,9 @@ def main():
     from transformers import WhisperFeatureExtractor
 
     tok = synthetic_tokenizer()
-    mod = import_reference_dataset()
+    mod = import_reference_dataset(ref)
     gold_dir = os.path.join(ROOT, "tests", "golden")
-    rows = [json.loads(l) for l in open(os.path.join(REF, "data", "medical-united-syn-med-test-jsonl", "test.jsonl"))][:12]
+    rows = [json.loads(l) for l in open(os.path.join(ref, "data", "medical-united-syn-med-test-jsonl", "test.jsonl"))][:12]
     with open(os.path.join(gold_dir, "dataset_golden_rows.jsonl"), "w") as f:
         for r in rows:
             f.write(json.dumps(r) + "\n")
@@ -105,4 +104,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

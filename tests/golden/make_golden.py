@@ -11,6 +11,10 @@ reference pins 4.51.3), invoked exactly like REF/data_utils/data_loader.py:171 -
 call, `.input_features[0]` -- for both dispatch paths (torch fp32 default, numpy fp64 fallback).
 Inputs are regenerated from seeds by `oracle.logmel_oracle.synth_clip`; a sha256 of every input
 is stored so generator drift is detected rather than silently compared.
+
+The numpy path's outputs go to `tests/golden/logmel_golden_numpy.npz`, each as its difference from
+the default path's output of the same case (exact in float32, zero for ~98 % of the elements): that
+keeps both files under 1 MB.  `default + difference` gives back the numpy path's output bit for bit.
 """
 from __future__ import annotations
 
@@ -38,7 +42,12 @@ def sha(x: np.ndarray) -> str:
 
 
 def main():
-    store = {}
+    store, numpy_path = {}, {}
+
+    def add_numpy_path(name, out):
+        numpy_path[name] = out - store[name + "_default"]
+        assert np.array_equal(store[name + "_default"] + numpy_path[name], out), name
+
     meta = {"cases": [], "frame_subsample": FRAME_SUBSAMPLE.tolist(),
             "transformers": __import__("transformers").__version__,
             "torch": __import__("torch").__version__, "numpy": np.__version__}
@@ -51,7 +60,7 @@ def main():
             x = synth_clip(fam, SHORT_N, seed)
             name = f"short_{fam}_m{n_mels}"
             store[name + "_default"] = hf_features([x], n_mels, "default")[0]
-            store[name + "_numpy"] = hf_features([x], n_mels, "numpy")[0]
+            add_numpy_path(name, hf_features([x], n_mels, "numpy")[0])
             meta["cases"].append({"name": name, "kind": "short", "family": fam, "seed": seed,
                                   "n": SHORT_N, "n_mels": n_mels, "sha256": sha(x), "full": True})
 
@@ -61,7 +70,7 @@ def main():
         x = synth_clip(fam, 480000, seed)
         name = f"full_{fam}_m{n_mels}"
         store[name + "_default"] = hf_features([x], n_mels, "default")[0][:, FRAME_SUBSAMPLE]
-        store[name + "_numpy"] = hf_features([x], n_mels, "numpy")[0][:, FRAME_SUBSAMPLE]
+        add_numpy_path(name, hf_features([x], n_mels, "numpy")[0][:, FRAME_SUBSAMPLE])
         meta["cases"].append({"name": name, "kind": "full", "family": fam, "seed": seed,
                               "n": 480000, "n_mels": n_mels, "sha256": sha(x), "full": False})
 
@@ -83,6 +92,7 @@ def main():
     store["meta_json"] = np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8)
     out = os.path.join(ROOT, "tests", "golden", "logmel_golden.npz")
     np.savez_compressed(out, **store)
+    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "logmel_golden_numpy.npz"), **numpy_path)
     print(out, os.path.getsize(out) / 1e6, "MB", len(meta["cases"]), "cases")
 
 

@@ -1,11 +1,11 @@
 """PCM-returning dataset (SURVEY 8f rank 1, second half) against a golden produced by the reference's OWN
-`PromptWhisperDataset` (tests/golden/make_dataset_golden.py).  Token ids are integers: exact.  The reference class is
-only importable where /root/reference exists (the build container); elsewhere the test is skipped and the GPU test
-`test_pcm_dataset_items_through_the_device_collator` covers the golden items."""
+`PromptWhisperDataset` (tests/golden/make_dataset_golden.py).  Token ids are integers: exact.  The reference's source is
+not part of this repository, so its class is replaced by a stand-in that makes the same feature-extractor call
+(REF/data_utils/data_loader.py:170-172) and hands back the labels and bias spans the reference item carried; everything
+the wrapper itself produces is compared with the golden."""
 import hashlib
 import json
 import os
-import random
 import sys
 
 import numpy as np
@@ -32,56 +32,60 @@ def test_passthrough_extractor_contract():
         pt(x, sampling_rate=8000)
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/data_utils/data_loader.py"), reason="reference checkout absent")
-def test_pcm_dataset_matches_reference_dataset(tmp_path):
+def test_pcm_dataset_matches_reference_dataset():
     import torch
+
+    pytest.importorskip("transformers")                       # the synthetic tokenizer is a WhisperTokenizer
     from make_collator_golden import synthetic_tokenizer
-    from make_dataset_golden import STRATEGIES, import_reference_dataset, synth_audio_for
+    from make_dataset_golden import STRATEGIES, synth_audio_for
 
     from oracle import logmel_oracle as O
     from whisper_context_biasing_b200 import pcm_dataset_class
 
     z, meta = _golden()
-    mod = import_reference_dataset()
-    loads = []
-    real_load = mod.librosa.load
-    mod.librosa.load = lambda path, sr=16000: (loads.append(path), real_load(path, sr))[1]
+    rows = [json.loads(l) for l in open(os.path.join(GOLD, "dataset_golden_rows.jsonl"))]
     tok = synthetic_tokenizer()
-    (tmp_path / "test.jsonl").write_text(open(os.path.join(GOLD, "dataset_golden_rows.jsonl")).read())
-    from transformers import WhisperFeatureExtractor
+    loads = []
 
-    Pcm = pcm_dataset_class(mod.PromptWhisperDataset)
+    class ReferenceStandIn:
+        """The constructor and `__getitem__` of the reference class as far as the wrapper relies on them: records with
+        the bias words at index 4 (what `bias_spans_only` reads), one audio load and one extractor call per item."""
+
+        def __init__(self, base_path, jsonl_data, phase, feature_extractor, tokenizer, audio_type=".mp3",
+                     gold_items=(), **kwargs):
+            self.base_path, self.phase = base_path, phase
+            self.feature_extractor, self.tokenizer = feature_extractor, tokenizer
+            self.data = [(r["file"], r["text"], r["description"], r["id"], r["bias_words"]) for r in rows]
+            self.gold_items = gold_items
+
+        def __len__(self):
+            return len(self.data)
+
+        def __getitem__(self, i):
+            path = os.path.join(self.base_path, self.phase, self.data[i][0])
+            loads.append(path)
+            audio, sr = synth_audio_for(path)                                        # librosa.load stand-in
+            processed_audio = self.feature_extractor(audio, sampling_rate=sr).input_features      # :171
+            g = self.gold_items[i]
+            return {"input_features": torch.tensor(processed_audio[0]),                            # :172
+                    "labels": torch.tensor(g["labels"]), "bias_spans": g["bias_spans"]}
+
+    Pcm = pcm_dataset_class(ReferenceStandIn)
     sentinel = object()                                        # the device extractor is only carried along
-    hf = WhisperFeatureExtractor()
     for name, kw in STRATEGIES.items():
-        random.seed(0)
-        torch.manual_seed(0)
-        ds = Pcm("/nonexistent", str(tmp_path), "test", sentinel, tok, audio_type=".mp3", **kw)
-        random.seed(0)
-        torch.manual_seed(0)
-        ref_ds = mod.PromptWhisperDataset("/nonexistent", str(tmp_path), "test", hf, tok, audio_type=".mp3", **kw)
-        assert ds.device_feature_extractor is sentinel and len(ds) == meta["n"] == len(ref_ds)
         gold = meta["strategies"][name]["items"]
-        # the bias-list strategies draw from `list(set - set)` (data_loader.py:216,222): their order depends on the
-        # process' string-hash seed, so only the live reference (same process, same seeds) pins them; the golden pins the rest
-        deterministic = not kw.get("bias_list")
+        ds = Pcm("/nonexistent", "rows", "test", sentinel, tok, audio_type=".mp3", gold_items=gold, **kw)
+        assert ds.device_feature_extractor is sentinel and len(ds) == meta["n"]
         n0 = len(loads)
         spans = ds.all_bias_spans()                            # train.py:163 / evaluation.py:147 without the audio
         assert len(loads) == n0
         for i in range(len(ds)):
-            random.seed(100 + i)
-            torch.manual_seed(100 + i)
-            ref_it = ref_ds[i]                                 # the reference's own item (features computed on the CPU)
+            assert spans[i] == gold[i]["bias_spans"], (name, i)   # the restated tokenisation == the reference's spans
             n0 = len(loads)
-            random.seed(100 + i)
-            torch.manual_seed(100 + i)
             it = ds[i]
             assert len(loads) == n0 + 1
             assert set(it) == {"audio", "labels", "bias_spans"}
-            assert torch.equal(torch.as_tensor(it["labels"]), torch.as_tensor(ref_it["labels"])), (name, i)
-            assert it["bias_spans"] == ref_it["bias_spans"] == spans[i]
-            if deterministic:
-                assert [int(x) for x in it["labels"]] == gold[i]["labels"], (name, i)
+            assert [int(x) for x in it["labels"]] == gold[i]["labels"], (name, i)
             assert [[int(t) for t in s] for s in it["bias_spans"]] == gold[i]["bias_spans"]
             a = it["audio"]
             assert a.dtype == np.float32 and a.ndim == 1 and a.shape[0] == gold[i]["n"]
@@ -90,4 +94,3 @@ def test_pcm_dataset_matches_reference_dataset(tmp_path):
                 ref = z[f"{name}_{i}_features_sub"]
                 got = O.extract([a], 80, "f32")[0][:, ::37]
                 assert np.abs(got - ref).max() <= 1e-4
-                assert np.abs(got - ref_it["input_features"].numpy()[:, ::37]).max() <= 1e-4
