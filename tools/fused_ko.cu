@@ -63,10 +63,8 @@ int main(int argc, char** argv) {
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3(fused::kCluster * 148); cfg.blockDim = dim3(fused::kThreads); cfg.dynamicSmemBytes = fused::kSmemBytes;
     at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = fused::kCluster; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-#if WLM_PDL_CHAIN
-    at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[1].val.programmaticStreamSerializationAllowed = 1; cfg.numAttrs = 2;
-#endif
+    at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[1].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at; cfg.numAttrs = 2;
     int maxc = 0;
     CK(cudaOccupancyMaxActiveClusters(&maxc, fn, &cfg));
     ClipArgs a;

@@ -25,15 +25,13 @@
 // Template parameters of the kernel: NMELS (80 / 128: mel stage unrolled with the structure of that Whisper bank; 0: table-
 // driven), FLAT (the cluster-less twin for the SMs clusters cannot cover), OutT (float / bfloat16 / half feature store), DYN
 // (clips from the queue both kernels share -- ragged batches -- or a static split -- dense batches).
-// Two restructurings of this kernel were built and measured in round 2 and are NOT used (tools/experiments/, DESIGN.md
-// section 4): warp-specialised FFT / mel+output warps, and a streaming variant with multi-buffered raw and P.
+// Two restructurings of this kernel were built and measured in round 2 and are NOT used (DESIGN.md section 4):
+// warp-specialised FFT / mel+output warps, and a streaming variant with multi-buffered raw and P.
 #pragma once
 #include <cooperative_groups.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
-
-#include <type_traits>
 
 #include "wlm_common.cuh"
 
@@ -85,17 +83,6 @@ constexpr bool kKoTinyTma = (WLM_KO & 64) != 0, kKoStg = (WLM_KO & 128) != 0,
 #define WLM_WS_BEGIN()
 #define WLM_WS_END(k)
 #endif
-// suspend-time hint (ns) of the CTA-scope mbarrier waits; 0 = none
-#ifndef WLM_WAIT_HINT
-#define WLM_WAIT_HINT 0
-#endif
-// 1: the cluster kernel is itself a programmatic dependent launch (see the kernel's prologue)
-#ifndef WLM_PDL_CHAIN
-#define WLM_PDL_CHAIN 1
-#endif
-#ifndef WLM_OPAQUE_BASE
-#define WLM_OPAQUE_BASE 1
-#endif
 constexpr int kGroups = 2;                // independent warp groups per CTA
 constexpr int kGroupWarps = 8;
 constexpr int kGroupThreads = kGroupWarps * 32;
@@ -127,13 +114,10 @@ constexpr int kPFloats = 2 * kPairs * kPPair;
 
 // The raw buffer starts kRawShift floats into its 128-byte-aligned slab: the TMA source of a half-tile of a dense batch
 // sits at (5120 t - 200) * 4 = 96 mod 128 bytes, and a copy whose destination has the same offset inside a 128-byte line
-// is cheaper (tools/fused_ko.cu, -DWLM_RAW_SHIFT=0/8/16/24: 7,530 / 7,445 / 7,530 / 7,445 cycles per 64 frames; the two
+// is cheaper (tools/fused_ko.cu, shifts of 0/8/16/24 floats: 7,530 / 7,445 / 7,530 / 7,445 cycles per 64 frames; the two
 // sub-regions are 64 bytes apart modulo 128 for the bank layout, so only one of them can be co-aligned).
-#ifndef WLM_RAW_SHIFT
-#define WLM_RAW_SHIFT 24
-#endif
-constexpr int kRawShift = WLM_RAW_SHIFT;
-constexpr int kSmemRaw = kRawFloats * 4 + (kRawShift ? 128 : 0);        // 22,400 + 128
+constexpr int kRawShift = 24;
+constexpr int kSmemRaw = kRawFloats * 4 + 128;                          // 22,400 + 128
 constexpr int kSmemY = kYFloat2 * 8;
 constexpr int kSmemP = kPFloats * 4;
 constexpr int kSmemGroup = kSmemRaw + kSmemY + kSmemP;
@@ -172,7 +156,6 @@ struct KernelTables {
     int16_t nf[kGroupWarps];                             // number of filters of warp w (<= 16)
     int16_t n_mels;
 };
-using MelParams = KernelTables;
 
 // Host-visible tables
 struct Tables {
@@ -255,20 +238,18 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, int count) {
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
 }
+// (operand %2 is unused, but it stays: without it the PTX registers are numbered differently and ptxas allocates the
+// registers of logmel_cluster_kernel<0, false, float, true> differently)
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     asm volatile(
         "{\n"
         ".reg .pred p;\n"
         "WAIT_%=:\n"
-#if WLM_WAIT_HINT
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
-#else
         "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-#endif
         "@p bra DONE_%=;\n"
         "bra WAIT_%=;\n"
         "DONE_%=:\n"
-        "}\n" ::"r"(bar), "r"(parity), "r"(WLM_WAIT_HINT) : "memory");
+        "}\n" ::"r"(bar), "r"(parity), "r"(0) : "memory");
 }
 // same, acquiring at cluster scope: the data the barrier guards was written by other CTAs of the cluster.  (The acquire
 // costs a CCTL.IVALL after the wait; a CTA-scope wait measured the same launch time, so the documented form stays.)
@@ -404,7 +385,6 @@ __device__ __forceinline__ void tile_issue_tma(const ClipArgs& a, const ClipCtx&
 // half-tile never executes -- it measured 3 % SLOWER)
 __device__ __forceinline__ void tile_fixup(int pcm_format, int clip_len, int tile, float* raw, int grp, int tg) {
     const int s0 = tile_s0(tile);
-    struct { int len; } c{clip_len};
     if (pcm_format == WLM_PCM_I16) {
         const int16_t* st = reinterpret_cast<const int16_t*>(raw + kSubLen);
         constexpr float kScale = 1.0f / 32768.0f;
@@ -431,27 +411,27 @@ __device__ __forceinline__ void tile_fixup(int pcm_format, int clip_len, int til
 #pragma unroll 1
         for (int idx = tg; idx < -s0; idx += kGroupThreads) {
             const int sr = -(s0 + idx);
-            raw[idx] = sr < c.len ? raw[sr - s0] : 0.f;        // (sr - s0 <= 400 < kSubLen: same sub-region)
+            raw[idx] = sr < clip_len ? raw[sr - s0] : 0.f;       // (sr - s0 <= 400 < kSubLen: same sub-region)
         }
     }
-    if (s0 + kTileSamples > c.len) {   // the half-tile runs past the clip: zero padding, reflected at sample 480000
+    if (s0 + kTileSamples > clip_len) {   // the half-tile runs past the clip: zero padding, reflected at sample 480000
 #pragma unroll
         for (int r = 0; r < 2; ++r) {
             const int s_lo = s0 + r * kSubStep;
 #pragma unroll 1
-            for (int i = max(c.len - s_lo, 0) + tg; i < kSubLen; i += kGroupThreads) {
+            for (int i = max(clip_len - s_lo, 0) + tg; i < kSubLen; i += kGroupThreads) {
                 const int s = s_lo + i;
                 float v = 0.f;
                 if (s >= kNSamples) {
                     const int sr = 2 * (kNSamples - 1) - s;
                     const int u = sr - s0;
-                    if (sr < c.len && u >= 0) v = raw[u < kSubLen ? u : kSubLen + (u - kSubStep)];
+                    if (sr < clip_len && u >= 0) v = raw[u < kSubLen ? u : kSubLen + (u - kSubStep)];
                 }
                 raw[r * kSubLen + i] = v;
             }
         }
     }
-    if (s0 < 0 || s0 + kTileSamples > c.len) group_sync(grp);
+    if (s0 < 0 || s0 + kTileSamples > clip_len) group_sync(grp);
 }
 
 // ---- stage 1 ----------------------------------------------------------------------------------
@@ -662,7 +642,8 @@ template <> __device__ __forceinline__ float from_out<__nv_bfloat16>(__nv_bfloat
 template <> __device__ __forceinline__ float from_out<__half>(__half v) { return __half2float(v); }
 
 // The element type is a template parameter of the kernel (a run-time switch tripled the code of the output pass and
-// cost 6 % through the instruction cache): f(T*) is called with a.out as OutT*.
+// cost 6 % through the instruction cache): f is called with a.out as OutT*.  A lambda, not a block with a typed pointer:
+// the lambda's scope shapes ptxas's register allocation, and the block form changed the SASS of every kernel instance.
 template <class OutT, class F>
 __device__ __forceinline__ void with_out_type(const ClipArgs& a, F f) { f(static_cast<OutT*>(a.out)); }
 // One base pointer, immediate row offsets and one compare per row: left to the compiler, every row carried its own
@@ -758,6 +739,14 @@ __device__ __forceinline__ void output_rows(T* of, const float (&r)[16], float f
     if constexpr (8 < NFC) output_block<T, 8, NFC>(of, r, floor4, lim, NFC);
     if constexpr (12 < NFC) output_block<T, 12, NFC>(of, r, floor4, lim, NFC);
 }
+// all rows of a warp whose run length `nf` (warp-uniform) is only known at run time
+template <class T>
+__device__ __forceinline__ void output_rows(T* of, const float (&r)[16], float floor4, int lim, int nf) {
+    if (0 < nf) output_block<T, 0>(of, r, floor4, lim, nf);
+    if (4 < nf) output_block<T, 4>(of, r, floor4, lim, nf);
+    if (8 < nf) output_block<T, 8>(of, r, floor4, lim, nf);
+    if (12 < nf) output_block<T, 12>(of, r, floor4, lim, nf);
+}
 
 // ---- the clip queue -----------------------------------------------------------------------------------------------
 // Clips are handed out dynamically: a worker (a cluster, or a CTA of the flat kernel) takes clip `worker` first (its
@@ -839,35 +828,22 @@ logmel_cluster_kernel(const ClipArgs a, const __grid_constant__ KernelTables kt,
     constexpr int kVC = FLAT ? kGroups : kVCluster;      // virtual CTAs (warp groups) that share a clip
     constexpr int kCl = FLAT ? 1 : kCluster;
     extern __shared__ __align__(128) unsigned char smem_sym[];
-#if WLM_OPAQUE_BASE
     // The shared-memory base and the thread index as OPAQUE register values: left alone, the compiler re-derives every
     // shared address from S2R SR_CgaCtaId and re-reads SR_TID.X wherever it is short of registers -- 13 S2R per warp and
     // step, each ~50 cycles of latency on the path (3 % of the stall samples).
     uint32_t smem_base_u32;
     asm volatile("mov.b32 %0, %1;" : "=r"(smem_base_u32) : "r"(static_cast<uint32_t>(__cvta_generic_to_shared(smem_sym))));
     unsigned char* const smem = static_cast<unsigned char*>(__cvta_shared_to_generic(smem_base_u32));
-#else
-    unsigned char* const smem = smem_sym;
-#endif
-#if !WLM_PDL_CHAIN
-    // this CTA is resident: once all of them are, the flat kernel (a programmatic dependent launch) may take the free SMs
-    if constexpr (!FLAT) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#else
     // (flat kernel) the NEXT launch's cluster kernel may be queued now: its CTAs become resident as the clusters of this
     // launch exit and run their prologue; they wait for this launch to complete before they read or write anything of the
     // caller's (griddepcontrol.wait below)
     if constexpr (FLAT) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-#if WLM_OPAQUE_BASE
     // (a special-register read is rematerialised by ptxas wherever it is short of a register, volatile or not; the result
     // of a shuffle is not: the thread index goes through one)
     int tid;
     asm volatile("mov.u32 %0, %%tid.x;" : "=r"(tid));
     tid = __shfl_sync(0xffffffffu, tid, tid & 31);
     const int lane = tid & 31;
-#else
-    const int tid = threadIdx.x, lane = tid & 31;
-#endif
     const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);   // warp-uniform for the compiler
     int tg;                                                   // thread index inside the warp group
     asm volatile("mov.b32 %0, %1;" : "=r"(tg) : "r"(tid & (kGroupThreads - 1)));
@@ -958,7 +934,6 @@ logmel_cluster_kernel(const ClipArgs a, const __grid_constant__ KernelTables kt,
 #pragma unroll
     for (int t = 0; t < 25; ++t) wv[t] = win_lane[n1 * 25 + t];
     if constexpr (!FLAT) {
-#if WLM_PDL_CHAIN
         // Launched as a programmatic dependent of whatever precedes it in the stream (normally the previous wlm_logmel
         // launch): the launch latency and the prologue above -- barrier and tensor-memory set-up, the cluster barrier, the
         // window table -- overlap the tail of that kernel.  Nothing of the caller's has been touched so far (not the PCM,
@@ -966,7 +941,6 @@ logmel_cluster_kernel(const ClipArgs a, const __grid_constant__ KernelTables kt,
         // visible.  Only then may this launch's own dependent (the flat kernel, which reads PCM at once) start.
         asm volatile("griddepcontrol.wait;" ::: "memory");
         asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
         if (leader) {                                            // (DYN) ordinals 1 and 2 of this cluster: one atomic
             const unsigned int c = static_cast<unsigned int>(a.n_workers) + atomicAdd(&a.queue->next, 2u);
             queue_put<false, kCluster>(clipq, 1, c < static_cast<unsigned int>(a.B) ? static_cast<int>(c) : kClipEnd);
@@ -1134,18 +1108,14 @@ logmel_cluster_kernel(const ClipArgs a, const __grid_constant__ KernelTables kt,
             const int otile = vrank + j * kVC;
             const int64_t e0 = pend_e0 + otile * kTile;
             const int lim = (j != tail_j && !(kKoStg && a.B > 0)) ? nf : 0;       // rows this lane stores
-            with_out_type<OutT>(a, [&](auto* outp) {
-                using T = std::remove_pointer_t<decltype(outp)>;
-                T* of = outp + e0;
+            with_out_type<OutT>(a, [&](OutT* outp) {
+                OutT* of = outp + e0;
                 // rows in blocks of four (output_block): straight-line code inside a block, so four MUFU.LG2 chains overlap
                 if constexpr (NMELS == 128) {      // eight runs of 16: no run-length branches, one compare per block (-2 %)
-                    output_rows<T, kMaxFiltersPerWarp>(of, r, floor4, lim);       // (the same per warp for the 80-mel bank, behind
+                    output_rows<OutT, kMaxFiltersPerWarp>(of, r, floor4, lim);    // (the same per warp for the 80-mel bank, behind
                                                                                   // an 8-way dispatch: 500 more instructions, 4.5 % SLOWER)
                 } else {
-                    if (0 < nf) output_block<T, 0>(of, r, floor4, lim, nf);
-                    if (4 < nf) output_block<T, 4>(of, r, floor4, lim, nf);
-                    if (8 < nf) output_block<T, 8>(of, r, floor4, lim, nf);
-                    if (12 < nf) output_block<T, 12>(of, r, floor4, lim, nf);
+                    output_rows<OutT>(of, r, floor4, lim, nf);
                 }
             });
         };
@@ -1176,13 +1146,12 @@ logmel_cluster_kernel(const ClipArgs a, const __grid_constant__ KernelTables kt,
                 const float silent = floor4;
                 const int nf = warp_nf();
                 const int64_t e0 = pend_e0;
-                with_out_type<OutT>(a, [&](auto* outp) {
-                    using T = std::remove_pointer_t<decltype(outp)>;
+                with_out_type<OutT>(a, [&](OutT* outp) {
                     // (left to the compiler's unrolling: ragged batches of short clips spend real time here)
                     for (int tile = vrank + pend_n_my * kVCluster; tile < kTilesPerClip; tile += kVCluster) {
-                        T* of = outp + e0 + tile * kTile;
+                        OutT* of = outp + e0 + tile * kTile;
                         if (tile * kTile + lane < kNFrames)
-                            for (int q = 0; q < nf; ++q) of[q * kNFrames] = to_out<T>(silent);
+                            for (int q = 0; q < nf; ++q) of[q * kNFrames] = to_out<OutT>(silent);
                     }
                 });
             }
@@ -1207,13 +1176,9 @@ logmel_cluster_kernel(const ClipArgs a, const __grid_constant__ KernelTables kt,
                 const int64_t e0 = (static_cast<int64_t>(pb) * a.n_mels + warp_m0()) * kNFrames + ptile * kTile + lane;
                 const int lim = pj != tail_j ? nf : 0;      // rows this lane stores
                 auto sink = [&](const float (&o)[kMaxFiltersPerWarp]) {
-                    with_out_type<OutT>(a, [&](auto* outp) {
-                        using T = std::remove_pointer_t<decltype(outp)>;
-                        T* of = outp + e0;
-                        if (0 < nf) output_block<T, 0>(of, o, -1.5f, lim, nf);      // (-10 + 4) / 4
-                        if (4 < nf) output_block<T, 4>(of, o, -1.5f, lim, nf);
-                        if (8 < nf) output_block<T, 8>(of, o, -1.5f, lim, nf);
-                        if (12 < nf) output_block<T, 12>(of, o, -1.5f, lim, nf);
+                    with_out_type<OutT>(a, [&](OutT* outp) {
+                        OutT* of = outp + e0;
+                        output_rows<OutT>(of, o, -1.5f, lim, nf);      // floor (-10 + 4) / 4
                     });
                 };
                 m1 = NMELS == 0 ? mel_stage(kt, P, wg, lane, sink) : mel_fixed<NMELS == 0 ? 80 : NMELS>(kt, P, wg, lane, sink);
@@ -1258,13 +1223,12 @@ logmel_cluster_kernel(const ClipArgs a, const __grid_constant__ KernelTables kt,
                 if (a.gmax) a.gmax[pb] = gmax;
             }
             const int n_valid = min(kNFrames, pn_act * kTile);          // frames of half-tiles that hold real samples
-            with_out_type<OutT>(a, [&](auto* outp) {
-                using T = std::remove_pointer_t<decltype(outp)>;
-                constexpr int kPer = 16 / static_cast<int>(sizeof(T));  // elements per 16-byte vector (3000 % kPer == 0)
-                struct alignas(16) Vec { T e[kPer]; };
+            with_out_type<OutT>(a, [&](OutT* outp) {
+                constexpr int kPer = 16 / static_cast<int>(sizeof(OutT));   // elements per 16-byte vector (3000 % kPer == 0)
+                struct alignas(16) Vec { OutT e[kPer]; };
                 Vec* oc = reinterpret_cast<Vec*>(outp + static_cast<int64_t>(pb) * a.n_mels * kNFrames);
-                const T thr_t = to_out<T>(thr);                          // rounded like the features: max(round x, round t) = round max(x, t)
-                const float thr_f = from_out<T>(thr_t);
+                const OutT thr_t = to_out<OutT>(thr);                       // rounded like the features: max(round x, round t) = round max(x, t)
+                const float thr_f = from_out<OutT>(thr_t);
                 // eight 16-byte loads in flight per thread: the clip may have left L2 by now (the cluster kernel streams through it)
                 constexpr int kRow = kNFrames / kPer;
                 const int nv = a.n_mels * kRow;
@@ -1285,7 +1249,7 @@ logmel_cluster_kernel(const ClipArgs a, const __grid_constant__ KernelTables kt,
                         const int i = i0 + u * kThreads;
 #pragma unroll
                         for (int e = 0; e < kPer; ++e)
-                            if (from_out<T>(v[u].e[e]) < thr_f) v[u].e[e] = thr_t;
+                            if (from_out<OutT>(v[u].e[e]) < thr_f) v[u].e[e] = thr_t;
                         if (i < nv) *reinterpret_cast<float4*>(oc + i) = *reinterpret_cast<const float4*>(&v[u]);
                     }
                 }
@@ -1400,7 +1364,7 @@ logmel_cluster_kernel(const ClipArgs a, const __grid_constant__ KernelTables kt,
 }
 
 typedef void (*KernelFn)(const ClipArgs, const KernelTables, const float*);
-#ifndef WLM_DEVICE_ONLY   /* tools/stream_ko.cu compiles one kernel, not the whole family */
+#ifndef WLM_DEVICE_ONLY   /* tools/fused_ko.cu compiles one kernel, not the whole family */
 // ---- host side -----------------------------------------------------------------------------------
 // variant: 80 / 128 when the table's structure equals the baked one (and the partition was taken from it)
 template <class OutT, bool DYN>
@@ -1435,14 +1399,11 @@ inline void fill_launch_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* at,
     at[0].val.clusterDim.x = kCluster;
     at[0].val.clusterDim.y = 1;
     at[0].val.clusterDim.z = 1;
-    cfg->attrs = at;
-    cfg->numAttrs = 1;
-#if WLM_PDL_CHAIN
     // the cluster kernel waits (griddepcontrol.wait) for its predecessor in the stream itself, after its prologue
     at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[1].val.programmaticStreamSerializationAllowed = 1;
+    cfg->attrs = at;
     cfg->numAttrs = 2;
-#endif
 }
 
 inline cudaError_t configure(int variant, int* max_clusters) {

@@ -242,6 +242,24 @@ extern "C" size_t wlm_workspace_bytes(const wlm_plan* p, int B) {
 // ------------------------------------------------------------------------------------------
 // launch
 // ------------------------------------------------------------------------------------------
+// the per-call fields of a launch; fused::launch fills in the work split (clip_first, n_workers, ...), launch_logmel the queue
+static ClipArgs clip_args(const wlm_plan* p, const void* pcm, int pcm_format, const int64_t* offsets, const int32_t* lengths,
+                          int64_t row_stride, int B, void* out, float* gmax) {
+    ClipArgs a{};
+    a.pcm = pcm;
+    a.offsets = offsets;
+    a.lengths = lengths;
+    a.row_stride = row_stride;
+    a.dense_len = (int32_t)std::min<int64_t>(row_stride > 0 ? row_stride : 0, kNSamples);
+    a.pcm_format = pcm_format;
+    a.n_mels = p->n_mels;
+    a.B = B;
+    a.out = out;
+    a.gmax = gmax;
+    a.out_format = p->out_format;
+    return a;
+}
+
 static int launch_logmel(wlm_plan* p, const ClipArgs& a0, cudaStream_t st) {
     int n_launches = 0;
     bool flat_broken = false;
@@ -285,18 +303,7 @@ extern "C" int wlm_logmel(wlm_plan* p, const void* pcm_dev, int pcm_format, cons
         gmax = static_cast<float*>(workspace);
     }
     WLM_CUDA(cudaSetDevice(p->device));
-    ClipArgs a;
-    a.pcm = pcm_dev;
-    a.offsets = offsets_dev;
-    a.lengths = lengths_dev;
-    a.row_stride = row_stride;
-    a.dense_len = (int32_t)std::min<int64_t>(row_stride > 0 ? row_stride : 0, kNSamples);
-    a.pcm_format = pcm_format;
-    a.n_mels = p->n_mels;
-    a.B = B;
-    a.out = out_dev;
-    a.gmax = gmax;
-    a.out_format = p->out_format;
+    const ClipArgs a = clip_args(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, B, out_dev, gmax);
     return launch_logmel(p, a, static_cast<cudaStream_t>(stream));
 }
 
@@ -404,18 +411,8 @@ extern "C" int wlm_logmel_host(wlm_plan* p, const void* const* clips_host, const
                                          (size_t)p->h_lengths[b] * esz, cudaMemcpyHostToDevice, st));
         WLM_CUDA(cudaMemcpyAsync(p->d_offsets, p->h_offsets, sizeof(int64_t) * B, cudaMemcpyHostToDevice, st));
         WLM_CUDA(cudaMemcpyAsync(p->d_lengths, p->h_lengths, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
-        ClipArgs a;
-        a.pcm = p->d_stage;
-        a.offsets = p->d_offsets;
-        a.lengths = p->d_lengths;
-        a.row_stride = 0;
-        a.dense_len = 0;
-        a.pcm_format = pcm_format;
-        a.n_mels = p->n_mels;
-        a.B = B;
-            a.out = out_dev;
-        a.gmax = static_cast<float*>(p->d_ws);
-        a.out_format = p->out_format;
+        const ClipArgs a = clip_args(p, p->d_stage, pcm_format, p->d_offsets, p->d_lengths, 0, B, out_dev,
+                                     static_cast<float*>(p->d_ws));
         int rc = launch_logmel(p, a, st);
         if (rc != WLM_OK) return rc;
         WLM_CUDA(cudaEventRecord(p->ev_kernels_done, st));
@@ -488,18 +485,9 @@ extern "C" int wlm_logmel_host(wlm_plan* p, const void* const* clips_host, const
         cudaEvent_t ev = p->ev_chunk[chunk & 3];
         WLM_CUDA(cudaEventRecord(ev, p->copy_stream));
         WLM_CUDA(cudaStreamWaitEvent(st, ev, 0));
-        ClipArgs a;
-        a.pcm = p->d_stage;
-        a.offsets = p->d_offsets + b0;
-        a.lengths = p->d_lengths + b0;
-        a.row_stride = 0;
-        a.dense_len = 0;
-        a.pcm_format = pcm_format;
-        a.n_mels = p->n_mels;
-        a.B = b1 - b0;
-            a.out = static_cast<char*>(out_dev) + (size_t)b0 * p->n_mels * kNFrames * out_elem_size(p);
-        a.gmax = static_cast<float*>(p->d_ws) + b0;
-        a.out_format = p->out_format;
+        const ClipArgs a = clip_args(p, p->d_stage, pcm_format, p->d_offsets + b0, p->d_lengths + b0, 0, b1 - b0,
+                                     static_cast<char*>(out_dev) + (size_t)b0 * p->n_mels * kNFrames * out_elem_size(p),
+                                     static_cast<float*>(p->d_ws) + b0);
         int rc = launch_logmel(p, a, st);
         if (rc != WLM_OK) return rc;
         b0 = b1;
