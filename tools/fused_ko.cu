@@ -1,6 +1,6 @@
 // Knock-out timing of the SHIPPED cluster kernel (results are wrong with any knock-out; timing only): -DWLM_KO=<bits>
 //   1 no raw wait / TMA re-arm   2 no wait for "P full"   4 no wait for "P free"   8 no mel arithmetic   16 no output pass
-//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -DWLM_KO=.. -DWLM_DEVICE_ONLY -I whisper_context_biasing_b200/csrc -I include -o tools/fused_ko_N tools/fused_ko.cu
+//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -DWLM_KO=.. -I whisper_context_biasing_b200/csrc -I include -o tools/fused_ko_N tools/fused_ko.cu
 #include <cuda_runtime.h>
 #include <cmath>
 #include <cstdio>

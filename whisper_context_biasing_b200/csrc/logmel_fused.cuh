@@ -1363,171 +1363,5 @@ logmel_cluster_kernel(const ClipArgs a, const __grid_constant__ KernelTables kt,
     }
 }
 
-typedef void (*KernelFn)(const ClipArgs, const KernelTables, const float*);
-#ifndef WLM_DEVICE_ONLY   /* tools/fused_ko.cu compiles one kernel, not the whole family */
-// ---- host side -----------------------------------------------------------------------------------
-// variant: 80 / 128 when the table's structure equals the baked one (and the partition was taken from it)
-template <class OutT, bool DYN>
-inline KernelFn kernel_for_t(int variant, bool flat) {
-    if (flat) {
-        if (variant == 80) return logmel_cluster_kernel<80, true, OutT, DYN>;
-        if (variant == 128) return logmel_cluster_kernel<128, true, OutT, DYN>;
-        return logmel_cluster_kernel<0, true, OutT, DYN>;
-    }
-    if (variant == 80) return logmel_cluster_kernel<80, false, OutT, DYN>;
-    if (variant == 128) return logmel_cluster_kernel<128, false, OutT, DYN>;
-    return logmel_cluster_kernel<0, false, OutT, DYN>;
-}
-inline KernelFn kernel_for(int variant, bool flat = false, int out_format = WLM_OUT_F32, bool dyn = false) {
-    if (dyn) {
-        if (out_format == WLM_OUT_BF16) return kernel_for_t<__nv_bfloat16, true>(variant, flat);
-        if (out_format == WLM_OUT_F16) return kernel_for_t<__half, true>(variant, flat);
-        return kernel_for_t<float, true>(variant, flat);
-    }
-    if (out_format == WLM_OUT_BF16) return kernel_for_t<__nv_bfloat16, false>(variant, flat);
-    if (out_format == WLM_OUT_F16) return kernel_for_t<__half, false>(variant, flat);
-    return kernel_for_t<float, false>(variant, flat);
-}
-
-inline void fill_launch_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* at, int n_clusters, cudaStream_t st) {
-    memset(cfg, 0, sizeof(*cfg));
-    cfg->gridDim = dim3(kCluster * n_clusters);
-    cfg->blockDim = dim3(kThreads);
-    cfg->dynamicSmemBytes = kSmemBytes;
-    cfg->stream = st;
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = kCluster;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    // the cluster kernel waits (griddepcontrol.wait) for its predecessor in the stream itself, after its prologue
-    at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg->attrs = at;
-    cfg->numAttrs = 2;
-}
-
-inline cudaError_t configure(int variant, int* max_clusters) {
-    KernelFn fn = kernel_for(variant);
-    cudaError_t e = cudaSuccess;
-    for (int fmt : {WLM_OUT_F32, WLM_OUT_BF16, WLM_OUT_F16})
-        for (int k = 0; k < 4; ++k) {
-            e = cudaFuncSetAttribute(kernel_for(variant, (k & 1) != 0, fmt, (k & 2) != 0), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-            if (e != cudaSuccess) return e;
-        }
-    cudaLaunchConfig_t cfg;
-    cudaLaunchAttribute at[2];
-    fill_launch_config(&cfg, at, 148, nullptr);
-    int n = 0;
-    e = cudaOccupancyMaxActiveClusters(&n, fn, &cfg);
-    if (e != cudaSuccess) return e;
-    if (n < 1) return cudaErrorLaunchOutOfResources;
-    *max_clusters = n;
-    return cudaSuccess;
-}
-
-// The flat kernel runs on the `flat_ctas` SMs the clusters leave idle.  Next to a running cluster kernel a flat CTA needs
-// about `rounds_per_clip` cluster rounds (one clip per co-resident cluster) for a clip (tools/flat_time.py), so it is only
-// worth starting -- and, in a dynamic launch, only worth taking another clip -- while the clusters still have at least that
-// many rounds of clips ahead of them; otherwise the whole GPU would wait for 16 SMs at the end of the batch.
-inline double flat_rounds_per_clip(int n_mels) { return 6.5 + 0.00625 * n_mels; }
-inline int flat_reserve_clips(int n_mels, int n_clusters) {
-    return static_cast<int>(flat_rounds_per_clip(n_mels) * n_clusters + 0.999);
-}
-// static split of a dense batch: the largest number of whole flat rounds (one clip per flat CTA) that finish no later
-// than the cluster kernel does with the rest
-inline int flat_clip_count(const ClipArgs& a, int max_clusters, int flat_ctas) {
-    if (flat_ctas <= 0 || a.B < 2 * max_clusters) return 0;
-    const double rounds_per_clip = flat_rounds_per_clip(a.n_mels);
-    int k = 0;
-    while ((k + 1) * flat_ctas < a.B &&
-           (k + 1) * rounds_per_clip <= (a.B - (k + 1) * flat_ctas + max_clusters - 1) / max_clusters) ++k;
-    return k * flat_ctas;
-}
-
-// One launch = the cluster kernel plus, when it pays, its flat twin, as a PROGRAMMATIC DEPENDENT launch: the flat kernel
-// becomes schedulable when every CTA of the cluster kernel has executed griddepcontrol.launch_dependents, i.e. is resident --
-// its CTAs can then only land on the SMs the clusters left free.  (Submitted as an independent kernel on a second stream it
-// sometimes got SMs first and kept clusters from being placed.)  It consumes nothing the cluster kernel produces; it
-// executes griddepcontrol.wait just before it exits, so the last kernel in the stream completes after both have written
-// everything and later work in the stream is ordered behind both.
-//   dense batch (no per-clip lengths), flat_override < 0:  STATIC -- clips [0, B - n_flat) round-robin over the clusters,
-//       the last n_flat over the flat CTAs (every clip costs the same, so the split is known up front and the kernels carry
-//       no queue code: the dynamic variant measured 6 % slower on dense batches);
-//   everything else:  DYNAMIC -- both kernels pull clips from the plan's queue.
-// flat_override: -1 = the rules above; 0 = no flat kernel; n > 0 = dynamic, the flat kernel may take up to n clips, no
-// reserve (tests: any assignment must give bit-identical features).
-inline cudaError_t launch(const ClipArgs& a0, const Tables* d_tables, const Tables& h_tables, int variant,
-                          int max_clusters, cudaStream_t st, int* n_launches, int flat_ctas = 0, int flat_override = -1,
-                          bool* flat_broken = nullptr) {
-    ClipArgs a = a0;
-    const bool dyn = !(a.lengths == nullptr && flat_override < 0);
-    int nc, nf = 0;
-    ClipArgs af = a;
-    a.clip_first = 0;
-    a.worker_base = 0;
-    a.flat_reserve = 0;
-    a.flat_cap = 0x7fffffff;
-    if (!dyn) {
-        const int n_flat = flat_clip_count(a, max_clusters, flat_ctas);
-        af = a;
-        af.clip_first = a.B - n_flat;
-        a.B -= n_flat;
-        nc = a.B < max_clusters ? a.B : max_clusters;
-        nf = n_flat < flat_ctas ? n_flat : flat_ctas;
-        a.n_workers = nc;
-        af.n_workers = nf;
-    } else {
-        nc = a.B < max_clusters ? a.B : max_clusters;
-        a.flat_reserve = flat_reserve_clips(a.n_mels, nc);
-        if (flat_ctas > 0 && flat_override != 0) {
-            if (flat_override > 0) {
-                nf = flat_override < flat_ctas ? flat_override : flat_ctas;
-                if (nf > a.B - nc) nf = a.B - nc;
-                a.flat_reserve = 0;
-                a.flat_cap = nf > 0 ? (flat_override + nf - 1) / nf : 0;
-            } else {
-                nf = a.B - a.flat_reserve;
-                if (nf > flat_ctas) nf = flat_ctas;
-            }
-            if (nf < 0) nf = 0;
-        }
-        a.n_workers = nc + nf;
-        af = a;
-        af.worker_base = nc;
-    }
-    cudaLaunchConfig_t cfg;
-    cudaLaunchAttribute at[2];
-    fill_launch_config(&cfg, at, nc, st);
-    *n_launches = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, kernel_for(variant, false, a.out_format, dyn), a, h_tables.mel,
-                                       static_cast<const float*>(d_tables->win_lane));
-    if (e != cudaSuccess || nf == 0) return e;
-    cudaLaunchConfig_t fcfg;
-    memset(&fcfg, 0, sizeof(fcfg));
-    fcfg.gridDim = dim3(nf);
-    fcfg.blockDim = dim3(kThreads);
-    fcfg.dynamicSmemBytes = kSmemBytes;
-    fcfg.stream = st;
-    cudaLaunchAttribute fat[1];
-    fat[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    fat[0].val.programmaticStreamSerializationAllowed = 1;
-    fcfg.attrs = fat;
-    fcfg.numAttrs = 1;
-    *n_launches = 2;
-    e = cudaLaunchKernelEx(&fcfg, kernel_for(variant, true, af.out_format, dyn), af, h_tables.mel,
-                           static_cast<const float*>(d_tables->win_lane));
-    if (e == cudaSuccess) return e;
-    // the dependent launch was refused (driver without programmatic launches?): the flat CTAs' clips are already theirs, so
-    // the same kernel goes out as an ordinary launch (it then runs after the cluster kernel) and the plan stops using it
-    (void)cudaGetLastError();
-    if (flat_broken) *flat_broken = true;
-    fcfg.attrs = nullptr;
-    fcfg.numAttrs = 0;
-    return cudaLaunchKernelEx(&fcfg, kernel_for(variant, true, af.out_format, dyn), af, h_tables.mel,
-                              static_cast<const float*>(d_tables->win_lane));
-}
-
-#endif  // WLM_DEVICE_ONLY
-
 }  // namespace fused
 }  // namespace wlm

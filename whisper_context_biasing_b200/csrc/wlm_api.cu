@@ -1,7 +1,8 @@
 // libwlm.so -- C ABI (include/wlm.h) over the sm_100a log-mel kernels.
 //
 // Host side only: plan construction (mel table -> sparse form, constant tables), argument
-// validation, launch sequencing, the pinned-ring H2D pipeline of wlm_logmel_host.
+// validation, the launch policy (which kernel instance, how the clips split between the cluster
+// kernel and its flat twin), the pinned-ring H2D pipeline of wlm_logmel_host.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -43,6 +44,72 @@ static int fail(int code, const char* fmt, ...) {
     } while (0)
 
 // ------------------------------------------------------------------------------------------
+// kernel instances
+// ------------------------------------------------------------------------------------------
+typedef void (*KernelFn)(const ClipArgs, const fused::KernelTables, const float*);
+
+// variant: 80 / 128 when the table's structure equals the baked one (and the partition was taken from it)
+template <class OutT, bool DYN>
+static KernelFn kernel_for_t(int variant, bool flat) {
+    using fused::logmel_cluster_kernel;
+    if (flat) {
+        if (variant == 80) return logmel_cluster_kernel<80, true, OutT, DYN>;
+        if (variant == 128) return logmel_cluster_kernel<128, true, OutT, DYN>;
+        return logmel_cluster_kernel<0, true, OutT, DYN>;
+    }
+    if (variant == 80) return logmel_cluster_kernel<80, false, OutT, DYN>;
+    if (variant == 128) return logmel_cluster_kernel<128, false, OutT, DYN>;
+    return logmel_cluster_kernel<0, false, OutT, DYN>;
+}
+static KernelFn kernel_for(int variant, bool flat, int out_format, bool dyn) {
+    if (dyn) {
+        if (out_format == WLM_OUT_BF16) return kernel_for_t<__nv_bfloat16, true>(variant, flat);
+        if (out_format == WLM_OUT_F16) return kernel_for_t<__half, true>(variant, flat);
+        return kernel_for_t<float, true>(variant, flat);
+    }
+    if (out_format == WLM_OUT_BF16) return kernel_for_t<__nv_bfloat16, false>(variant, flat);
+    if (out_format == WLM_OUT_F16) return kernel_for_t<__half, false>(variant, flat);
+    return kernel_for_t<float, false>(variant, flat);
+}
+
+// launch configuration of the cluster kernel; the flat kernel uses the same one without the cluster dimension (at[0])
+static void fill_launch_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* at, int n_clusters, cudaStream_t st) {
+    memset(cfg, 0, sizeof(*cfg));
+    cfg->gridDim = dim3(fused::kCluster * n_clusters);
+    cfg->blockDim = dim3(fused::kThreads);
+    cfg->dynamicSmemBytes = fused::kSmemBytes;
+    cfg->stream = st;
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = fused::kCluster;
+    at[0].val.clusterDim.y = 1;
+    at[0].val.clusterDim.z = 1;
+    // the cluster kernel waits (griddepcontrol.wait) for its predecessor in the stream itself, after its prologue
+    at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[1].val.programmaticStreamSerializationAllowed = 1;
+    cfg->attrs = at;
+    cfg->numAttrs = 2;
+}
+
+static cudaError_t configure(int variant, int* max_clusters) {
+    cudaError_t e = cudaSuccess;
+    for (int fmt : {WLM_OUT_F32, WLM_OUT_BF16, WLM_OUT_F16})
+        for (int k = 0; k < 4; ++k) {
+            e = cudaFuncSetAttribute(kernel_for(variant, (k & 1) != 0, fmt, (k & 2) != 0),
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, fused::kSmemBytes);
+            if (e != cudaSuccess) return e;
+        }
+    cudaLaunchConfig_t cfg;
+    cudaLaunchAttribute at[2];
+    fill_launch_config(&cfg, at, 148, nullptr);
+    int n = 0;
+    e = cudaOccupancyMaxActiveClusters(&n, kernel_for(variant, false, WLM_OUT_F32, false), &cfg);
+    if (e != cudaSuccess) return e;
+    if (n < 1) return cudaErrorLaunchOutOfResources;
+    *max_clusters = n;
+    return cudaSuccess;
+}
+
+// ------------------------------------------------------------------------------------------
 // plan
 // ------------------------------------------------------------------------------------------
 struct wlm_plan {
@@ -54,15 +121,14 @@ struct wlm_plan {
     int flat_override = -1;        // clips for the flat kernel (dense batches); -1 = the library's split
 
     // constant tables: the sparse mel form travels in the constant bank (kernel argument), the window on the device
-    MelSparse h_sparse;
-    fused::Tables* d_fused_tables = nullptr;
-    fused::Tables h_fused_tables;
+    fused::KernelTables mel;
+    float* d_win_lane = nullptr;
     ClipQueue* d_queue = nullptr;  // clip counter the two kernels of a launch pull from (self-resetting)
     int max_clusters = 0;          // co-resident clusters of the fused kernel (occupancy query)
     int flat_ctas = 0;             // SMs the clusters cannot cover: they run the flat kernel (programmatic dependent launch)
     int variant = 0;               // 80 / 128: unrolled mel stage (Whisper banks); 0: table-driven
 
-    // wlm_logmel_host pipeline
+    // wlm_logmel_host pipeline; its buffers only grow (grow_buffer), each *_bytes is the size allocated
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_chunk[4] = {nullptr, nullptr, nullptr, nullptr};
     cudaEvent_t ev_slot_free[2] = {nullptr, nullptr};
@@ -70,13 +136,16 @@ struct wlm_plan {
     bool kernels_done_valid = false;
     void* d_stage = nullptr;  // packed PCM
     size_t d_stage_bytes = 0;
-    void* h_ring[2] = {nullptr, nullptr};
-    size_t h_ring_bytes = 0;
+    void* h_ring[2] = {nullptr, nullptr};  // pinned
+    size_t h_ring_bytes[2] = {0, 0};
     int64_t* d_offsets = nullptr;
+    size_t d_offsets_bytes = 0;
     int32_t* d_lengths = nullptr;
+    size_t d_lengths_bytes = 0;
     int64_t* h_offsets = nullptr;  // pinned
+    size_t h_offsets_bytes = 0;
     int32_t* h_lengths = nullptr;  // pinned
-    int meta_cap = 0;
+    size_t h_lengths_bytes = 0;
     void* d_ws = nullptr;
     size_t d_ws_bytes = 0;
 };
@@ -84,11 +153,8 @@ struct wlm_plan {
 extern "C" int wlm_version(void) { return WLM_VERSION; }
 extern "C" const char* wlm_last_error(void) { return g_last_error.c_str(); }
 
-static int build_sparse(const float* dense, int n_mels, MelSparse* sp, std::vector<int16_t>* klo,
-                        std::vector<int16_t>* khi) {
-    klo->assign(n_mels, 0);
-    khi->assign(n_mels, -1);
-    std::vector<int> seen(n_mels, 0);
+static int build_sparse(const float* dense, int n_mels, MelSparse* sp) {
+    std::vector<int16_t> khi(n_mels, -1);  // last bin of filter m so far: its support must be contiguous
     memset(sp, 0, sizeof(*sp));
     for (int k = 0; k < kNFreq + 3; ++k) sp->lo[k] = -1;  // -1 = "filter before the first" (dummy)
     int prev_lo = -1;
@@ -100,10 +166,9 @@ static int build_sparse(const float* dense, int n_mels, MelSparse* sp, std::vect
             if (w != 0.0f) {
                 if (n == 2) return fail(WLM_ERR_UNSUPPORTED, "mel table: FFT bin %d feeds more than two filters", k);
                 idx[n++] = m;
-                if (!seen[m]) { (*klo)[m] = (int16_t)k; seen[m] = 1; }
-                if ((*khi)[m] >= 0 && (*khi)[m] != k - 1)
+                if (khi[m] >= 0 && khi[m] != k - 1)
                     return fail(WLM_ERR_UNSUPPORTED, "mel table: filter %d has non-contiguous support at bin %d", m, k);
-                (*khi)[m] = (int16_t)k;
+                khi[m] = (int16_t)k;
             }
         }
         if (n == 2 && idx[1] != idx[0] + 1)
@@ -127,8 +192,6 @@ static int build_sparse(const float* dense, int n_mels, MelSparse* sp, std::vect
         if (sp->lo[k] < prev_lo) return fail(WLM_ERR_UNSUPPORTED, "mel table: filter order not monotone at bin %d", k);
         prev_lo = sp->lo[k];
     }
-    for (int m = 0; m < n_mels; ++m)
-        if (!seen[m]) { (*klo)[m] = 0; (*khi)[m] = -1; }  // empty filter: contributes 0 -> log10(1e-10)
     return WLM_OK;
 }
 
@@ -148,13 +211,20 @@ extern "C" int wlm_plan_create(int device, int n_mels, const float* mel_dense_ho
         return fail(WLM_ERR_NO_DEVICE, "device %d is sm_%d%d; libwlm is built for sm_100a only", device, prop.major, prop.minor);
     WLM_CUDA(cudaSetDevice(device));
 
+    MelSparse sparse;
+    const int rc = build_sparse(mel_dense_host, n_mels, &sparse);
+    if (rc != WLM_OK) return rc;
+    fused::Tables tables;
+    int variant = 0;
+    if (fused::build_tables(sparse, n_mels, &tables, &variant) != 0)
+        return fail(WLM_ERR_UNSUPPORTED, "mel table: a filter has no FFT bin (num_mel_filters too high for 201 bins)");
+
     wlm_plan* p = new wlm_plan();
     p->device = device;
     p->n_mels = n_mels;
     p->sm_count = prop.multiProcessorCount;
-    std::vector<int16_t> klo, khi;
-    int rc = build_sparse(mel_dense_host, n_mels, &p->h_sparse, &klo, &khi);
-    if (rc != WLM_OK) { delete p; return rc; }
+    p->variant = variant;
+    p->mel = tables.mel;
 
 #define WLM_CUDA_P(expr)                                                                          \
     do {                                                                                          \
@@ -165,26 +235,20 @@ extern "C" int wlm_plan_create(int device, int n_mels, const float* mel_dense_ho
         }                                                                                         \
     } while (0)
 
-    {
-        if (fused::build_tables(p->h_sparse, n_mels, &p->h_fused_tables, &p->variant) != 0) {
-            wlm_plan_destroy(p);
-            return fail(WLM_ERR_UNSUPPORTED, "mel table: a filter has no FFT bin (num_mel_filters too high for 201 bins)");
-        }
-        WLM_CUDA_P(cudaMalloc(&p->d_fused_tables, sizeof(fused::Tables)));
-        WLM_CUDA_P(cudaMemcpy(p->d_fused_tables, &p->h_fused_tables, sizeof(fused::Tables), cudaMemcpyHostToDevice));
-        WLM_CUDA_P(cudaMalloc(&p->d_queue, sizeof(ClipQueue)));
-        WLM_CUDA_P(cudaMemset(p->d_queue, 0, sizeof(ClipQueue)));
-        cudaError_t fe = fused::configure(p->variant, &p->max_clusters);
-        if (fe != cudaSuccess) {
-            wlm_plan_destroy(p);
-            return fail(WLM_ERR_CUDA, "fused kernel configuration failed: %s", cudaGetErrorString(fe));
-        }
-        // the SMs that whole clusters cannot cover run the flat kernel (WLM_FLAT=0 turns that off)
-        const char* fl = getenv("WLM_FLAT");
-        p->flat_ctas = (fl && atoi(fl) == 0) ? 0 : std::max(0, p->sm_count - fused::kCluster * p->max_clusters);
-        // read ONCE (not per launch); clamped to [0, B - 1] when used
-        if (const char* fc = getenv("WLM_FLAT_CLIPS")) p->flat_override = std::max(-1, atoi(fc));
+    WLM_CUDA_P(cudaMalloc(&p->d_win_lane, sizeof(tables.win_lane)));
+    WLM_CUDA_P(cudaMemcpy(p->d_win_lane, tables.win_lane, sizeof(tables.win_lane), cudaMemcpyHostToDevice));
+    WLM_CUDA_P(cudaMalloc(&p->d_queue, sizeof(ClipQueue)));
+    WLM_CUDA_P(cudaMemset(p->d_queue, 0, sizeof(ClipQueue)));
+    cudaError_t fe = configure(p->variant, &p->max_clusters);
+    if (fe != cudaSuccess) {
+        wlm_plan_destroy(p);
+        return fail(WLM_ERR_CUDA, "fused kernel configuration failed: %s", cudaGetErrorString(fe));
     }
+    // the SMs that whole clusters cannot cover run the flat kernel (WLM_FLAT=0 turns that off)
+    const char* fl = getenv("WLM_FLAT");
+    p->flat_ctas = (fl && atoi(fl) == 0) ? 0 : std::max(0, p->sm_count - fused::kCluster * p->max_clusters);
+    // read ONCE (not per launch); clamped to [0, B - 1] when used
+    if (const char* fc = getenv("WLM_FLAT_CLIPS")) p->flat_override = std::max(-1, atoi(fc));
 
     WLM_CUDA_P(cudaStreamCreateWithFlags(&p->copy_stream, cudaStreamNonBlocking));
     for (auto& ev : p->ev_chunk) WLM_CUDA_P(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
@@ -199,7 +263,7 @@ extern "C" int wlm_plan_destroy(wlm_plan* p) {
     if (!p) return WLM_OK;
     cudaSetDevice(p->device);
     cudaDeviceSynchronize();
-    cudaFree(p->d_fused_tables);
+    cudaFree(p->d_win_lane);
     cudaFree(p->d_queue);
     cudaFree(p->d_stage); cudaFree(p->d_offsets); cudaFree(p->d_lengths); cudaFree(p->d_ws);
     for (auto& r : p->h_ring) if (r) cudaFreeHost(r);
@@ -242,7 +306,7 @@ extern "C" size_t wlm_workspace_bytes(const wlm_plan* p, int B) {
 // ------------------------------------------------------------------------------------------
 // launch
 // ------------------------------------------------------------------------------------------
-// the per-call fields of a launch; fused::launch fills in the work split (clip_first, n_workers, ...), launch_logmel the queue
+// the per-call fields of a launch; launch_logmel fills in the queue and the work split (clip_first, n_workers, ...)
 static ClipArgs clip_args(const wlm_plan* p, const void* pcm, int pcm_format, const int64_t* offsets, const int32_t* lengths,
                           int64_t row_stride, int B, void* out, float* gmax) {
     ClipArgs a{};
@@ -260,19 +324,119 @@ static ClipArgs clip_args(const wlm_plan* p, const void* pcm, int pcm_format, co
     return a;
 }
 
-static int launch_logmel(wlm_plan* p, const ClipArgs& a0, cudaStream_t st) {
-    int n_launches = 0;
-    bool flat_broken = false;
-    ClipArgs a = a0;
+// The flat kernel runs on the `flat_ctas` SMs the clusters leave idle.  Next to a running cluster kernel a flat CTA needs
+// about `rounds_per_clip` cluster rounds (one clip per co-resident cluster) for a clip (tools/flat_time.py), so it is only
+// worth starting -- and, in a dynamic launch, only worth taking another clip -- while the clusters still have at least that
+// many rounds of clips ahead of them; otherwise the whole GPU would wait for 16 SMs at the end of the batch.
+static double flat_rounds_per_clip(int n_mels) { return 6.5 + 0.00625 * n_mels; }
+static int flat_reserve_clips(int n_mels, int n_clusters) {
+    return static_cast<int>(flat_rounds_per_clip(n_mels) * n_clusters + 0.999);
+}
+// static split of a dense batch: the largest number of whole flat rounds (one clip per flat CTA) that finish no later
+// than the cluster kernel does with the rest
+static int flat_clip_count(int B, int n_mels, int max_clusters, int flat_ctas) {
+    if (flat_ctas <= 0 || B < 2 * max_clusters) return 0;
+    const double rounds_per_clip = flat_rounds_per_clip(n_mels);
+    int k = 0;
+    while ((k + 1) * flat_ctas < B &&
+           (k + 1) * rounds_per_clip <= (B - (k + 1) * flat_ctas + max_clusters - 1) / max_clusters) ++k;
+    return k * flat_ctas;
+}
+
+// Which clips the cluster kernel and its flat twin take:
+//   dense batch (no per-clip lengths), flat_override < 0:  STATIC -- clips [0, B - n_flat) round-robin over the clusters,
+//       the last n_flat over the flat CTAs (every clip costs the same, so the split is known up front and the kernels carry
+//       no queue code: the dynamic variant measured 6 % slower on dense batches);
+//   everything else:  DYNAMIC -- both kernels pull clips from the plan's queue.
+// flat_override: -1 = the rules above; 0 = no flat kernel; n > 0 = dynamic, the flat kernel may take up to n clips, no
+// reserve (tests: any assignment must give bit-identical features).
+struct Split {
+    struct Part { int B, clip_first, n_workers, worker_base; };   // the ClipArgs fields that differ between the kernels
+    bool dyn;
+    int n_clusters;               // grid of the cluster kernel, in clusters
+    int n_flat;                   // grid of the flat kernel, in CTAs; 0 = the cluster kernel runs alone
+    int flat_reserve, flat_cap;   // ClipArgs fields, the same for both kernels
+    Part cluster, flat;
+};
+
+static Split split_clips(int B, bool dense, int n_mels, int max_clusters, int flat_ctas, int flat_override) {
+    Split s{};
+    s.dyn = !(dense && flat_override < 0);
+    s.flat_cap = 0x7fffffff;
+    if (!s.dyn) {
+        const int n_flat = flat_clip_count(B, n_mels, max_clusters, flat_ctas);
+        s.n_clusters = std::min(B - n_flat, max_clusters);
+        s.n_flat = std::min(n_flat, flat_ctas);
+        s.cluster = {B - n_flat, 0, s.n_clusters, 0};
+        s.flat = {B, B - n_flat, s.n_flat, 0};
+        return s;
+    }
+    const int nc = std::min(B, max_clusters);
+    int nf = 0;
+    s.flat_reserve = flat_reserve_clips(n_mels, nc);
+    if (flat_ctas > 0 && flat_override != 0) {
+        if (flat_override > 0) {
+            nf = std::min(std::min(flat_override, flat_ctas), B - nc);
+            s.flat_reserve = 0;
+            s.flat_cap = nf > 0 ? (flat_override + nf - 1) / nf : 0;
+        } else {
+            nf = std::min(B - s.flat_reserve, flat_ctas);
+        }
+        nf = std::max(nf, 0);
+    }
+    s.n_clusters = nc;
+    s.n_flat = nf;
+    s.cluster = {B, 0, nc + nf, 0};
+    s.flat = {B, 0, nc + nf, nc};
+    return s;
+}
+
+// One launch = the cluster kernel plus, when it pays, its flat twin, as a PROGRAMMATIC DEPENDENT launch: the flat kernel
+// becomes schedulable when every CTA of the cluster kernel has executed griddepcontrol.launch_dependents, i.e. is resident --
+// its CTAs can then only land on the SMs the clusters left free.  (Submitted as an independent kernel on a second stream it
+// sometimes got SMs first and kept clusters from being placed.)  It consumes nothing the cluster kernel produces; it
+// executes griddepcontrol.wait just before it exits, so the last kernel in the stream completes after both have written
+// everything and later work in the stream is ordered behind both.
+static int launch_logmel(wlm_plan* p, ClipArgs a, cudaStream_t st) {
+    const Split s = split_clips(a.B, a.lengths == nullptr, a.n_mels, p->max_clusters, p->flat_ctas, p->flat_override);
     a.queue = p->d_queue;
-    cudaError_t e = fused::launch(a, p->d_fused_tables, p->h_fused_tables, p->variant, p->max_clusters, st, &n_launches,
-                                  p->flat_ctas, p->flat_override, &flat_broken);
-    if (flat_broken) p->flat_ctas = 0;
+    a.flat_reserve = s.flat_reserve;
+    a.flat_cap = s.flat_cap;
+    auto args = [&](const Split::Part& k) {
+        ClipArgs r = a;
+        r.B = k.B;
+        r.clip_first = k.clip_first;
+        r.n_workers = k.n_workers;
+        r.worker_base = k.worker_base;
+        return r;
+    };
+    cudaLaunchConfig_t cfg;
+    cudaLaunchAttribute at[2];
+    fill_launch_config(&cfg, at, s.n_clusters, st);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kernel_for(p->variant, false, a.out_format, s.dyn), args(s.cluster), p->mel,
+                                       p->d_win_lane);
+    if (e == cudaSuccess && s.n_flat > 0) {
+        const KernelFn flat_fn = kernel_for(p->variant, true, a.out_format, s.dyn);
+        cfg.gridDim = dim3(s.n_flat);
+        cfg.attrs = at + 1;   // programmatic stream serialisation only
+        cfg.numAttrs = 1;
+        e = cudaLaunchKernelEx(&cfg, flat_fn, args(s.flat), p->mel, p->d_win_lane);
+        if (e != cudaSuccess) {
+            // the dependent launch was refused (driver without programmatic launches?): the flat CTAs' clips are already
+            // theirs, so the same kernel goes out as an ordinary launch (it then runs after the cluster kernel) and the
+            // plan stops using it
+            (void)cudaGetLastError();
+            p->flat_ctas = 0;
+            cfg.attrs = nullptr;
+            cfg.numAttrs = 0;
+            e = cudaLaunchKernelEx(&cfg, flat_fn, args(s.flat), p->mel, p->d_win_lane);
+        }
+    }
     if (e != cudaSuccess) {
         cudaMemsetAsync(p->d_queue, 0, sizeof(ClipQueue), st);      // whatever was launched has left: start clean next time
         return fail(WLM_ERR_CUDA, "fused launch failed: %s", cudaGetErrorString(e));
     }
-    p->launches += n_launches;
+    p->launches += s.n_flat > 0 ? 2 : 1;
     WLM_CUDA(cudaGetLastError());
     return WLM_OK;
 }
@@ -345,91 +509,33 @@ static bool is_pinned_host(const void* ptr) {
     return at.type == cudaMemoryTypeHost;
 }
 
-extern "C" int wlm_logmel_host(wlm_plan* p, const void* const* clips_host, const int32_t* lengths_host,
-                               int pcm_format, int B, void* out_dev, void* out_host, void* stream) {
-    if (!p) return fail(WLM_ERR_BAD_ARG, "plan is NULL");
-    if (B < 0) return fail(WLM_ERR_BAD_ARG, "B=%d is negative", B);
-    if (B == 0) return WLM_OK;
-    if (!clips_host || !lengths_host || !out_dev) return fail(WLM_ERR_BAD_ARG, "clips_host/lengths_host/out_dev is NULL");
-    if (pcm_format != WLM_PCM_F32 && pcm_format != WLM_PCM_I16) return fail(WLM_ERR_BAD_ARG, "unknown pcm_format %d", pcm_format);
-    if (reinterpret_cast<uintptr_t>(out_dev) & 15) return fail(WLM_ERR_BAD_ARG, "out_dev must be 16-byte aligned");
-    WLM_CUDA(cudaSetDevice(p->device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const size_t esz = pcm_format == WLM_PCM_I16 ? 2 : 4;
-    const int64_t align_el = 16 / esz * 2;  // clip starts at 32-byte boundaries of the packed buffer
+// Grows a buffer of the plan (device memory, or pinned host memory) to at least `bytes`; *cap is its allocated size.
+template <class T>
+static cudaError_t grow_buffer(T** buf, size_t* cap, size_t bytes, bool pinned) {
+    if (bytes <= *cap) return cudaSuccess;
+    void** b = reinterpret_cast<void**>(buf);
+    if (*b) {
+        if (pinned) cudaFreeHost(*b);
+        else cudaFree(*b);
+    }
+    *b = nullptr;
+    *cap = 0;
+    const cudaError_t e = pinned ? cudaMallocHost(b, bytes) : cudaMalloc(b, bytes);
+    if (e == cudaSuccess) *cap = bytes;
+    return e;
+}
 
-    // metadata
-    if (B > p->meta_cap) {
-        cudaFree(p->d_offsets); cudaFree(p->d_lengths);
-        if (p->h_offsets) cudaFreeHost(p->h_offsets);
-        if (p->h_lengths) cudaFreeHost(p->h_lengths);
-        p->d_offsets = nullptr; p->d_lengths = nullptr; p->h_offsets = nullptr; p->h_lengths = nullptr;
-        p->meta_cap = 0;
-        const int cap = std::max(B, 256);
-        WLM_CUDA(cudaMalloc(&p->d_offsets, sizeof(int64_t) * cap));
-        WLM_CUDA(cudaMalloc(&p->d_lengths, sizeof(int32_t) * cap));
-        WLM_CUDA(cudaMallocHost(&p->h_offsets, sizeof(int64_t) * cap));
-        WLM_CUDA(cudaMallocHost(&p->h_lengths, sizeof(int32_t) * cap));
-        p->meta_cap = cap;
-    }
-    // a previous call's kernels may still be reading the staging buffers / metadata
-    if (p->kernels_done_valid) WLM_CUDA(cudaEventSynchronize(p->ev_kernels_done));
+static constexpr size_t kRingBytes = 64u << 20;   // each of the two pinned slots pageable clips bounce through
 
-    int64_t total_el = 0;
-    for (int b = 0; b < B; ++b) {
-        if (lengths_host[b] < 0) return fail(WLM_ERR_BAD_ARG, "lengths_host[%d]=%d is negative", b, lengths_host[b]);
-        if (lengths_host[b] > 0 && !clips_host[b]) return fail(WLM_ERR_BAD_ARG, "clips_host[%d] is NULL", b);
-        const int32_t len = std::min<int32_t>(lengths_host[b], kNSamples);
-        p->h_offsets[b] = total_el;
-        p->h_lengths[b] = len;
-        total_el += (len + align_el - 1) / align_el * align_el;
-    }
-    const size_t total_bytes = std::max<size_t>((size_t)total_el * esz, 256);
-    if (total_bytes > p->d_stage_bytes) {
-        cudaFree(p->d_stage);
-        p->d_stage = nullptr; p->d_stage_bytes = 0;
-        WLM_CUDA(cudaMalloc(&p->d_stage, total_bytes));
-        p->d_stage_bytes = total_bytes;
-    }
-    const size_t ws_need = wlm_workspace_bytes(p, B);
-    if (ws_need > p->d_ws_bytes) {
-        cudaFree(p->d_ws);
-        p->d_ws = nullptr; p->d_ws_bytes = 0;
-        WLM_CUDA(cudaMalloc(&p->d_ws, ws_need));
-        p->d_ws_bytes = ws_need;
-    }
-    // Small pageable batches -- the reference's own call shape, ONE clip per call (REF/data_utils/data_loader.py:171):
-    // no ring bounce, no copy stream, no events.  cudaMemcpyAsync from pageable memory returns once the source has been
-    // staged by the driver, so the host buffers are reusable on return without any synchronisation here.
-    bool small_pageable = (size_t)total_el * esz <= (4u << 20);
-    for (int b = 0; small_pageable && b < B; ++b)
-        if (p->h_lengths[b] > 0 && is_pinned_host(clips_host[b])) small_pageable = false;
-    if (small_pageable) {
-        for (int b = 0; b < B; ++b)
-            if (p->h_lengths[b] > 0)
-                WLM_CUDA(cudaMemcpyAsync(static_cast<char*>(p->d_stage) + p->h_offsets[b] * esz, clips_host[b],
-                                         (size_t)p->h_lengths[b] * esz, cudaMemcpyHostToDevice, st));
-        WLM_CUDA(cudaMemcpyAsync(p->d_offsets, p->h_offsets, sizeof(int64_t) * B, cudaMemcpyHostToDevice, st));
-        WLM_CUDA(cudaMemcpyAsync(p->d_lengths, p->h_lengths, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
-        const ClipArgs a = clip_args(p, p->d_stage, pcm_format, p->d_offsets, p->d_lengths, 0, B, out_dev,
-                                     static_cast<float*>(p->d_ws));
-        int rc = launch_logmel(p, a, st);
-        if (rc != WLM_OK) return rc;
-        WLM_CUDA(cudaEventRecord(p->ev_kernels_done, st));
-        p->kernels_done_valid = true;
-        if (out_host) {
-            WLM_CUDA(cudaMemcpyAsync(out_host, out_dev, out_elem_size(p) * (size_t)B * p->n_mels * kNFrames,
-                                     cudaMemcpyDeviceToHost, st));
-            WLM_CUDA(cudaStreamSynchronize(st));
-        }
-        return WLM_OK;
-    }
+// wlm_logmel_host for all but small pageable batches: the PCM goes over on the plan's copy stream, chunk by chunk, and
+// every chunk's kernels wait for its copies only.  h_offsets / h_lengths hold the batch's layout already.
+static int launch_chunked(wlm_plan* p, const void* const* clips_host, int pcm_format, size_t esz, int B, void* out_dev,
+                          cudaStream_t st) {
     WLM_CUDA(cudaMemcpyAsync(p->d_offsets, p->h_offsets, sizeof(int64_t) * B, cudaMemcpyHostToDevice, p->copy_stream));
     WLM_CUDA(cudaMemcpyAsync(p->d_lengths, p->h_lengths, sizeof(int32_t) * B, cudaMemcpyHostToDevice, p->copy_stream));
 
     // chunks of ~48 MB of PCM: copy chunk c+1 while the kernels of chunk c run
     const size_t kChunkBytes = 48u << 20;
-    const size_t kRingBytes = 64u << 20;
     int b0 = 0, chunk = 0, slot_uses[2] = {0, 0};
     while (b0 < B) {
         int b1 = b0;
@@ -456,11 +562,7 @@ extern "C" int wlm_logmel_host(wlm_plan* p, const void* const* clips_host, const
                 b = e;
             } else {
                 // pageable source: bounce through the pinned ring, as many clips as fit
-                if (!p->h_ring[0]) {
-                    WLM_CUDA(cudaMallocHost(&p->h_ring[0], kRingBytes));
-                    WLM_CUDA(cudaMallocHost(&p->h_ring[1], kRingBytes));
-                    p->h_ring_bytes = kRingBytes;
-                }
+                for (int r = 0; r < 2; ++r) WLM_CUDA(grow_buffer(&p->h_ring[r], &p->h_ring_bytes[r], kRingBytes, true));
                 const int slot = (slot_uses[0] + slot_uses[1]) & 1;
                 if (slot_uses[slot]) WLM_CUDA(cudaEventSynchronize(p->ev_slot_free[slot]));
                 char* ring = static_cast<char*>(p->h_ring[slot]);
@@ -470,7 +572,7 @@ extern "C" int wlm_logmel_host(wlm_plan* p, const void* const* clips_host, const
                 while (e < b1 && !is_pinned_host(clips_host[e] ? clips_host[e] : ring)) {
                     const size_t rel = (size_t)(p->h_offsets[e] - first_off) * esz;
                     const size_t nbytes = (size_t)p->h_lengths[e] * esz;
-                    if (rel + nbytes > p->h_ring_bytes) break;
+                    if (rel + nbytes > kRingBytes) break;
                     if (nbytes) memcpy(ring + rel, clips_host[e], nbytes);
                     used = rel + nbytes;
                     ++e;
@@ -493,6 +595,61 @@ extern "C" int wlm_logmel_host(wlm_plan* p, const void* const* clips_host, const
         b0 = b1;
         ++chunk;
     }
+    return WLM_OK;
+}
+
+extern "C" int wlm_logmel_host(wlm_plan* p, const void* const* clips_host, const int32_t* lengths_host,
+                               int pcm_format, int B, void* out_dev, void* out_host, void* stream) {
+    if (!p) return fail(WLM_ERR_BAD_ARG, "plan is NULL");
+    if (B < 0) return fail(WLM_ERR_BAD_ARG, "B=%d is negative", B);
+    if (B == 0) return WLM_OK;
+    if (!clips_host || !lengths_host || !out_dev) return fail(WLM_ERR_BAD_ARG, "clips_host/lengths_host/out_dev is NULL");
+    if (pcm_format != WLM_PCM_F32 && pcm_format != WLM_PCM_I16) return fail(WLM_ERR_BAD_ARG, "unknown pcm_format %d", pcm_format);
+    if (reinterpret_cast<uintptr_t>(out_dev) & 15) return fail(WLM_ERR_BAD_ARG, "out_dev must be 16-byte aligned");
+    WLM_CUDA(cudaSetDevice(p->device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const size_t esz = pcm_format == WLM_PCM_I16 ? 2 : 4;
+    const int64_t align_el = 16 / esz * 2;  // clip starts at 32-byte boundaries of the packed buffer
+
+    // a previous call's kernels may still be reading the staging buffers / metadata: wait before reusing or replacing them
+    if (p->kernels_done_valid) WLM_CUDA(cudaEventSynchronize(p->ev_kernels_done));
+    const size_t meta_n = std::max(B, 256);
+    WLM_CUDA(grow_buffer(&p->d_offsets, &p->d_offsets_bytes, sizeof(int64_t) * meta_n, false));
+    WLM_CUDA(grow_buffer(&p->d_lengths, &p->d_lengths_bytes, sizeof(int32_t) * meta_n, false));
+    WLM_CUDA(grow_buffer(&p->h_offsets, &p->h_offsets_bytes, sizeof(int64_t) * meta_n, true));
+    WLM_CUDA(grow_buffer(&p->h_lengths, &p->h_lengths_bytes, sizeof(int32_t) * meta_n, true));
+
+    int64_t total_el = 0;
+    for (int b = 0; b < B; ++b) {
+        if (lengths_host[b] < 0) return fail(WLM_ERR_BAD_ARG, "lengths_host[%d]=%d is negative", b, lengths_host[b]);
+        if (lengths_host[b] > 0 && !clips_host[b]) return fail(WLM_ERR_BAD_ARG, "clips_host[%d] is NULL", b);
+        const int32_t len = std::min<int32_t>(lengths_host[b], kNSamples);
+        p->h_offsets[b] = total_el;
+        p->h_lengths[b] = len;
+        total_el += (len + align_el - 1) / align_el * align_el;
+    }
+    WLM_CUDA(grow_buffer(&p->d_stage, &p->d_stage_bytes, std::max<size_t>((size_t)total_el * esz, 256), false));
+    WLM_CUDA(grow_buffer(&p->d_ws, &p->d_ws_bytes, wlm_workspace_bytes(p, B), false));
+    // Small pageable batches -- the reference's own call shape, ONE clip per call (REF/data_utils/data_loader.py:171):
+    // no ring bounce, no copy stream, no events.  cudaMemcpyAsync from pageable memory returns once the source has been
+    // staged by the driver, so the host buffers are reusable on return without any synchronisation here.
+    bool small_pageable = (size_t)total_el * esz <= (4u << 20);
+    for (int b = 0; small_pageable && b < B; ++b)
+        if (p->h_lengths[b] > 0 && is_pinned_host(clips_host[b])) small_pageable = false;
+    int rc;
+    if (small_pageable) {
+        for (int b = 0; b < B; ++b)
+            if (p->h_lengths[b] > 0)
+                WLM_CUDA(cudaMemcpyAsync(static_cast<char*>(p->d_stage) + p->h_offsets[b] * esz, clips_host[b],
+                                         (size_t)p->h_lengths[b] * esz, cudaMemcpyHostToDevice, st));
+        WLM_CUDA(cudaMemcpyAsync(p->d_offsets, p->h_offsets, sizeof(int64_t) * B, cudaMemcpyHostToDevice, st));
+        WLM_CUDA(cudaMemcpyAsync(p->d_lengths, p->h_lengths, sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
+        rc = launch_logmel(p, clip_args(p, p->d_stage, pcm_format, p->d_offsets, p->d_lengths, 0, B, out_dev,
+                                        static_cast<float*>(p->d_ws)), st);
+    } else {
+        rc = launch_chunked(p, clips_host, pcm_format, esz, B, out_dev, st);
+    }
+    if (rc != WLM_OK) return rc;
     WLM_CUDA(cudaEventRecord(p->ev_kernels_done, st));
     p->kernels_done_valid = true;
     if (out_host) {
@@ -500,8 +657,7 @@ extern "C" int wlm_logmel_host(wlm_plan* p, const void* const* clips_host, const
                                  cudaMemcpyDeviceToHost, st));
         WLM_CUDA(cudaStreamSynchronize(st));
     }
-    // host buffers must be reusable on return
-    WLM_CUDA(cudaStreamSynchronize(p->copy_stream));
+    // host buffers must be reusable on return: the chunked path's copies may still be in flight
+    if (!small_pageable) WLM_CUDA(cudaStreamSynchronize(p->copy_stream));
     return WLM_OK;
 }
-
