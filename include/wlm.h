@@ -168,6 +168,34 @@ int wlm_frame_mask(wlm_plan* plan, const int32_t* lengths_dev, int B, int32_t* m
                    void* stream);
 
 /*
+ * Long-form features (`truncation=False, padding="longest"` of TF-FE:189-342): every clip is
+ * zero-padded to ONE common length padded_len = L of any value (the longest clip of the batch,
+ * possibly rounded up by pad_to_multiple_of), reflected by 200 samples at sample 0 and at L
+ * (torch.stft center=True), and the last STFT frame is dropped: T = L / 160 frames.  The max - 8
+ * clamp uses each clip's maximum over all its T frames.
+ *
+ *   pcm_dev ... stream  as wlm_logmel; clip b contributes min(lengths_dev[b], padded_len) samples
+ *                       (dense layout without lengths: min(row_stride, padded_len)).
+ *   padded_len          L, in [201, INT32_MAX]; otherwise WLM_ERR_BAD_ARG.
+ *   out_dev             device [B][n_mels][L / 160] of the plan's output format, 16-byte aligned (rows
+ *                       are L / 160 elements, so they need not be aligned).
+ *   workspace           device scratch of at least wlm_padded_workspace_bytes(plan, B) bytes, 16-byte
+ *                       aligned; always required (it holds the per-clip maxima and a work counter).
+ * At padded_len = 480000 the features and gmax equal those of wlm_logmel bit for bit.
+ */
+size_t wlm_padded_workspace_bytes(const wlm_plan* plan, int B);
+int wlm_logmel_padded(wlm_plan* plan, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
+                      const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B, void* out_dev,
+                      float* gmax_dev, void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * Attention mask of the long-form call: int32 [B][padded_len / 160], 1 where 160*t < min(len, padded_len)
+ * (TF-FE:328-337, including the trim of the last column when padded_len % 160 != 0).
+ */
+int wlm_frame_mask_padded(wlm_plan* plan, const int32_t* lengths_dev, int B, int64_t padded_len,
+                          int32_t* mask_dev, void* stream);
+
+/*
  * End-to-end convenience with HOST buffers (what the reference-facing Python shim calls for
  * numpy inputs): stages the ragged host clips through the plan's pinned ring, copies H2D in
  * chunks on an internal copy stream overlapped with the kernels, and leaves the features on

@@ -42,6 +42,9 @@ SYMBOLS = {
     "wlm_plan_set_output_format": (_i, [_vp, _i]),
     "wlm_plan_output_format": (_i, [_vp]),
     "wlm_plan_set_flat_clips": (_i, [_vp, _i]),
+    "wlm_padded_workspace_bytes": (_sz, [_vp, _i]),
+    "wlm_logmel_padded": (_i, [_vp, _vp, _i, _vp, _vp, _i64, _i64, _i, _vp, _vp, _vp, _sz, _vp]),
+    "wlm_frame_mask_padded": (_i, [_vp, _vp, _i, _i64, _vp, _vp]),
 }
 
 

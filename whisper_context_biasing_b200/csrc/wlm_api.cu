@@ -16,6 +16,7 @@
 #include <vector>
 
 #include "logmel_fused.cuh"
+#include "logmel_long.cuh"
 #include "wlm_common.cuh"
 
 using namespace wlm;
@@ -72,6 +73,27 @@ static KernelFn kernel_for(int variant, bool flat, int out_format, bool dyn) {
     return kernel_for_t<float, false>(variant, flat);
 }
 
+typedef void (*LongKernelFn)(const longform::LongArgs, const fused::KernelTables, const float*);
+typedef void (*ClampKernelFn)(const longform::LongArgs);
+
+template <class OutT>
+static LongKernelFn long_kernel_for_t(int variant) {
+    using longform::logmel_long_kernel;
+    if (variant == 80) return logmel_long_kernel<80, OutT>;
+    if (variant == 128) return logmel_long_kernel<128, OutT>;
+    return logmel_long_kernel<0, OutT>;
+}
+static LongKernelFn long_kernel_for(int variant, int out_format) {
+    if (out_format == WLM_OUT_BF16) return long_kernel_for_t<__nv_bfloat16>(variant);
+    if (out_format == WLM_OUT_F16) return long_kernel_for_t<__half>(variant);
+    return long_kernel_for_t<float>(variant);
+}
+static ClampKernelFn clamp_kernel_for(int out_format) {
+    if (out_format == WLM_OUT_BF16) return longform::logmel_long_clamp_kernel<__nv_bfloat16>;
+    if (out_format == WLM_OUT_F16) return longform::logmel_long_clamp_kernel<__half>;
+    return longform::logmel_long_clamp_kernel<float>;
+}
+
 // launch configuration of the cluster kernel; the flat kernel uses the same one without the cluster dimension (at[0])
 static void fill_launch_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* at, int n_clusters, cudaStream_t st) {
     memset(cfg, 0, sizeof(*cfg));
@@ -98,6 +120,10 @@ static cudaError_t configure(int variant, int* max_clusters) {
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, fused::kSmemBytes);
             if (e != cudaSuccess) return e;
         }
+    for (int fmt : {WLM_OUT_F32, WLM_OUT_BF16, WLM_OUT_F16}) {
+        e = cudaFuncSetAttribute(long_kernel_for(variant, fmt), cudaFuncAttributeMaxDynamicSharedMemorySize, fused::kSmemBytes);
+        if (e != cudaSuccess) return e;
+    }
     cudaLaunchConfig_t cfg;
     cudaLaunchAttribute at[2];
     fill_launch_config(&cfg, at, 148, nullptr);
@@ -474,25 +500,117 @@ extern "C" int wlm_logmel(wlm_plan* p, const void* pcm_dev, int pcm_format, cons
 // ------------------------------------------------------------------------------------------
 // attention mask (TF-FE:328-337)
 // ------------------------------------------------------------------------------------------
-__global__ void frame_mask_kernel(const int32_t* __restrict__ lengths, int B, int32_t* __restrict__ mask) {
-    const int64_t total = (int64_t)B * kNFrames;
+// [B][n_frames] of clips padded (or trimmed) to n_samples: 1 where 160 t < min(len, n_samples)
+__global__ void frame_mask_kernel(const int32_t* __restrict__ lengths, int B, int n_frames, int n_samples,
+                                  int32_t* __restrict__ mask) {
+    const int64_t total = (int64_t)B * n_frames;
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        const int b = (int)(i / kNFrames), t = (int)(i - (int64_t)b * kNFrames);
-        const int len = max(0, min(lengths[b], kNSamples));
+        const int b = (int)(i / n_frames), t = (int)(i - (int64_t)b * n_frames);
+        const int len = max(0, min(lengths[b], n_samples));
         mask[i] = (t * kHop < len) ? 1 : 0;
     }
+}
+
+static int launch_frame_mask(wlm_plan* p, const int32_t* lengths_dev, int B, int n_frames, int n_samples, int32_t* mask_dev,
+                             void* stream) {
+    if (!lengths_dev || !mask_dev) return fail(WLM_ERR_BAD_ARG, "lengths_dev/mask_dev is NULL");
+    WLM_CUDA(cudaSetDevice(p->device));
+    const int64_t total = (int64_t)B * n_frames;
+    const int blocks = (int)std::min<int64_t>((total + 255) / 256, (int64_t)p->sm_count * 8);
+    frame_mask_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(lengths_dev, B, n_frames, n_samples, mask_dev);
+    p->launches += 1;
+    WLM_CUDA(cudaGetLastError());
+    return WLM_OK;
 }
 
 extern "C" int wlm_frame_mask(wlm_plan* p, const int32_t* lengths_dev, int B, int32_t* mask_dev, void* stream) {
     if (!p) return fail(WLM_ERR_BAD_ARG, "plan is NULL");
     if (B < 0) return fail(WLM_ERR_BAD_ARG, "B=%d is negative", B);
     if (B == 0) return WLM_OK;
-    if (!lengths_dev || !mask_dev) return fail(WLM_ERR_BAD_ARG, "lengths_dev/mask_dev is NULL");
+    return launch_frame_mask(p, lengths_dev, B, kNFrames, kNSamples, mask_dev, stream);
+}
+
+// torch.stft(center=True) needs more than n_fft / 2 samples to reflect; the frame index 160 t stays in int32
+static int check_padded_len(int64_t padded_len) {
+    if (padded_len <= kNfft / 2 || padded_len > INT32_MAX)
+        return fail(WLM_ERR_BAD_ARG, "padded_len=%lld outside [%d, %d]", (long long)padded_len, kNfft / 2 + 1, INT32_MAX);
+    return WLM_OK;
+}
+
+extern "C" int wlm_frame_mask_padded(wlm_plan* p, const int32_t* lengths_dev, int B, int64_t padded_len, int32_t* mask_dev,
+                                     void* stream) {
+    if (!p) return fail(WLM_ERR_BAD_ARG, "plan is NULL");
+    if (B < 0) return fail(WLM_ERR_BAD_ARG, "B=%d is negative", B);
+    if (check_padded_len(padded_len) != WLM_OK) return WLM_ERR_BAD_ARG;
+    if (B == 0) return WLM_OK;
+    return launch_frame_mask(p, lengths_dev, B, (int)(padded_len / kHop), (int)padded_len, mask_dev, stream);
+}
+
+// ------------------------------------------------------------------------------------------
+// long-form features: any padded length (logmel_long.cuh)
+// ------------------------------------------------------------------------------------------
+// workspace: the per-clip maximum of the mel power, then the unit counter
+static size_t padded_max_bytes(int B) { return ((size_t)B * sizeof(int) + 255) / 256 * 256; }
+
+extern "C" size_t wlm_padded_workspace_bytes(const wlm_plan* p, int B) {
+    if (!p || B <= 0) return 0;
+    return padded_max_bytes(B) + 256;
+}
+
+extern "C" int wlm_logmel_padded(wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
+                                 const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B, void* out_dev,
+                                 float* gmax_dev, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!p) return fail(WLM_ERR_BAD_ARG, "plan is NULL");
+    if (B < 0) return fail(WLM_ERR_BAD_ARG, "B=%d is negative", B);
+    if (check_padded_len(padded_len) != WLM_OK) return WLM_ERR_BAD_ARG;
+    if (B == 0) return WLM_OK;
+    if (!pcm_dev || !out_dev) return fail(WLM_ERR_BAD_ARG, "pcm_dev/out_dev is NULL");
+    if (pcm_format != WLM_PCM_F32 && pcm_format != WLM_PCM_I16) return fail(WLM_ERR_BAD_ARG, "unknown pcm_format %d", pcm_format);
+    if ((reinterpret_cast<uintptr_t>(pcm_dev) & 15) || (reinterpret_cast<uintptr_t>(out_dev) & 15))
+        return fail(WLM_ERR_BAD_ARG, "pcm_dev and out_dev must be 16-byte aligned");
+    if (!offsets_dev) {
+        if (row_stride <= 0) return fail(WLM_ERR_BAD_ARG, "dense layout needs row_stride > 0 (got %lld)", (long long)row_stride);
+        const int gran = pcm_format == WLM_PCM_I16 ? 8 : 4;
+        if (row_stride % gran)
+            return fail(WLM_ERR_BAD_ARG, "dense row_stride must be a multiple of %d elements (16 bytes), got %lld", gran, (long long)row_stride);
+    } else if (!lengths_dev) {
+        return fail(WLM_ERR_BAD_ARG, "ragged layout (offsets_dev) needs lengths_dev");
+    }
+    const size_t need = wlm_padded_workspace_bytes(p, B);
+    if (!workspace || workspace_bytes < need)
+        return fail(WLM_ERR_WORKSPACE, "workspace %zu B < required %zu B", workspace_bytes, need);
+    if (reinterpret_cast<uintptr_t>(workspace) & 15) return fail(WLM_ERR_BAD_ARG, "workspace must be 16-byte aligned");
     WLM_CUDA(cudaSetDevice(p->device));
-    const int64_t total = (int64_t)B * kNFrames;
-    const int blocks = (int)std::min<int64_t>((total + 255) / 256, (int64_t)p->sm_count * 8);
-    frame_mask_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(lengths_dev, B, mask_dev);
-    p->launches += 1;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+
+    longform::LongArgs a{};
+    a.pcm = pcm_dev;
+    a.offsets = offsets_dev;
+    a.lengths = lengths_dev;
+    a.row_stride = offsets_dev ? 0 : row_stride;
+    a.padded_len = (int32_t)padded_len;
+    a.n_frames = (int32_t)(padded_len / kHop);
+    a.n_tiles = (a.n_frames + fused::kTile - 1) / fused::kTile;
+    a.units_per_clip = (a.n_tiles + longform::kLongRun - 1) / longform::kLongRun;
+    a.pcm_format = pcm_format;
+    a.n_mels = p->n_mels;
+    a.B = B;
+    a.out = out_dev;
+    a.gmax = gmax_dev;
+    a.pmax = static_cast<int*>(workspace);
+    a.next_unit = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + padded_max_bytes(B));
+
+    // plain launches in stream order: pass 1 starts after everything before it, pass 2 after pass 1
+    WLM_CUDA(cudaMemsetAsync(workspace, 0, need, st));
+    const int64_t units = (int64_t)B * a.units_per_clip;
+    const int ctas = (int)std::min<int64_t>(p->sm_count, (units + fused::kGroups - 1) / fused::kGroups);
+    long_kernel_for(p->variant, p->out_format)<<<ctas, fused::kThreads, fused::kSmemBytes, st>>>(a, p->mel, p->d_win_lane);
+    WLM_CUDA(cudaGetLastError());
+    const int64_t vecs = ((int64_t)a.n_mels * a.n_frames * (int64_t)out_elem_size(p) + 15) / 16;
+    const int gy = std::min(B, 65535);
+    const int gx = (int)std::max<int64_t>(1, std::min<int64_t>((vecs + 1023) / 1024, std::max(1, 8 * p->sm_count / gy)));
+    clamp_kernel_for(p->out_format)<<<dim3(gx, gy), 256, 0, st>>>(a);
+    p->launches += 2;
     WLM_CUDA(cudaGetLastError());
     return WLM_OK;
 }

@@ -62,6 +62,16 @@ def slaney_mel_filters(n_mels: int, n_freq: int = 1 + N_FFT // 2, sampling_rate:
     return tri * (2.0 / (edges[2:n_mels + 2] - edges[:n_mels]))[None, :]
 
 
+def padded_length(lengths, pad_to_multiple_of=None) -> int:
+    """Common length L of a `padding="longest", truncation=False` batch, as `SequenceFeatureExtractor.pad` computes
+    it (TF-SU:51-219, `_pad`): the longest clip, rounded up to a multiple of `pad_to_multiple_of` when given.
+    `max_length` plays no part.  The features then have L // 160 frames."""
+    L = max((int(n) for n in lengths), default=0)
+    if pad_to_multiple_of is not None and L % pad_to_multiple_of != 0:
+        L = (L // pad_to_multiple_of + 1) * pad_to_multiple_of
+    return L
+
+
 class LogMelBatch(dict):
     """dict with attribute access, like `BatchFeature.__getattr__`
     (feature_extraction_utils.py:95-99): `out.input_features`, `out["input_features"]`, item
@@ -196,33 +206,36 @@ class B200WhisperFeatureExtractor:
         N.check(N.LIB.wlm_plan_set_flat_clips(self._plan, int(n)))
 
     # -- helpers -----------------------------------------------------------------------------
-    def _check_out(self, out, B):
-        if (tuple(out.shape) != (B, self.feature_size, self.nb_max_frames) or out.dtype != self.feature_dtype
+    def _check_out(self, out, B, n_frames=None):
+        n_frames = self.nb_max_frames if n_frames is None else n_frames
+        if (tuple(out.shape) != (B, self.feature_size, n_frames) or out.dtype != self.feature_dtype
                 or not out.is_cuda or out.device != self.device or not out.is_contiguous()):
             raise ValueError(f"out must be a contiguous {self.feature_dtype} tensor [B={B}, {self.feature_size}, "
-                             f"{self.nb_max_frames}] on {self.device}")
+                             f"{n_frames}] on {self.device}")
 
     def _stream(self):
         import torch
 
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
-    def _workspace(self, B):
+    def _workspace(self, B, padded=False):
         import torch
 
-        need = int(N.LIB.wlm_workspace_bytes(self._plan, B))
+        need = int((N.LIB.wlm_padded_workspace_bytes if padded else N.LIB.wlm_workspace_bytes)(self._plan, B))
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(max(need, 256), dtype=torch.uint8, device=self.device)
         return self._ws, need
 
     # -- device-resident entry points (new; the reference has no device path) -------------------
-    def extract_device(self, pcm, lengths=None, offsets=None, out=None, return_gmax=False):
+    def extract_device(self, pcm, lengths=None, offsets=None, out=None, return_gmax=False, padded_len=None):
         """PCM already in HBM -> features in HBM.
 
         pcm      CUDA tensor, float32 or int16 (int16 is scaled by 1/32768 on the GPU).
                  dense: [B, L] (row stride L, L % 4 == 0); ragged: 1-D with `offsets`/`lengths`.
         lengths  optional int32 CUDA tensor [B] of valid samples (required when ragged).
         offsets  optional int64 CUDA tensor [B] of clip starts (elements) in the 1-D buffer.
+        padded_len  None: every clip is padded / trimmed to 30 s, features [B, M, 3000].  An int L > 200: every
+                 clip is zero-padded to L samples (long-form, `truncation=False`), features [B, M, L // 160].
         """
         import torch
 
@@ -252,33 +265,47 @@ class B200WhisperFeatureExtractor:
                 raise ValueError("offsets must be a CUDA int64 tensor")
         if lengths is not None and (lengths.dtype != torch.int32 or not lengths.is_cuda or lengths.shape[0] != B):
             raise ValueError("lengths must be a CUDA int32 tensor of shape [B]")
+        if padded_len is not None:
+            padded_len = int(padded_len)
+            if padded_len <= N_FFT // 2:
+                raise ValueError(f"padded_len={padded_len}: the reflect padding of the STFT needs more than "
+                                 f"{N_FFT // 2} samples")
+        n_frames = self.nb_max_frames if padded_len is None else padded_len // self.hop_length
         if out is None:
-            out = torch.empty((B, self.feature_size, self.nb_max_frames), dtype=self.feature_dtype, device=self.device)
+            out = torch.empty((B, self.feature_size, n_frames), dtype=self.feature_dtype, device=self.device)
         else:
-            self._check_out(out, B)
+            self._check_out(out, B, n_frames)
         gmax = torch.empty((max(B, 1),), dtype=torch.float32, device=self.device) if return_gmax else None
-        ws, need = self._workspace(B)
+        ws, need = self._workspace(B, padded=padded_len is not None)
         if B:
-            with torch.cuda.device(self.device):
-                N.check(N.LIB.wlm_logmel(
-                    self._plan, C.c_void_p(pcm.data_ptr()), fmt,
+            args = (C.c_void_p(pcm.data_ptr()), fmt,
                     C.c_void_p(offsets.data_ptr()) if offsets is not None else None,
-                    C.c_void_p(lengths.data_ptr()) if lengths is not None else None,
-                    stride, B, C.c_void_p(out.data_ptr()),
-                    C.c_void_p(gmax.data_ptr()) if gmax is not None else None,
-                    C.c_void_p(ws.data_ptr()), need, self._stream()))
+                    C.c_void_p(lengths.data_ptr()) if lengths is not None else None, stride)
+            tail = (B, C.c_void_p(out.data_ptr()), C.c_void_p(gmax.data_ptr()) if gmax is not None else None,
+                    C.c_void_p(ws.data_ptr()), need, self._stream())
+            with torch.cuda.device(self.device):
+                if padded_len is None:
+                    N.check(N.LIB.wlm_logmel(self._plan, *args, *tail))
+                else:
+                    N.check(N.LIB.wlm_logmel_padded(self._plan, *args, padded_len, *tail))
         return (out, gmax[:B]) if return_gmax else out
 
-    def frame_mask_device(self, lengths):
-        """int32 [B, 3000] attention mask on the device (TF-FE:328-337)."""
+    def frame_mask_device(self, lengths, padded_len=None):
+        """int32 [B, 3000] attention mask on the device (TF-FE:328-337); with `padded_len` = L the long-form
+        mask [B, L // 160]."""
         import torch
 
         B = lengths.shape[0]
-        mask = torch.empty((B, self.nb_max_frames), dtype=torch.int32, device=self.device)
-        if B:
-            with torch.cuda.device(self.device):
-                N.check(N.LIB.wlm_frame_mask(self._plan, C.c_void_p(lengths.data_ptr()), B,
-                                             C.c_void_p(mask.data_ptr()), self._stream()))
+        n_frames = self.nb_max_frames if padded_len is None else int(padded_len) // self.hop_length
+        mask = torch.empty((B, max(n_frames, 0)), dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            if padded_len is None:
+                if B:
+                    N.check(N.LIB.wlm_frame_mask(self._plan, C.c_void_p(lengths.data_ptr()), B,
+                                                 C.c_void_p(mask.data_ptr()), self._stream()))
+            else:
+                N.check(N.LIB.wlm_frame_mask_padded(self._plan, C.c_void_p(lengths.data_ptr()), B, int(padded_len),
+                                                    C.c_void_p(mask.data_ptr()), self._stream()))
         return mask
 
     def extract_host(self, clips, out=None, out_host=None):
@@ -360,18 +387,22 @@ class B200WhisperFeatureExtractor:
             logger.warning(
                 f"It is strongly recommended to pass the `sampling_rate` argument to `{self.__class__.__name__}()`. "
                 "Failing to do so can result in silent errors that might be hard to debug.")
-        if padding != "max_length" or (max_length not in (None, self.n_samples)) or not truncation \
-                or pad_to_multiple_of is not None:
+        longform = padding == "longest" and truncation is False      # max_length is ignored, as TF-SU:51-219 does
+        if not longform and (padding != "max_length" or (max_length not in (None, self.n_samples)) or not truncation
+                             or pad_to_multiple_of is not None):
             raise NotImplementedError(
-                "only the reference's argument combination is implemented: padding='max_length', "
-                "max_length=None (30 s), truncation=True, pad_to_multiple_of=None")
+                "implemented argument combinations: padding='max_length', max_length=None (30 s), truncation=True, "
+                "pad_to_multiple_of=None (the reference's), and padding='longest', truncation=False (long-form)")
         if do_normalize:
             raise NotImplementedError("do_normalize=True is not used by the reference and not implemented")
         if device not in (None, "cpu") and torch.device(device).type != "cuda":
             raise NotImplementedError(f"device={device!r}: features are always computed on {self.device}")
 
         lengths_np = None
-        if isinstance(raw_speech, torch.Tensor):
+        n_samples = self.n_samples                                          # samples every clip is padded to
+        if longform:
+            feats, lengths_np, n_samples = self._call_longform(raw_speech, pad_to_multiple_of)
+        elif isinstance(raw_speech, torch.Tensor):
             if raw_speech.dim() > 2:
                 raise ValueError(f"Only mono-channel audio is supported for input to {self}")
             x = raw_speech if raw_speech.dim() == 2 else raw_speech[None]
@@ -387,16 +418,7 @@ class B200WhisperFeatureExtractor:
                 feats = self.extract_host(clips)
                 lengths_np = np.array([min(c.shape[0], self.n_samples) for c in clips], dtype=np.int32)
         else:
-            is_batched_numpy = isinstance(raw_speech, np.ndarray) and raw_speech.ndim > 1      # TF-FE:274
-            if is_batched_numpy and raw_speech.ndim > 2:
-                raise ValueError(f"Only mono-channel audio is supported for input to {self}")  # TF-FE:275-276
-            is_batched = is_batched_numpy or (
-                isinstance(raw_speech, (list, tuple)) and len(raw_speech) > 0
-                and isinstance(raw_speech[0], (np.ndarray, tuple, list)))                       # TF-FE:277-279
-            if is_batched:                                                                     # TF-FE:281-282
-                clips = [np.ascontiguousarray(np.asarray(s, dtype=np.float32).reshape(-1)) for s in raw_speech]
-            else:                                                                              # TF-FE:283-290
-                clips = [np.ascontiguousarray(np.asarray(raw_speech, dtype=np.float32).reshape(-1))]
+            clips = self._host_clips(raw_speech)
             feats = self.extract_host(clips)
             lengths_np = np.array([min(c.shape[0], self.n_samples) for c in clips], dtype=np.int32)
 
@@ -413,15 +435,74 @@ class B200WhisperFeatureExtractor:
             raise NotImplementedError(f"return_tensors={return_tensors!r} (use None, 'pt' or 'np')")
         if return_attention_mask:                                                              # TF-FE:328-337
             lens_dev = torch.from_numpy(lengths_np).to(self.device)
-            mask = self.frame_mask_device(lens_dev)
+            mask = self.frame_mask_device(lens_dev, padded_len=n_samples if longform else None)
             out["attention_mask"] = mask.cpu().numpy() if want == "np" else mask
         elif return_attention_mask is None and self.return_attention_mask:
             # The reference's quirk, kept: pad() falls back to the ctor attribute (TF-SU:135-137) and returns the
-            # SAMPLE-level mask [B, 480000], which TF-FE:328 then does not rescale because the call argument is None.
+            # SAMPLE-level mask [B, 480000] (long-form: [B, L]), which TF-FE:328 then does not rescale because the
+            # call argument is None.
             lens_dev = torch.from_numpy(lengths_np).to(self.device)
-            mask = (torch.arange(self.n_samples, device=self.device, dtype=torch.int32)[None, :] < lens_dev[:, None]).to(torch.int32)
+            mask = (torch.arange(n_samples, device=self.device, dtype=torch.int32)[None, :] < lens_dev[:, None]).to(torch.int32)
             out["attention_mask"] = mask.cpu().numpy() if want == "np" else mask
         return out
+
+    def _call_longform(self, raw_speech, pad_to_multiple_of):
+        """`truncation=False, padding="longest"`: every clip is zero-padded to L = padded_length(...) samples.
+        A CUDA tensor goes to the kernels as it is (dense rows); host input is packed into one pinned buffer, clip
+        starts 16-byte aligned, copied over in one transfer and run as a ragged batch.
+        Returns (features [B, M, L // 160], int32 lengths, L)."""
+        import torch
+
+        if isinstance(raw_speech, torch.Tensor):
+            if raw_speech.dim() > 2:
+                raise ValueError(f"Only mono-channel audio is supported for input to {self}")
+            x = raw_speech if raw_speech.dim() == 2 else raw_speech[None]
+            if x.dtype != torch.float32:
+                x = x.to(torch.float32)
+            if x.is_cuda:
+                B, n = x.shape
+                L = padded_length([n] * B, pad_to_multiple_of)
+                self._check_padded_len(L)
+                if n % 4:          # rows must start on 16-byte boundaries; the padding is zeros, as HF pads
+                    x = torch.nn.functional.pad(x, (0, 4 - n % 4))
+                return self.extract_device(x, padded_len=L), np.full((B,), n, dtype=np.int32), L
+            clips = [r.numpy() for r in x]
+        else:
+            clips = self._host_clips(raw_speech)
+        lens = np.array([c.shape[0] for c in clips], dtype=np.int64)
+        L = padded_length(lens, pad_to_multiple_of)
+        self._check_padded_len(L)
+        starts = (lens + 3) // 4 * 4                       # 16-byte aligned clip starts
+        offs = np.concatenate([[0], np.cumsum(starts)[:-1]]).astype(np.int64)
+        host = torch.empty(int(starts.sum()) + 4, dtype=torch.float32, pin_memory=True)
+        h = host.numpy()
+        for o, c in zip(offs, clips):
+            h[o:o + c.shape[0]] = c
+        pcm = host.to(self.device, non_blocking=True)     # (the caching host allocator keeps `host` until the copy is done)
+        lens32 = lens.astype(np.int32)
+        feats = self.extract_device(pcm, lengths=torch.from_numpy(lens32).to(self.device),
+                                    offsets=torch.from_numpy(offs).to(self.device), padded_len=L)
+        return feats, lens32, L
+
+    def _host_clips(self, raw_speech):
+        """numpy / list input -> list of contiguous float32 1-D clips"""
+        is_batched_numpy = isinstance(raw_speech, np.ndarray) and raw_speech.ndim > 1          # TF-FE:274
+        if is_batched_numpy and raw_speech.ndim > 2:
+            raise ValueError(f"Only mono-channel audio is supported for input to {self}")      # TF-FE:275-276
+        is_batched = is_batched_numpy or (
+            isinstance(raw_speech, (list, tuple)) and len(raw_speech) > 0
+            and isinstance(raw_speech[0], (np.ndarray, tuple, list)))                           # TF-FE:277-279
+        if is_batched:                                                                         # TF-FE:281-282
+            return [np.ascontiguousarray(np.asarray(s, dtype=np.float32).reshape(-1)) for s in raw_speech]
+        return [np.ascontiguousarray(np.asarray(raw_speech, dtype=np.float32).reshape(-1))]   # TF-FE:283-290
+
+    @staticmethod
+    def _check_padded_len(L):
+        if L <= N_FFT // 2:
+            raise ValueError(f"the longest clip has {L} samples: the reflect padding of the STFT needs more than "
+                             f"{N_FFT // 2} (torch.stft refuses it too)")
+        if L >= 2 ** 31:
+            raise ValueError(f"padded length {L} does not fit 32 bits")
 
     # -- the collator's stack (REF/data_utils/data_collator.py:64-76) --------------------------
     def pad(self, processed_features, padding="longest", max_length=None, truncation=False,
