@@ -80,7 +80,7 @@ const char* wlm_last_error(void);
 
 /*
  * Replaces WhisperFeatureExtractor.__init__ (TF-FE:69-103): fixes n_fft=400, hop=160,
- * 30 s chunks, padding_value 0.0, dither 0.0 and takes the mel table the constructor builds.
+ * 30 s chunks, padding_value 0.0 (dither is an argument of wlm_logmel_conditioned) and takes the mel table the constructor builds.
  *
  *   device              CUDA ordinal
  *   n_mels              feature_size (80 whisper-base/small, 128 large-v3)
@@ -187,6 +187,36 @@ size_t wlm_padded_workspace_bytes(const wlm_plan* plan, int B);
 int wlm_logmel_padded(wlm_plan* plan, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
                       const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B, void* out_dev,
                       float* gmax_dev, void* workspace, size_t workspace_bytes, void* stream);
+
+/*
+ * The two waveform steps HF runs between padding and the STFT, for the long-form geometry and (with
+ * padded_len = 480000) the 30-s one: `do_normalize=True` of TF-FE:189-342 (zero_mean_unit_var_norm
+ * with the pad's mask) and the constructor's `dither` (TF-FE:141-161 adds dither * randn to the
+ * whole padded waveform before torch.stft reflects it).  For clip b with n_b = min(len_b, L) valid
+ * samples, in this order:
+ *   1. do_normalize != 0: y = (x - mean) / sqrt(var + 1e-7) on [0, n_b), mean and population
+ *      variance of x[:n_b] (x = pcm, or int16 / 32768); an empty clip stays zero;
+ *   2. y = 0 on [n_b, L);
+ *   3. y[n] += dither * z(seed, b, n) on [0, L), the pad region included;
+ *   4. reflection at 0 and at L of the conditioned y, then the STFT etc. as wlm_logmel_padded.
+ * The noise z is not torch.randn's; it is this stream, independent of B, the layout, the formats
+ * and the work split (b is the clip's index in the call):
+ *   Philox4x32-10 (Random123) with key (lo32(seed), hi32(seed)) and counter (n >> 2, b, 0, 0)
+ *   gives words r0..r3; u_i = ((r_i >> 8) + 0.5) * 2^-24;
+ *   (z0, z1) = sqrt(-2 ln u0) * (cos 2 pi u1, sin 2 pi u1), (z2, z3) likewise from (u2, u3);
+ *   sample n takes z_{n & 3}.
+ * The per-clip moments are reduced in a fixed order: repeated calls give bit-identical results.
+ *
+ *   arguments and errors as wlm_logmel_padded; in addition a non-finite dither is WLM_ERR_BAD_ARG.
+ *   workspace     at least wlm_conditioned_workspace_bytes(plan, B, padded_len) bytes, 16-byte aligned
+ *                 (0 when padded_len is out of range).
+ * With do_normalize = 0 and dither = 0 the results equal wlm_logmel_padded's bit for bit.
+ */
+size_t wlm_conditioned_workspace_bytes(const wlm_plan* plan, int B, int64_t padded_len);
+int wlm_logmel_conditioned(wlm_plan* plan, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
+                           const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B,
+                           int do_normalize, float dither, uint64_t seed,
+                           void* out_dev, float* gmax_dev, void* workspace, size_t workspace_bytes, void* stream);
 
 /*
  * Attention mask of the long-form call: int32 [B][padded_len / 160], 1 where 160*t < min(len, padded_len)

@@ -45,6 +45,9 @@ SYMBOLS = {
     "wlm_padded_workspace_bytes": (_sz, [_vp, _i]),
     "wlm_logmel_padded": (_i, [_vp, _vp, _i, _vp, _vp, _i64, _i64, _i, _vp, _vp, _vp, _sz, _vp]),
     "wlm_frame_mask_padded": (_i, [_vp, _vp, _i, _i64, _vp, _vp]),
+    "wlm_conditioned_workspace_bytes": (_sz, [_vp, _i, _i64]),
+    "wlm_logmel_conditioned": (_i, [_vp, _vp, _i, _vp, _vp, _i64, _i64, _i, _i, C.c_float, C.c_uint64, _vp, _vp, _vp, _sz,
+                                    _vp]),
 }
 
 

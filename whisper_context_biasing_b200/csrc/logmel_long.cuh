@@ -19,6 +19,10 @@
 // At L = 480000 both passes reproduce wlm_logmel bit for bit: the raw buffer holds the same values (same
 // reflection and zero fill), stages 1/2 and the mel stage are the same code, and the clamp is the flat
 // kernel's.
+//
+// A conditioned call (wlm_logmel_conditioned: do_normalize, dither) runs logmel_long_cond_kernel, the same pass 1
+// with cond_fixup on every half-tile, and, for do_normalize, the per-clip moments kernels before it.  Pass 2 is
+// unchanged.
 #pragma once
 #include "logmel_fused.cuh"
 
@@ -110,34 +114,38 @@ __device__ __forceinline__ void long_issue_tma(const LongArgs& a, const LongClip
     }
 }
 
-// int16 -> float32 expansion in place (as fused::tile_fixup), then every position outside [0, len) of the half-tile:
-// reflection at sample 0 (s < 0 -> -s), reflection at L (s >= L -> 2 (L - 1) - s; torch.stft center=True pads the
-// L-sample array at both ends), zero padding in [len, L).  A reflected position only reads samples inside [0, len),
-// which nobody patches; positions whose reflection falls outside the half-tile belong to frames >= T (never stored).
+// int16 -> float32 expansion in place (as fused::tile_fixup).  Runs on the 256 threads of one group.
+__device__ __forceinline__ void long_expand_i16(float* raw, int grp, int tg) {
+    using fused::group_sync;
+    const int16_t* st = reinterpret_cast<const int16_t*>(raw + kSubLen);
+    constexpr float kScale = 1.0f / 32768.0f;
+    constexpr int kPer = (kSubLen + kGroupThreads - 1) / kGroupThreads;
+#pragma unroll 1
+    for (int i = tg; i < kSubLen; i += kGroupThreads) raw[i] = static_cast<float>(st[i]) * kScale;
+    float tmp[kPer];
+#pragma unroll
+    for (int j = 0; j < kPer; ++j) {
+        const int i = tg + j * kGroupThreads;
+        tmp[j] = i < kSubLen ? static_cast<float>(st[kSubLen + i]) * kScale : 0.f;
+    }
+    group_sync(grp);
+#pragma unroll
+    for (int j = 0; j < kPer; ++j) {
+        const int i = tg + j * kGroupThreads;
+        if (i < kSubLen) raw[kSubLen + i] = tmp[j];
+    }
+    group_sync(grp);
+}
+
+// int16 expansion, then every position outside [0, len) of the half-tile: reflection at sample 0 (s < 0 -> -s),
+// reflection at L (s >= L -> 2 (L - 1) - s; torch.stft center=True pads the L-sample array at both ends), zero padding in
+// [len, L).  A reflected position only reads samples inside [0, len), which nobody patches; positions whose reflection
+// falls outside the half-tile belong to frames >= T (never stored).
 // Runs on the 256 threads of one group; the condition for calling it is group-uniform.
 __device__ __forceinline__ void long_fixup(int pcm_format, int64_t len, int64_t L, int tile, float* raw, int grp, int tg) {
     using fused::group_sync;
     const int64_t s0 = long_s0(tile);
-    if (pcm_format == WLM_PCM_I16) {
-        const int16_t* st = reinterpret_cast<const int16_t*>(raw + kSubLen);
-        constexpr float kScale = 1.0f / 32768.0f;
-        constexpr int kPer = (kSubLen + kGroupThreads - 1) / kGroupThreads;
-#pragma unroll 1
-        for (int i = tg; i < kSubLen; i += kGroupThreads) raw[i] = static_cast<float>(st[i]) * kScale;
-        float tmp[kPer];
-#pragma unroll
-        for (int j = 0; j < kPer; ++j) {
-            const int i = tg + j * kGroupThreads;
-            tmp[j] = i < kSubLen ? static_cast<float>(st[kSubLen + i]) * kScale : 0.f;
-        }
-        group_sync(grp);
-#pragma unroll
-        for (int j = 0; j < kPer; ++j) {
-            const int i = tg + j * kGroupThreads;
-            if (i < kSubLen) raw[kSubLen + i] = tmp[j];
-        }
-        group_sync(grp);
-    }
+    if (pcm_format == WLM_PCM_I16) long_expand_i16(raw, grp, tg);
     if (s0 < 0 || s0 + kTileSamples > len) {
 #pragma unroll 1
         for (int r = 0; r < 2; ++r) {
@@ -159,11 +167,191 @@ __device__ __forceinline__ void long_fixup(int pcm_format, int64_t len, int64_t 
     }
 }
 
+// ---- conditioning: do_normalize and dither (wlm_logmel_conditioned) ----------------------------------------------
+struct CondArgs {
+    const float2* moments;   // [B] (mean, 1 / sqrt(var + 1e-7)) of x[:len]; nullptr: no normalisation
+    float dither;            // 0: no noise
+    uint32_t key0, key1;     // Philox key: lo32 / hi32 of the seed
+};
+
+// Philox4x32-10 (Salmon et al., SC'11; the Random123 constants) of counter (c0, c1, 0, 0), then Box-Muller on (u0, u1) and
+// (u2, u3) with u = ((r >> 8) + 0.5) 2^-24: four standard normal values.  The stream of include/wlm.h.
+__device__ __forceinline__ void philox_normal4(uint32_t k0, uint32_t k1, uint32_t c0, uint32_t c1, float (&z)[4]) {
+    uint32_t x0 = c0, x1 = c1, x2 = 0u, x3 = 0u;
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        if (r) { k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+        const uint32_t hi0 = __umulhi(0xD2511F53u, x0), lo0 = 0xD2511F53u * x0;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, x2), lo1 = 0xCD9E8D57u * x2;
+        x0 = hi1 ^ x1 ^ k0; x1 = lo1; x2 = hi0 ^ x3 ^ k1; x3 = lo0;
+    }
+    const uint32_t w[4] = {x0, x1, x2, x3};
+#pragma unroll
+    for (int p = 0; p < 2; ++p) {
+        const float ua = fmaf(static_cast<float>(w[2 * p] >> 8), 0x1p-24f, 0x1p-25f);
+        const float ub = fmaf(static_cast<float>(w[2 * p + 1] >> 8), 0x1p-24f, 0x1p-25f);
+        const float rad = sqrtf(-2.0f * logf(ua));
+        float sn, cs;
+        sincospif(2.0f * ub, &sn, &cs);
+        z[2 * p] = rad * cs;
+        z[2 * p + 1] = rad * sn;
+    }
+}
+
+// long_fixup for a conditioned call, on EVERY half-tile (also those the TMA filled completely), in HF's order:
+//   1. every position with sample s in [0, L): (x - mean) scale on [0, len) (x when not normalising), 0 on [len, L), then
+//      + dither z(seed, b, s).  A thread takes four consecutive samples: half-tiles and sub-regions start at multiples of
+//      4, so one Philox call serves the quad;
+//   2. then the positions outside [0, L) are reflected from the CONDITIONED values (a source may lie in the pad region,
+//      which carries noise).
+// The two sub-regions overlap by 240 samples; both copies get the same value, as z depends on (b, s) only.
+__device__ __forceinline__ void cond_fixup(const CondArgs& cnd, int pcm_format, int b, float2 ms, int64_t len, int64_t L,
+                                           int tile, float* raw, int grp, int tg) {
+    using fused::group_sync;
+    const int64_t s0 = long_s0(tile);
+    if (pcm_format == WLM_PCM_I16) long_expand_i16(raw, grp, tg);
+    constexpr int kQuads = kSubLen / 4;
+    static_assert(kSubLen % 4 == 0 && kSubStep % 4 == 0 && (kTile * kHop) % 4 == 0 && (kNfft / 2) % 4 == 0,
+                  "quads of the half-tile are quads of the noise stream");
+#pragma unroll 1
+    for (int q = tg; q < 2 * kQuads; q += kGroupThreads) {
+        const int r = q >= kQuads ? 1 : 0;
+        const int i = 4 * (q - r * kQuads);
+        const int64_t s = s0 + r * kSubStep + i;         // a multiple of 4: the quad lies wholly below 0 or at/above 0
+        if (s < 0 || s >= L) continue;
+        float z[4] = {0.f, 0.f, 0.f, 0.f};
+        if (cnd.dither != 0.f) philox_normal4(cnd.key0, cnd.key1, static_cast<uint32_t>(s >> 2), static_cast<uint32_t>(b), z);
+        float* p = raw + r * kSubLen + i;
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            if (s + e >= L) break;
+            const float x = s + e < len ? (cnd.moments ? (p[e] - ms.x) * ms.y : p[e]) : 0.f;
+            p[e] = fmaf(cnd.dither, z[e], x);
+        }
+    }
+    group_sync(grp);
+    if (s0 < 0 || s0 + kTileSamples > L) {
+#pragma unroll 1
+        for (int r = 0; r < 2; ++r) {
+            const int64_t s_lo = s0 + r * kSubStep;
+#pragma unroll 1
+            for (int i = tg; i < kSubLen; i += kGroupThreads) {
+                const int64_t s = s_lo + i;
+                if (s >= 0 && s < L) continue;
+                const int64_t sr = s < 0 ? -s : 2 * (L - 1) - s;
+                const int64_t u = sr - s0;
+                raw[r * kSubLen + i] = sr >= 0 && sr < L && u >= 0 && u < kTileSamples
+                                             ? raw[u < kSubLen ? u : kSubLen + (u - kSubStep)] : 0.f;
+            }
+        }
+        group_sync(grp);
+    }
+}
+
+// ---- per-clip moments (do_normalize) -----------------------------------------------------------------------------
+// Deterministic two-step reduction over x[:len] of every clip (len up to 2^31 - 1):
+//   logmel_moments_kernel        CTA (chunk, clip): float64 sums of d and d^2 over the chunk's kMomChunk samples, with
+//                                d = x - x[0] (the shift keeps a large DC offset from cancelling the variance away), in
+//                                a fixed order -> partial[b][chunk];
+//   logmel_moments_merge_kernel  one warp per clip: the partials in chunk order -> (mean, 1 / sqrt(var + 1e-7)), the
+//                                population variance, as HF's zero_mean_unit_var_norm.
+// No atomics: the result does not depend on scheduling.
+constexpr int kMomChunk = 1 << 16;
+constexpr int kMomThreads = 256;
+
+__device__ __forceinline__ float pcm_at(const LongArgs& a, int64_t i) {
+    return a.pcm_format == WLM_PCM_I16 ? static_cast<float>(static_cast<const int16_t*>(a.pcm)[i]) * (1.0f / 32768.0f)
+                                       : static_cast<const float*>(a.pcm)[i];
+}
+
+__global__ void __launch_bounds__(kMomThreads) logmel_moments_kernel(const LongArgs a, double2* __restrict__ partial,
+                                                                    int n_chunks) {
+    __shared__ double2 red[kMomThreads / 32];
+    const int tid = threadIdx.x;
+    for (int b = blockIdx.y; b < a.B; b += gridDim.y) {
+        const LongClip c = long_clip(a, b);
+        const int64_t lo = static_cast<int64_t>(blockIdx.x) * kMomChunk;
+        if (lo >= c.len) continue;                                        // CTA-uniform
+        const int64_t hi = min(lo + kMomChunk, c.len);
+        const double k = pcm_at(a, c.base);
+        double s1 = 0.0, s2 = 0.0;
+        // quads: the clip start is 16-byte aligned and so is every chunk start (f32: 16 B, i16: 8 B per quad)
+        const int64_t q_hi = lo / 4 + (hi - lo) / 4;
+        for (int64_t q = lo / 4 + tid; q < q_hi; q += kMomThreads) {
+            float x[4];
+            if (a.pcm_format == WLM_PCM_I16) {
+                const short4 v = reinterpret_cast<const short4*>(static_cast<const int16_t*>(a.pcm) + c.base)[q];
+                x[0] = v.x * (1.0f / 32768.0f); x[1] = v.y * (1.0f / 32768.0f);
+                x[2] = v.z * (1.0f / 32768.0f); x[3] = v.w * (1.0f / 32768.0f);
+            } else {
+                const float4 v = __ldcs(reinterpret_cast<const float4*>(static_cast<const float*>(a.pcm) + c.base) + q);
+                x[0] = v.x; x[1] = v.y; x[2] = v.z; x[3] = v.w;
+            }
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+                const double d = static_cast<double>(x[e]) - k;
+                s1 += d;
+                s2 = fma(d, d, s2);
+            }
+        }
+        for (int64_t i = 4 * q_hi + tid; i < hi; i += kMomThreads) {
+            const double d = static_cast<double>(pcm_at(a, c.base + i)) - k;
+            s1 += d;
+            s2 = fma(d, d, s2);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+            s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+        }
+        if ((tid & 31) == 0) red[tid >> 5] = make_double2(s1, s2);
+        __syncthreads();
+        if (tid == 0) {
+            double2 t = red[0];
+            for (int w = 1; w < kMomThreads / 32; ++w) { t.x += red[w].x; t.y += red[w].y; }
+            partial[static_cast<int64_t>(b) * n_chunks + blockIdx.x] = t;
+        }
+        __syncthreads();
+    }
+}
+
+__global__ void __launch_bounds__(256) logmel_moments_merge_kernel(const LongArgs a, const double2* __restrict__ partial,
+                                                                  int n_chunks, float2* __restrict__ moments) {
+    const int lane = threadIdx.x & 31;
+    const int w0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = (gridDim.x * blockDim.x) >> 5;
+    for (int b = w0; b < a.B; b += nw) {
+        const LongClip c = long_clip(a, b);
+        const int nc = static_cast<int>((c.len + kMomChunk - 1) / kMomChunk);
+        double s1 = 0.0, s2 = 0.0;
+        for (int j = lane; j < nc; j += 32) {
+            const double2 t = partial[static_cast<int64_t>(b) * n_chunks + j];
+            s1 += t.x;
+            s2 += t.y;
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+            s2 += __shfl_xor_sync(0xffffffffu, s2, o);
+        }
+        if (lane == 0) {
+            float2 m = make_float2(0.f, 0.f);             // an empty clip is all padding: nothing is normalised
+            if (c.len > 0) {
+                const double n = static_cast<double>(c.len), d1 = s1 / n;
+                const double var = fmax(s2 / n - d1 * d1, 0.0);
+                m = make_float2(static_cast<float>(static_cast<double>(pcm_at(a, c.base)) + d1),
+                                static_cast<float>(1.0 / sqrt(var + 1e-7)));
+            }
+            moments[b] = m;
+        }
+    }
+}
+
 // ---- pass 1 ------------------------------------------------------------------------------------------------------
 // NMELS = 80 / 128: unrolled mel stage of that Whisper bank; 0: table-driven.
-template <int NMELS, class OutT>
-__global__ void __launch_bounds__(kThreads, 1)
-logmel_long_kernel(const LongArgs a, const __grid_constant__ KernelTables kt, const float* __restrict__ win_lane) {
+// COND: a conditioned call (cond_fixup on every half-tile; with dither every half-tile of every clip is active).
+template <int NMELS, class OutT, bool COND>
+__device__ __forceinline__ void long_pass1(const LongArgs& a, const KernelTables& kt, const float* __restrict__ win_lane,
+                                           const CondArgs& cnd) {
     using namespace fused;
     extern __shared__ __align__(128) unsigned char smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -191,6 +379,11 @@ logmel_long_kernel(const LongArgs a, const __grid_constant__ KernelTables kt, co
     const int m0 = kt.m0[wg];
     const int U = a.units_per_clip;
     const long long n_units = static_cast<long long>(a.B) * U;
+    auto clip = [&](int b) {
+        LongClip c = long_clip(a, b);
+        if (COND && cnd.dither != 0.f) c.n_act = a.n_tiles;       // the noise reaches every half-tile
+        return c;
+    };
 
     // (thread 0 of the group) the next unit that holds an active half-tile, or -1.  The units of a clip are handed out
     // in order, so the first empty one ends the clip: the counter then skips the clip's remaining units.
@@ -199,14 +392,14 @@ logmel_long_kernel(const LongArgs a, const __grid_constant__ KernelTables kt, co
             const unsigned long long u = atomicAdd(a.next_unit, 1ull);
             if (u >= static_cast<unsigned long long>(n_units)) return -1;
             const int b = static_cast<int>(u / U), j = static_cast<int>(u % U);
-            if (j * kLongRun < long_clip(a, b).n_act) return static_cast<long long>(u);
+            if (j * kLongRun < clip(b).n_act) return static_cast<long long>(u);
             atomicMax(a.next_unit, static_cast<unsigned long long>(b + 1) * U);
         }
     };
     if (tg == 0) {
         const long long u = fetch();
         unit_slot[0] = u;
-        if (u >= 0) long_issue_tma(a, long_clip(a, static_cast<int>(u / U)), static_cast<int>(u % U) * kLongRun, raw, bar_raw);
+        if (u >= 0) long_issue_tma(a, clip(static_cast<int>(u / U)), static_cast<int>(u % U) * kLongRun, raw, bar_raw);
     }
     __syncthreads();
 
@@ -216,8 +409,10 @@ logmel_long_kernel(const LongArgs a, const __grid_constant__ KernelTables kt, co
         if (u < 0) break;
         const int b = static_cast<int>(u / U);
         const int t0 = static_cast<int>(u % U) * kLongRun;
-        const LongClip c = long_clip(a, b);
+        const LongClip c = clip(b);
         const int t1 = min(t0 + kLongRun, c.n_act);
+        float2 ms = make_float2(0.f, 1.f);
+        if (COND && cnd.moments) ms = cnd.moments[b];
         // the following unit: fetched now, so that its first copy can go out while this unit's last half-tile runs
         long long un = -1;
         if (tg == 0) {
@@ -229,7 +424,9 @@ logmel_long_kernel(const LongArgs a, const __grid_constant__ KernelTables kt, co
         for (int t = t0; t < t1; ++t, ++tnum) {
             mbar_wait(bar_raw, tnum & 1);
             const int64_t s0 = long_s0(t);
-            if (a.pcm_format == WLM_PCM_I16 || s0 < 0 || s0 + kTileSamples > c.len)
+            if (COND)
+                cond_fixup(cnd, a.pcm_format, b, ms, c.len, a.padded_len, t, raw, grp, tg);
+            else if (a.pcm_format == WLM_PCM_I16 || s0 < 0 || s0 + kTileSamples > c.len)
                 long_fixup(a.pcm_format, c.len, a.padded_len, t, raw, grp, tg);
             stage1(s1_base, Y, wv, wg, lane, [&]() {}, [&]() {});
             group_sync(grp);     // every warp is done with raw (and, from the previous half-tile, with P)
@@ -237,7 +434,7 @@ logmel_long_kernel(const LongArgs a, const __grid_constant__ KernelTables kt, co
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                 if (t + 1 < t1) long_issue_tma(a, c, t + 1, raw, bar_raw);
                 else if (un >= 0)
-                    long_issue_tma(a, long_clip(a, static_cast<int>(un / U)), static_cast<int>(un % U) * kLongRun, raw, bar_raw);
+                    long_issue_tma(a, clip(static_cast<int>(un / U)), static_cast<int>(un % U) * kLongRun, raw, bar_raw);
             }
             stage2(Y, P, wg, lane, [&]() {});
             group_sync(grp);     // P holds the half-tile's power
@@ -264,6 +461,20 @@ logmel_long_kernel(const LongArgs a, const __grid_constant__ KernelTables kt, co
         group_sync(grp);
         if (tg == 0) atomicMax(a.pmax + b, atomicExch(grp_max, 0));
     }
+}
+
+template <int NMELS, class OutT>
+__global__ void __launch_bounds__(kThreads, 1)
+logmel_long_kernel(const LongArgs a, const __grid_constant__ KernelTables kt, const float* __restrict__ win_lane) {
+    long_pass1<NMELS, OutT, false>(a, kt, win_lane, CondArgs{});
+}
+
+// pass 1 of wlm_logmel_conditioned
+template <int NMELS, class OutT>
+__global__ void __launch_bounds__(kThreads, 1)
+logmel_long_cond_kernel(const LongArgs a, const __grid_constant__ KernelTables kt, const float* __restrict__ win_lane,
+                        const CondArgs cnd) {
+    long_pass1<NMELS, OutT, true>(a, kt, win_lane, cnd);
 }
 
 // ---- pass 2 ------------------------------------------------------------------------------------------------------

@@ -88,6 +88,21 @@ static LongKernelFn long_kernel_for(int variant, int out_format) {
     if (out_format == WLM_OUT_F16) return long_kernel_for_t<__half>(variant);
     return long_kernel_for_t<float>(variant);
 }
+
+typedef void (*CondKernelFn)(const longform::LongArgs, const fused::KernelTables, const float*, const longform::CondArgs);
+
+template <class OutT>
+static CondKernelFn cond_kernel_for_t(int variant) {
+    using longform::logmel_long_cond_kernel;
+    if (variant == 80) return logmel_long_cond_kernel<80, OutT>;
+    if (variant == 128) return logmel_long_cond_kernel<128, OutT>;
+    return logmel_long_cond_kernel<0, OutT>;
+}
+static CondKernelFn cond_kernel_for(int variant, int out_format) {
+    if (out_format == WLM_OUT_BF16) return cond_kernel_for_t<__nv_bfloat16>(variant);
+    if (out_format == WLM_OUT_F16) return cond_kernel_for_t<__half>(variant);
+    return cond_kernel_for_t<float>(variant);
+}
 static ClampKernelFn clamp_kernel_for(int out_format) {
     if (out_format == WLM_OUT_BF16) return longform::logmel_long_clamp_kernel<__nv_bfloat16>;
     if (out_format == WLM_OUT_F16) return longform::logmel_long_clamp_kernel<__half>;
@@ -122,6 +137,8 @@ static cudaError_t configure(int variant, int* max_clusters) {
         }
     for (int fmt : {WLM_OUT_F32, WLM_OUT_BF16, WLM_OUT_F16}) {
         e = cudaFuncSetAttribute(long_kernel_for(variant, fmt), cudaFuncAttributeMaxDynamicSharedMemorySize, fused::kSmemBytes);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(cond_kernel_for(variant, fmt), cudaFuncAttributeMaxDynamicSharedMemorySize, fused::kSmemBytes);
         if (e != cudaSuccess) return e;
     }
     cudaLaunchConfig_t cfg;
@@ -557,9 +574,9 @@ extern "C" size_t wlm_padded_workspace_bytes(const wlm_plan* p, int B) {
     return padded_max_bytes(B) + 256;
 }
 
-extern "C" int wlm_logmel_padded(wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
-                                 const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B, void* out_dev,
-                                 float* gmax_dev, void* workspace, size_t workspace_bytes, void* stream) {
+// the checks of wlm_logmel_padded and wlm_logmel_conditioned before the workspace
+static int check_padded_call(const wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
+                             const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B, const void* out_dev) {
     if (!p) return fail(WLM_ERR_BAD_ARG, "plan is NULL");
     if (B < 0) return fail(WLM_ERR_BAD_ARG, "B=%d is negative", B);
     if (check_padded_len(padded_len) != WLM_OK) return WLM_ERR_BAD_ARG;
@@ -576,13 +593,20 @@ extern "C" int wlm_logmel_padded(wlm_plan* p, const void* pcm_dev, int pcm_forma
     } else if (!lengths_dev) {
         return fail(WLM_ERR_BAD_ARG, "ragged layout (offsets_dev) needs lengths_dev");
     }
-    const size_t need = wlm_padded_workspace_bytes(p, B);
+    return WLM_OK;
+}
+
+static int check_workspace(const void* workspace, size_t workspace_bytes, size_t need) {
     if (!workspace || workspace_bytes < need)
         return fail(WLM_ERR_WORKSPACE, "workspace %zu B < required %zu B", workspace_bytes, need);
     if (reinterpret_cast<uintptr_t>(workspace) & 15) return fail(WLM_ERR_BAD_ARG, "workspace must be 16-byte aligned");
-    WLM_CUDA(cudaSetDevice(p->device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    return WLM_OK;
+}
 
+// pass-1 arguments; the workspace starts with the per-clip maxima and the unit counter (wlm_padded_workspace_bytes)
+static longform::LongArgs long_args(const wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
+                                    const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B, void* out_dev,
+                                    float* gmax_dev, void* workspace) {
     longform::LongArgs a{};
     a.pcm = pcm_dev;
     a.offsets = offsets_dev;
@@ -599,18 +623,105 @@ extern "C" int wlm_logmel_padded(wlm_plan* p, const void* pcm_dev, int pcm_forma
     a.gmax = gmax_dev;
     a.pmax = static_cast<int*>(workspace);
     a.next_unit = reinterpret_cast<unsigned long long*>(static_cast<char*>(workspace) + padded_max_bytes(B));
+    return a;
+}
+
+static int64_t long_ctas(const wlm_plan* p, const longform::LongArgs& a) {
+    const int64_t units = (int64_t)a.B * a.units_per_clip;
+    return std::min<int64_t>(p->sm_count, (units + fused::kGroups - 1) / fused::kGroups);
+}
+
+// pass 2; `a` says which half-tiles pass 1 wrote (long_clip's n_act)
+static void launch_clamp(const wlm_plan* p, const longform::LongArgs& a, cudaStream_t st) {
+    const int64_t vecs = ((int64_t)a.n_mels * a.n_frames * (int64_t)out_elem_size(p) + 15) / 16;
+    const int gy = std::min(a.B, 65535);
+    const int gx = (int)std::max<int64_t>(1, std::min<int64_t>((vecs + 1023) / 1024, std::max(1, 8 * p->sm_count / gy)));
+    clamp_kernel_for(p->out_format)<<<dim3(gx, gy), 256, 0, st>>>(a);
+}
+
+extern "C" int wlm_logmel_padded(wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
+                                 const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B, void* out_dev,
+                                 float* gmax_dev, void* workspace, size_t workspace_bytes, void* stream) {
+    int rc = check_padded_call(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev);
+    if (rc != WLM_OK || B == 0) return rc;
+    const size_t need = wlm_padded_workspace_bytes(p, B);
+    if ((rc = check_workspace(workspace, workspace_bytes, need)) != WLM_OK) return rc;
+    WLM_CUDA(cudaSetDevice(p->device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const longform::LongArgs a = long_args(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev,
+                                           gmax_dev, workspace);
 
     // plain launches in stream order: pass 1 starts after everything before it, pass 2 after pass 1
     WLM_CUDA(cudaMemsetAsync(workspace, 0, need, st));
-    const int64_t units = (int64_t)B * a.units_per_clip;
-    const int ctas = (int)std::min<int64_t>(p->sm_count, (units + fused::kGroups - 1) / fused::kGroups);
-    long_kernel_for(p->variant, p->out_format)<<<ctas, fused::kThreads, fused::kSmemBytes, st>>>(a, p->mel, p->d_win_lane);
+    long_kernel_for(p->variant, p->out_format)<<<(int)long_ctas(p, a), fused::kThreads, fused::kSmemBytes, st>>>(a, p->mel,
+                                                                                                            p->d_win_lane);
     WLM_CUDA(cudaGetLastError());
-    const int64_t vecs = ((int64_t)a.n_mels * a.n_frames * (int64_t)out_elem_size(p) + 15) / 16;
-    const int gy = std::min(B, 65535);
-    const int gx = (int)std::max<int64_t>(1, std::min<int64_t>((vecs + 1023) / 1024, std::max(1, 8 * p->sm_count / gy)));
-    clamp_kernel_for(p->out_format)<<<dim3(gx, gy), 256, 0, st>>>(a);
+    launch_clamp(p, a, st);
     p->launches += 2;
+    WLM_CUDA(cudaGetLastError());
+    return WLM_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// conditioned long-form features: do_normalize and dither (logmel_long.cuh)
+// ------------------------------------------------------------------------------------------
+// workspace: that of wlm_logmel_padded, then the per-clip moments [B] float2, then the moments partials [B][n_chunks] double2
+static int64_t moment_chunks(int64_t padded_len) { return (padded_len + longform::kMomChunk - 1) / longform::kMomChunk; }
+static size_t moments_bytes(int B) { return ((size_t)B * sizeof(float2) + 255) / 256 * 256; }
+
+extern "C" size_t wlm_conditioned_workspace_bytes(const wlm_plan* p, int B, int64_t padded_len) {
+    if (!p || B <= 0 || padded_len <= kNfft / 2 || padded_len > INT32_MAX) return 0;
+    return wlm_padded_workspace_bytes(p, B) + moments_bytes(B) + (size_t)B * moment_chunks(padded_len) * sizeof(double2);
+}
+
+extern "C" int wlm_logmel_conditioned(wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
+                                      const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B,
+                                      int do_normalize, float dither, uint64_t seed, void* out_dev, float* gmax_dev,
+                                      void* workspace, size_t workspace_bytes, void* stream) {
+    int rc = check_padded_call(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev);
+    if (rc != WLM_OK) return rc;
+    if (!std::isfinite(dither)) return fail(WLM_ERR_BAD_ARG, "dither=%g is not finite", (double)dither);
+    if (B == 0) return WLM_OK;
+    const size_t need = wlm_conditioned_workspace_bytes(p, B, padded_len);
+    if ((rc = check_workspace(workspace, workspace_bytes, need)) != WLM_OK) return rc;
+    if (!do_normalize && dither == 0.0f)
+        return wlm_logmel_padded(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev, gmax_dev,
+                                 workspace, workspace_bytes, stream);
+    WLM_CUDA(cudaSetDevice(p->device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const longform::LongArgs a = long_args(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev,
+                                           gmax_dev, workspace);
+    char* ws = static_cast<char*>(workspace);
+    float2* moments = reinterpret_cast<float2*>(ws + wlm_padded_workspace_bytes(p, B));
+    double2* partial = reinterpret_cast<double2*>(ws + wlm_padded_workspace_bytes(p, B) + moments_bytes(B));
+    const int n_chunks = (int)moment_chunks(padded_len);
+
+    WLM_CUDA(cudaMemsetAsync(workspace, 0, wlm_padded_workspace_bytes(p, B), st));
+    int launches = 2;
+    if (do_normalize) {
+        longform::logmel_moments_kernel<<<dim3(n_chunks, std::min(B, 65535)), longform::kMomThreads, 0, st>>>(a, partial, n_chunks);
+        WLM_CUDA(cudaGetLastError());
+        const int blocks = (int)std::min<int64_t>(((int64_t)B * 32 + 255) / 256, (int64_t)p->sm_count * 8);
+        longform::logmel_moments_merge_kernel<<<blocks, 256, 0, st>>>(a, partial, n_chunks, moments);
+        WLM_CUDA(cudaGetLastError());
+        launches += 2;
+    }
+    longform::CondArgs c{};
+    c.moments = do_normalize ? moments : nullptr;
+    c.dither = dither;
+    c.key0 = (uint32_t)seed;
+    c.key1 = (uint32_t)(seed >> 32);
+    cond_kernel_for(p->variant, p->out_format)<<<(int)long_ctas(p, a), fused::kThreads, fused::kSmemBytes, st>>>(a, p->mel, p->d_win_lane, c);
+    WLM_CUDA(cudaGetLastError());
+    longform::LongArgs a2 = a;
+    if (dither != 0.0f) {
+        // pass 2 sees every clip as L samples long: every half-tile was written by pass 1
+        a2.offsets = nullptr;
+        a2.lengths = nullptr;
+        a2.row_stride = padded_len;
+    }
+    launch_clamp(p, a2, st);
+    p->launches += launches;
     WLM_CUDA(cudaGetLastError());
     return WLM_OK;
 }

@@ -32,6 +32,9 @@ class FeatureCache:
     def __init__(self, extractor, capacity_bytes: int = 8 << 30, dtype=None):
         import torch
 
+        if float(getattr(extractor, "dither", 0.0)) != 0.0:
+            raise ValueError("an extractor with dither != 0 draws new noise on every call; caching its features would "
+                             "freeze one draw")
         self.extractor = extractor
         self.n_mels = int(extractor.feature_size)
         self.device = extractor.device

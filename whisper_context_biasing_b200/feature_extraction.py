@@ -15,6 +15,7 @@ from __future__ import annotations
 
 import ctypes as C
 import logging
+import math
 import warnings
 from typing import Sequence
 
@@ -102,6 +103,11 @@ class B200WhisperFeatureExtractor:
                torch.float16: element type the kernel STORES (round-to-nearest of the float32
                value; the reference model runs under fp16 autocast, REF/scripts/train.py:250).
 
+    `dither` != 0 adds dither * z to the padded waveform of every featurising call (`__call__`,
+    `extract_host`, `extract_device`), as the reference adds dither * torch.randn; z is the
+    Philox stream of include/wlm.h, seeded per call from torch's default CPU generator, so
+    `torch.manual_seed` makes a run reproducible.
+
     Deviations from the reference class, on purpose: non-default geometry / padding arguments
     raise NotImplementedError; the object is bound to one CUDA device and (like every stateful
     CUDA plan) is meant to be driven from one host thread and one stream at a time.
@@ -121,8 +127,8 @@ class B200WhisperFeatureExtractor:
                 f"{(sampling_rate, hop_length, chunk_length, n_fft)}")
         if padding_value != 0.0:
             raise NotImplementedError("padding_value != 0.0 is not supported")
-        if dither != 0.0:
-            raise NotImplementedError("dither != 0.0 is not supported (the reference leaves it at 0.0)")
+        if not math.isfinite(float(dither)):
+            raise ValueError(f"dither={dither!r} must be a finite number")
         if output not in ("device", "numpy"):
             raise ValueError("output must be 'device' or 'numpy'")
         if not torch.cuda.is_available():
@@ -218,16 +224,35 @@ class B200WhisperFeatureExtractor:
 
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
-    def _workspace(self, B, padded=False):
+    def _workspace(self, B, padded=False, conditioned_len=None):
         import torch
 
-        need = int((N.LIB.wlm_padded_workspace_bytes if padded else N.LIB.wlm_workspace_bytes)(self._plan, B))
+        if conditioned_len is not None:
+            need = int(N.LIB.wlm_conditioned_workspace_bytes(self._plan, B, conditioned_len))
+        else:
+            need = int((N.LIB.wlm_padded_workspace_bytes if padded else N.LIB.wlm_workspace_bytes)(self._plan, B))
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(max(need, 256), dtype=torch.uint8, device=self.device)
         return self._ws, need
 
     # -- device-resident entry points (new; the reference has no device path) -------------------
-    def extract_device(self, pcm, lengths=None, offsets=None, out=None, return_gmax=False, padded_len=None):
+    def _conditioning(self, dither, seed):
+        """(dither, seed) of one featurising call: None -> the constructor's dither and a seed drawn from torch's default
+        CPU generator (drawn only when the call dithers)."""
+        import torch
+
+        dither = self.dither if dither is None else dither
+        dither = float(dither)
+        if not math.isfinite(dither):
+            raise ValueError(f"dither={dither!r} must be a finite number")
+        if dither == 0.0:
+            return 0.0, 0
+        if seed is None:
+            seed = int(torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), dtype=torch.int64).item())
+        return dither, int(seed) % 2 ** 64
+
+    def extract_device(self, pcm, lengths=None, offsets=None, out=None, return_gmax=False, padded_len=None,
+                       do_normalize=False, dither=None, seed=None):
         """PCM already in HBM -> features in HBM.
 
         pcm      CUDA tensor, float32 or int16 (int16 is scaled by 1/32768 on the GPU).
@@ -236,6 +261,9 @@ class B200WhisperFeatureExtractor:
         offsets  optional int64 CUDA tensor [B] of clip starts (elements) in the 1-D buffer.
         padded_len  None: every clip is padded / trimmed to 30 s, features [B, M, 3000].  An int L > 200: every
                  clip is zero-padded to L samples (long-form, `truncation=False`), features [B, M, L // 160].
+        do_normalize  HF's `do_normalize=True`: each clip's valid samples are scaled to zero mean, unit variance.
+        dither   noise amplitude added to the padded waveform (None: the constructor's `dither`).
+        seed     64-bit seed of the noise (None: drawn from torch's default CPU generator when the call dithers).
         """
         import torch
 
@@ -271,12 +299,15 @@ class B200WhisperFeatureExtractor:
                 raise ValueError(f"padded_len={padded_len}: the reflect padding of the STFT needs more than "
                                  f"{N_FFT // 2} samples")
         n_frames = self.nb_max_frames if padded_len is None else padded_len // self.hop_length
+        dither, seed = self._conditioning(dither, seed)
+        conditioned = bool(do_normalize) or dither != 0.0
         if out is None:
             out = torch.empty((B, self.feature_size, n_frames), dtype=self.feature_dtype, device=self.device)
         else:
             self._check_out(out, B, n_frames)
         gmax = torch.empty((max(B, 1),), dtype=torch.float32, device=self.device) if return_gmax else None
-        ws, need = self._workspace(B, padded=padded_len is not None)
+        L = self.n_samples if padded_len is None else padded_len       # the 30-s geometry of the conditioned call
+        ws, need = self._workspace(B, padded=padded_len is not None, conditioned_len=L if conditioned else None)
         if B:
             args = (C.c_void_p(pcm.data_ptr()), fmt,
                     C.c_void_p(offsets.data_ptr()) if offsets is not None else None,
@@ -284,7 +315,10 @@ class B200WhisperFeatureExtractor:
             tail = (B, C.c_void_p(out.data_ptr()), C.c_void_p(gmax.data_ptr()) if gmax is not None else None,
                     C.c_void_p(ws.data_ptr()), need, self._stream())
             with torch.cuda.device(self.device):
-                if padded_len is None:
+                if conditioned:
+                    N.check(N.LIB.wlm_logmel_conditioned(self._plan, *args, L, B, int(bool(do_normalize)), dither, seed,
+                                                         *tail[1:]))
+                elif padded_len is None:
                     N.check(N.LIB.wlm_logmel(self._plan, *args, *tail))
                 else:
                     N.check(N.LIB.wlm_logmel_padded(self._plan, *args, padded_len, *tail))
@@ -308,14 +342,58 @@ class B200WhisperFeatureExtractor:
                                                     C.c_void_p(mask.data_ptr()), self._stream()))
         return mask
 
-    def extract_host(self, clips, out=None, out_host=None):
+    def extract_host(self, clips, out=None, out_host=None, do_normalize=False, dither=None, seed=None):
         """Host PCM -> features in HBM through the plan's pinned H2D pipeline (wlm_logmel_host).
 
         clips   a list of 1-D float32 / int16 numpy arrays of any lengths (what a dataset yields), or -- without any
                 per-clip Python work -- a C-contiguous 2-D array [B, L] (dense batch), or a tuple
-                (buffer, offsets, lengths): one 1-D array holding every clip, int64 element offsets and lengths."""
+                (buffer, offsets, lengths): one 1-D array holding every clip, int64 element offsets and lengths.
+        do_normalize, dither, seed  as `extract_device`.  A conditioned call packs the clips into one pinned buffer
+                and runs `extract_device` on it (wlm_logmel_host has no conditioning)."""
         import torch
 
+        dither, seed = self._conditioning(dither, seed)
+        dt, B, ptr_arr, lens_arr, keep = self._host_batch(clips)
+        if B == 0:
+            return torch.empty((0, self.feature_size, self.nb_max_frames), dtype=self.feature_dtype, device=self.device)
+        if dt == np.float32:
+            fmt = N.WLM_PCM_F32
+        elif dt == np.int16:
+            fmt = N.WLM_PCM_I16
+        else:
+            raise ValueError(f"host PCM dtype {dt} not supported (float32 or int16)")
+        if out is None:
+            out = torch.empty((B, self.feature_size, self.nb_max_frames), dtype=self.feature_dtype, device=self.device)
+        else:
+            self._check_out(out, B)
+        if out_host is not None:
+            want = np.float32 if self.feature_dtype == torch.float32 else (np.float16 if self.feature_dtype == torch.float16 else np.uint16)
+            if (not isinstance(out_host, np.ndarray) or out_host.dtype != want or not out_host.flags["C_CONTIGUOUS"]
+                    or out_host.shape != (B, self.feature_size, self.nb_max_frames)):
+                raise ValueError(f"out_host must be a C-contiguous {np.dtype(want)} ndarray [B={B}, {self.feature_size}, "
+                                 f"{self.nb_max_frames}] (bfloat16 features: uint16 bit patterns)")
+        if do_normalize or dither != 0.0:
+            pcm, lens_dev, offs_dev = self._pack_host(dt, ptr_arr, lens_arr, self.n_samples)
+            del keep, ptr_arr, lens_arr
+            self.extract_device(pcm, lengths=lens_dev, offsets=offs_dev, out=out, do_normalize=do_normalize, dither=dither,
+                                seed=seed)
+            if out_host is not None:
+                bits = out.view(torch.int16) if self.feature_dtype == torch.bfloat16 else out
+                out_host[...] = bits.cpu().numpy().view(want)
+            return out
+        ptrs = ptr_arr.ctypes.data_as(C.POINTER(C.c_void_p))
+        lens = lens_arr.ctypes.data_as(C.POINTER(C.c_int32))
+        with torch.cuda.device(self.device):
+            N.check(N.LIB.wlm_logmel_host(
+                self._plan, ptrs, lens, fmt, B, C.c_void_p(out.data_ptr()),
+                C.c_void_p(out_host.ctypes.data) if out_host is not None else None, self._stream()))
+        del keep, ptr_arr, lens_arr
+        return out
+
+    @staticmethod
+    def _host_batch(clips):
+        """The host input forms of `extract_host` -> (dtype, B, uintp clip pointers, int32 lengths, what must stay alive
+        while the pointers are used).  dtype and the arrays are None for an empty list."""
         keep = clips
         if isinstance(clips, tuple) and len(clips) == 3 and isinstance(clips[0], np.ndarray):
             buf, offs, lens_np = clips
@@ -336,7 +414,7 @@ class B200WhisperFeatureExtractor:
         else:
             B = len(clips)
             if B == 0:
-                return torch.empty((0, self.feature_size, self.nb_max_frames), dtype=self.feature_dtype, device=self.device)
+                return None, 0, None, None, keep
             dt = clips[0].dtype
             if any(x.dtype != dt or x.ndim != 1 for x in clips):
                 raise ValueError("all clips must be 1-D arrays of the same dtype")
@@ -344,32 +422,32 @@ class B200WhisperFeatureExtractor:
                 clips = keep = [np.ascontiguousarray(x) for x in clips]
             ptr_arr = np.fromiter((x.__array_interface__["data"][0] for x in clips), dtype=np.uintp, count=B)
             lens_arr = np.fromiter((x.shape[0] for x in clips), dtype=np.int32, count=B)
-        if B == 0:
-            return torch.empty((0, self.feature_size, self.nb_max_frames), dtype=self.feature_dtype, device=self.device)
-        if dt == np.float32:
-            fmt = N.WLM_PCM_F32
-        elif dt == np.int16:
-            fmt = N.WLM_PCM_I16
-        else:
+        return dt, B, ptr_arr, lens_arr, keep
+
+    def _pack_host(self, dt, ptr_arr, lens_arr, max_len=None):
+        """Host clips (`_host_batch`'s pointers and lengths, float32 or int16) -> one pinned buffer on the device, each
+        clip trimmed to `max_len` samples and starting on a 16-byte boundary, copied over in one transfer.  Returns the
+        device buffer and the int32 lengths and int64 offsets of the ragged batch, on the device."""
+        import torch
+
+        if dt not in (np.float32, np.int16):
             raise ValueError(f"host PCM dtype {dt} not supported (float32 or int16)")
-        ptrs = ptr_arr.ctypes.data_as(C.POINTER(C.c_void_p))
-        lens = lens_arr.ctypes.data_as(C.POINTER(C.c_int32))
-        if out is None:
-            out = torch.empty((B, self.feature_size, self.nb_max_frames), dtype=self.feature_dtype, device=self.device)
-        else:
-            self._check_out(out, B)
-        if out_host is not None:
-            want = np.float32 if self.feature_dtype == torch.float32 else (np.float16 if self.feature_dtype == torch.float16 else np.uint16)
-            if (not isinstance(out_host, np.ndarray) or out_host.dtype != want or not out_host.flags["C_CONTIGUOUS"]
-                    or out_host.shape != (B, self.feature_size, self.nb_max_frames)):
-                raise ValueError(f"out_host must be a C-contiguous {np.dtype(want)} ndarray [B={B}, {self.feature_size}, "
-                                 f"{self.nb_max_frames}] (bfloat16 features: uint16 bit patterns)")
-        with torch.cuda.device(self.device):
-            N.check(N.LIB.wlm_logmel_host(
-                self._plan, ptrs, lens, fmt, B, C.c_void_p(out.data_ptr()),
-                C.c_void_p(out_host.ctypes.data) if out_host is not None else None, self._stream()))
-        del keep, ptr_arr, lens_arr
-        return out
+        esz = np.dtype(dt).itemsize
+        gran = 16 // esz
+        lens = lens_arr.astype(np.int64)
+        if max_len is not None:
+            lens = np.minimum(lens, max_len)
+        starts = (lens + gran - 1) // gran * gran
+        offs = np.concatenate([[0], np.cumsum(starts)[:-1]]).astype(np.int64)
+        host = torch.empty(int(starts.sum()) + gran, dtype=torch.float32 if dt == np.float32 else torch.int16,
+                           pin_memory=True)
+        base = host.data_ptr()
+        for o, n, p in zip(offs.tolist(), lens.tolist(), ptr_arr.tolist()):
+            if n:
+                C.memmove(base + o * esz, p, n * esz)
+        pcm = host.to(self.device, non_blocking=True)     # (the caching host allocator keeps `host` until the copy is done)
+        return (pcm, torch.from_numpy(lens.astype(np.int32)).to(self.device),
+                torch.from_numpy(offs).to(self.device))
 
     # -- the reference-facing call (TF-FE:189-342) ---------------------------------------------
     def __call__(self, raw_speech, truncation=True, pad_to_multiple_of=None, return_tensors=None,
@@ -393,15 +471,14 @@ class B200WhisperFeatureExtractor:
             raise NotImplementedError(
                 "implemented argument combinations: padding='max_length', max_length=None (30 s), truncation=True, "
                 "pad_to_multiple_of=None (the reference's), and padding='longest', truncation=False (long-form)")
-        if do_normalize:
-            raise NotImplementedError("do_normalize=True is not used by the reference and not implemented")
         if device not in (None, "cpu") and torch.device(device).type != "cuda":
             raise NotImplementedError(f"device={device!r}: features are always computed on {self.device}")
 
         lengths_np = None
         n_samples = self.n_samples                                          # samples every clip is padded to
+        do_normalize = bool(do_normalize)
         if longform:
-            feats, lengths_np, n_samples = self._call_longform(raw_speech, pad_to_multiple_of)
+            feats, lengths_np, n_samples = self._call_longform(raw_speech, pad_to_multiple_of, do_normalize)
         elif isinstance(raw_speech, torch.Tensor):
             if raw_speech.dim() > 2:
                 raise ValueError(f"Only mono-channel audio is supported for input to {self}")
@@ -409,17 +486,23 @@ class B200WhisperFeatureExtractor:
             if x.dtype != torch.float32:
                 x = x.to(torch.float32)
             if x.is_cuda:
-                if x.shape[1] % 4:         # rows must start on 16-byte boundaries (extract_device clones unaligned views)
-                    x = torch.nn.functional.pad(x, (0, 4 - x.shape[1] % 4))
-                feats = self.extract_device(x)
+                n = x.shape[1]
+                if n % 4:                  # rows must start on 16-byte boundaries (extract_device clones unaligned views)
+                    x = torch.nn.functional.pad(x, (0, 4 - n % 4))
+                if do_normalize or self.dither != 0.0:
+                    # the row padding above is not part of the clip: the moments and the noise see n samples
+                    lens = torch.full((x.shape[0],), n, dtype=torch.int32, device=self.device)
+                    feats = self.extract_device(x, lengths=lens, do_normalize=do_normalize)
+                else:
+                    feats = self.extract_device(x)
                 lengths_np = np.full((x.shape[0],), min(raw_speech.shape[-1], self.n_samples), dtype=np.int32)
             else:
                 clips = [r.numpy() for r in x]
-                feats = self.extract_host(clips)
+                feats = self.extract_host(clips, do_normalize=do_normalize)
                 lengths_np = np.array([min(c.shape[0], self.n_samples) for c in clips], dtype=np.int32)
         else:
             clips = self._host_clips(raw_speech)
-            feats = self.extract_host(clips)
+            feats = self.extract_host(clips, do_normalize=do_normalize)
             lengths_np = np.array([min(c.shape[0], self.n_samples) for c in clips], dtype=np.int32)
 
         want = return_tensors
@@ -437,16 +520,16 @@ class B200WhisperFeatureExtractor:
             lens_dev = torch.from_numpy(lengths_np).to(self.device)
             mask = self.frame_mask_device(lens_dev, padded_len=n_samples if longform else None)
             out["attention_mask"] = mask.cpu().numpy() if want == "np" else mask
-        elif return_attention_mask is None and self.return_attention_mask:
-            # The reference's quirk, kept: pad() falls back to the ctor attribute (TF-SU:135-137) and returns the
-            # SAMPLE-level mask [B, 480000] (long-form: [B, L]), which TF-FE:328 then does not rescale because the
-            # call argument is None.
+        elif do_normalize or (return_attention_mask is None and self.return_attention_mask):
+            # The reference's quirk, kept: pad() is asked for the mask (do_normalize needs it; otherwise it falls back
+            # to the ctor attribute, TF-SU:135-137) and returns the SAMPLE-level mask [B, 480000] (long-form: [B, L]),
+            # which TF-FE:328 then does not rescale because the call argument is not True.
             lens_dev = torch.from_numpy(lengths_np).to(self.device)
             mask = (torch.arange(n_samples, device=self.device, dtype=torch.int32)[None, :] < lens_dev[:, None]).to(torch.int32)
             out["attention_mask"] = mask.cpu().numpy() if want == "np" else mask
         return out
 
-    def _call_longform(self, raw_speech, pad_to_multiple_of):
+    def _call_longform(self, raw_speech, pad_to_multiple_of, do_normalize=False):
         """`truncation=False, padding="longest"`: every clip is zero-padded to L = padded_length(...) samples.
         A CUDA tensor goes to the kernels as it is (dense rows); host input is packed into one pinned buffer, clip
         starts 16-byte aligned, copied over in one transfer and run as a ragged batch.
@@ -465,24 +548,24 @@ class B200WhisperFeatureExtractor:
                 self._check_padded_len(L)
                 if n % 4:          # rows must start on 16-byte boundaries; the padding is zeros, as HF pads
                     x = torch.nn.functional.pad(x, (0, 4 - n % 4))
-                return self.extract_device(x, padded_len=L), np.full((B,), n, dtype=np.int32), L
+                if do_normalize or self.dither != 0.0:
+                    # the row padding above is not part of the clip: the moments and the noise see n samples
+                    lens = torch.full((B,), n, dtype=torch.int32, device=self.device)
+                    feats = self.extract_device(x, lengths=lens, padded_len=L, do_normalize=do_normalize)
+                else:
+                    feats = self.extract_device(x, padded_len=L)
+                return feats, np.full((B,), n, dtype=np.int32), L
             clips = [r.numpy() for r in x]
         else:
             clips = self._host_clips(raw_speech)
         lens = np.array([c.shape[0] for c in clips], dtype=np.int64)
         L = padded_length(lens, pad_to_multiple_of)
         self._check_padded_len(L)
-        starts = (lens + 3) // 4 * 4                       # 16-byte aligned clip starts
-        offs = np.concatenate([[0], np.cumsum(starts)[:-1]]).astype(np.int64)
-        host = torch.empty(int(starts.sum()) + 4, dtype=torch.float32, pin_memory=True)
-        h = host.numpy()
-        for o, c in zip(offs, clips):
-            h[o:o + c.shape[0]] = c
-        pcm = host.to(self.device, non_blocking=True)     # (the caching host allocator keeps `host` until the copy is done)
-        lens32 = lens.astype(np.int32)
-        feats = self.extract_device(pcm, lengths=torch.from_numpy(lens32).to(self.device),
-                                    offsets=torch.from_numpy(offs).to(self.device), padded_len=L)
-        return feats, lens32, L
+        dt, _, ptr_arr, lens_arr, keep = self._host_batch(clips)
+        pcm, lens_dev, offs_dev = self._pack_host(dt, ptr_arr, lens_arr)
+        del keep
+        feats = self.extract_device(pcm, lengths=lens_dev, offsets=offs_dev, padded_len=L, do_normalize=do_normalize)
+        return feats, lens.astype(np.int32), L
 
     def _host_clips(self, raw_speech):
         """numpy / list input -> list of contiguous float32 1-D clips"""
