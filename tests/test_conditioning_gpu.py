@@ -217,26 +217,38 @@ def test_unconditioned_abi_call_equals_wlm_logmel_padded(ex):
     B, L = 3, 123457
     x = torch.from_numpy(np.stack([O.synth_clip("speech", 123460, 90 + i) for i in range(B)])).to(e.device)
     lens = torch.tensor([123457, 5000, 0], dtype=torch.int32, device=e.device)
-    a = e.extract_device(x, lengths=lens, padded_len=L)
+    a = torch.empty((B, 80, L // 160), device=e.device)
     out = torch.empty_like(a)
+    padded_need = int(N.LIB.wlm_padded_workspace_bytes(e._plan, B))
     need = int(N.LIB.wlm_conditioned_workspace_bytes(e._plan, B, L))
-    assert need >= int(N.LIB.wlm_padded_workspace_bytes(e._plan, B))
+    assert need >= padded_need
     ws = torch.empty(need, dtype=torch.uint8, device=e.device)
     st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    n0 = e.launch_count
+    assert N.LIB.wlm_logmel_padded(e._plan, C.c_void_p(x.data_ptr()), N.WLM_PCM_F32, None, C.c_void_p(lens.data_ptr()),
+                                   x.shape[1], L, B, C.c_void_p(a.data_ptr()), None, C.c_void_p(ws.data_ptr()), padded_need,
+                                   st) == N.WLM_OK
+    n_padded = e.launch_count - n0
 
-    def call(padded_len=L, do_norm=0, dither=0.0, ws_bytes=need):
+    def call(padded_len=L, do_norm=0, dither=0.0, ws_bytes=need, b=B):
         return N.LIB.wlm_logmel_conditioned(e._plan, C.c_void_p(x.data_ptr()), N.WLM_PCM_F32, None,
-                                            C.c_void_p(lens.data_ptr()), x.shape[1], padded_len, B, do_norm, dither, 5,
+                                            C.c_void_p(lens.data_ptr()), x.shape[1], padded_len, b, do_norm, dither, 5,
                                             C.c_void_p(out.data_ptr()), None, C.c_void_p(ws.data_ptr()), ws_bytes, st)
+    n0 = e.launch_count
     assert call() == N.WLM_OK
+    assert e.launch_count - n0 == n_padded == 2
     torch.cuda.synchronize()
     assert torch.equal(a, out)
     # errors
     assert call(dither=float("nan")) == N.WLM_ERR_BAD_ARG
     assert call(dither=float("inf")) == N.WLM_ERR_BAD_ARG
     assert call(do_norm=1, ws_bytes=need - 1) == N.WLM_ERR_WORKSPACE
+    assert call(ws_bytes=need - 1) == N.WLM_ERR_WORKSPACE          # nothing to condition: still the conditioned workspace
     assert call(padded_len=200) == N.WLM_ERR_BAD_ARG
     assert call(padded_len=2 ** 31) == N.WLM_ERR_BAD_ARG
+    assert call(b=0) == N.WLM_OK
+    assert call(b=0, padded_len=200) == N.WLM_ERR_BAD_ARG
+    assert call(b=0, dither=float("nan")) == N.WLM_ERR_BAD_ARG
     assert int(N.LIB.wlm_conditioned_workspace_bytes(e._plan, B, 200)) == 0
     with pytest.raises(ValueError):
         e.extract_device(x, lengths=lens, padded_len=L, dither=float("nan"))

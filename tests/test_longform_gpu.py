@@ -282,25 +282,56 @@ def test_stream_order_with_the_30s_path(lf):
 def test_call_forms_and_errors(lf):
     import torch
 
+    from whisper_context_biasing_b200 import B200WhisperFeatureExtractor
     from whisper_context_biasing_b200 import _native as N
 
     ex, *_ = lf
     e = ex[80]
-    rows = np.stack([O.synth_clip("speech", 333333, 40 + i) for i in range(3)])
-    a = e(list(rows), **LONG, return_tensors="np").input_features
-    b = e(rows, **LONG, return_tensors="np").input_features
-    c = e(torch.from_numpy(rows), **LONG, return_tensors="np").input_features
-    d = e(torch.from_numpy(rows).to(e.device), **LONG, return_tensors="pt").input_features
-    assert a.shape == (3, 80, 333333 // 160)
-    assert np.array_equal(a, b) and np.array_equal(a, c) and np.array_equal(a, d.cpu().numpy())
+    q = B200WhisperFeatureExtractor(feature_size=80, return_attention_mask=True)
+    n = 333333                                           # n % 4 != 0: the CUDA rows are padded to 16-byte boundaries
+    rows = np.stack([O.synth_clip("speech", n, 40 + i) for i in range(3)])
+    kinds = {"list": list(rows), "numpy": rows, "cpu": torch.from_numpy(rows), "cuda": torch.from_numpy(rows).to(e.device)}
+    # every input kind gives the same features and mask bits, in both geometries, with and without do_normalize, in the
+    # three mask modes (none, the call's return_attention_mask=True, the constructor's); a 1-D array gives its row's
+    for geometry, L in ((dict(sampling_rate=16000), 480000), (LONG, n)):
+        for do_normalize in (False, True):
+            for fe, mask_kw in ((e, {}), (e, dict(return_attention_mask=True)), (q, {})):
+                kw = dict(**geometry, **mask_kw, do_normalize=do_normalize, return_tensors="np")
+                got = {k: fe(x, **kw) for k, x in kinds.items()}
+                ref = got["list"]
+                case = (L, do_normalize, fe is q, mask_kw)
+                assert ref["input_features"].shape == (3, 80, L // 160), case
+                if mask_kw:
+                    assert ref["attention_mask"].shape == (3, L // 160), case
+                elif do_normalize or fe is q:
+                    assert ref["attention_mask"].shape == (3, L), case             # HF's sample-level mask
+                else:
+                    assert "attention_mask" not in ref, case
+                got["1-D"] = fe(rows[1], **kw)
+                for k, r in got.items():
+                    assert sorted(r) == sorted(ref), (case, k)
+                    for key in ref:
+                        want = ref[key][1:2] if k == "1-D" else ref[key]
+                        assert np.array_equal(r[key], want), (case, k, key)
+    d = e(kinds["cuda"], **LONG, return_tensors="pt").input_features
     assert d.is_cuda
     one = e(rows[1], **LONG, pad_to_multiple_of=480000, max_length=1000, return_tensors="pt").input_features
     assert tuple(one.shape) == (1, 80, 3000)
+    q.close()
     # errors
+    for geometry in (dict(sampling_rate=16000), LONG):
+        for x in (rows[None], torch.from_numpy(rows)[None], kinds["cuda"][None]):
+            with pytest.raises(ValueError):
+                e(x, **geometry)
+    for x in (kinds["list"], kinds["cuda"]):
+        with pytest.raises(ValueError):
+            e(x, **LONG, pad_to_multiple_of=2 ** 31)
     with pytest.raises(ValueError):
         e([np.zeros(200, np.float32)], **LONG)
     with pytest.raises(ValueError):
         e.extract_device(torch.zeros(1, 400, device=e.device), padded_len=200)
+    with pytest.raises(ValueError):
+        e.extract_device(torch.zeros(1, 400, device=e.device), padded_len=2 ** 31)
     x = torch.zeros(2, 1024, device=e.device)
     out = torch.empty(2, 80, 6, device=e.device)
     need = int(N.LIB.wlm_padded_workspace_bytes(e._plan, 2))
@@ -316,6 +347,7 @@ def test_call_forms_and_errors(lf):
     assert call(x.data_ptr(), 1000, need - 1) == N.WLM_ERR_WORKSPACE
     assert call(x.data_ptr() + 4, 1000, need) == N.WLM_ERR_BAD_ARG
     assert call(x.data_ptr(), 1000, need, out.data_ptr() + 4) == N.WLM_ERR_BAD_ARG
+    assert N.LIB.wlm_logmel(e._plan, None, 0, None, None, 0, 0, None, None, None, 0, st) == N.WLM_OK      # B = 0
     m = torch.empty(2, 6, dtype=torch.int32, device=e.device)
     assert N.LIB.wlm_frame_mask_padded(e._plan, C.c_void_p(torch.zeros(2, dtype=torch.int32, device=e.device).data_ptr()),
                                        2, 200, C.c_void_p(m.data_ptr()), st) == N.WLM_ERR_BAD_ARG

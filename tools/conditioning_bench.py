@@ -4,8 +4,10 @@
 
 Workloads (device-resident float32 PCM larger than the 126 MB L2; CUDA events around `iters` calls after a warm-up; the
 entry points alternate `rounds` times and the best round is reported, every round is in the line):
-  30s   256 x 30 s, 80 mels: wlm_logmel, wlm_logmel_padded (L = 480000), conditioned with normalise, with dither, with both
-  20min 4 x 20 min, 128 mels: wlm_logmel_padded, conditioned with normalise, with dither, with both
+  30s   256 x 30 s, 80 mels: wlm_logmel, padded (L = 480000), conditioned with normalise, with dither, with both
+  20min 4 x 20 min, 128 mels: padded, conditioned with normalise, with dither, with both
+`padded` is `extract_device(padded_len=L)` with nothing to condition: `wlm_logmel_conditioned` issuing the launches of
+wlm_logmel_padded.
 and, on the same tensors, HF's device-resident torch operations as the baseline: the normalisation of
 zero_mean_unit_var_norm (mean, population variance, (x - mean) / sqrt(var + 1e-7)), `+ dither * torch.randn`, then
 TF-FE:141-161 (stft, |.|^2, mel matmul, clamp + log10, per-clip max, affine).

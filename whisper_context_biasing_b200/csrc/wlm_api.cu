@@ -484,12 +484,9 @@ static int launch_logmel(wlm_plan* p, ClipArgs a, cudaStream_t st) {
     return WLM_OK;
 }
 
-extern "C" int wlm_logmel(wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
-                          const int32_t* lengths_dev, int64_t row_stride, int B, void* out_dev,
-                          float* gmax_dev, void* workspace, size_t workspace_bytes, void* stream) {
-    if (!p) return fail(WLM_ERR_BAD_ARG, "plan is NULL");
-    if (B < 0) return fail(WLM_ERR_BAD_ARG, "B=%d is negative", B);
-    if (B == 0) return WLM_OK;
+// the batch arguments of every device-buffer entry point (B > 0): pointers, PCM format, alignment and layout
+static int check_batch(const void* pcm_dev, int pcm_format, const int64_t* offsets_dev, const int32_t* lengths_dev,
+                       int64_t row_stride, const void* out_dev) {
     if (!pcm_dev || !out_dev) return fail(WLM_ERR_BAD_ARG, "pcm_dev/out_dev is NULL");
     if (pcm_format != WLM_PCM_F32 && pcm_format != WLM_PCM_I16) return fail(WLM_ERR_BAD_ARG, "unknown pcm_format %d", pcm_format);
     if ((reinterpret_cast<uintptr_t>(pcm_dev) & 15) || (reinterpret_cast<uintptr_t>(out_dev) & 15))
@@ -502,6 +499,17 @@ extern "C" int wlm_logmel(wlm_plan* p, const void* pcm_dev, int pcm_format, cons
     } else if (!lengths_dev) {
         return fail(WLM_ERR_BAD_ARG, "ragged layout (offsets_dev) needs lengths_dev");
     }
+    return WLM_OK;
+}
+
+extern "C" int wlm_logmel(wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
+                          const int32_t* lengths_dev, int64_t row_stride, int B, void* out_dev,
+                          float* gmax_dev, void* workspace, size_t workspace_bytes, void* stream) {
+    if (!p) return fail(WLM_ERR_BAD_ARG, "plan is NULL");
+    if (B < 0) return fail(WLM_ERR_BAD_ARG, "B=%d is negative", B);
+    if (B == 0) return WLM_OK;
+    const int rc = check_batch(pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, out_dev);
+    if (rc != WLM_OK) return rc;
     float* gmax = gmax_dev;
     if (!gmax) {
         const size_t need = wlm_workspace_bytes(p, B);
@@ -581,19 +589,7 @@ static int check_padded_call(const wlm_plan* p, const void* pcm_dev, int pcm_for
     if (B < 0) return fail(WLM_ERR_BAD_ARG, "B=%d is negative", B);
     if (check_padded_len(padded_len) != WLM_OK) return WLM_ERR_BAD_ARG;
     if (B == 0) return WLM_OK;
-    if (!pcm_dev || !out_dev) return fail(WLM_ERR_BAD_ARG, "pcm_dev/out_dev is NULL");
-    if (pcm_format != WLM_PCM_F32 && pcm_format != WLM_PCM_I16) return fail(WLM_ERR_BAD_ARG, "unknown pcm_format %d", pcm_format);
-    if ((reinterpret_cast<uintptr_t>(pcm_dev) & 15) || (reinterpret_cast<uintptr_t>(out_dev) & 15))
-        return fail(WLM_ERR_BAD_ARG, "pcm_dev and out_dev must be 16-byte aligned");
-    if (!offsets_dev) {
-        if (row_stride <= 0) return fail(WLM_ERR_BAD_ARG, "dense layout needs row_stride > 0 (got %lld)", (long long)row_stride);
-        const int gran = pcm_format == WLM_PCM_I16 ? 8 : 4;
-        if (row_stride % gran)
-            return fail(WLM_ERR_BAD_ARG, "dense row_stride must be a multiple of %d elements (16 bytes), got %lld", gran, (long long)row_stride);
-    } else if (!lengths_dev) {
-        return fail(WLM_ERR_BAD_ARG, "ragged layout (offsets_dev) needs lengths_dev");
-    }
-    return WLM_OK;
+    return check_batch(pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, out_dev);
 }
 
 static int check_workspace(const void* workspace, size_t workspace_bytes, size_t need) {
@@ -639,39 +635,70 @@ static void launch_clamp(const wlm_plan* p, const longform::LongArgs& a, cudaStr
     clamp_kernel_for(p->out_format)<<<dim3(gx, gy), 256, 0, st>>>(a);
 }
 
-extern "C" int wlm_logmel_padded(wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
-                                 const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B, void* out_dev,
-                                 float* gmax_dev, void* workspace, size_t workspace_bytes, void* stream) {
-    int rc = check_padded_call(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev);
-    if (rc != WLM_OK || B == 0) return rc;
-    const size_t need = wlm_padded_workspace_bytes(p, B);
-    if ((rc = check_workspace(workspace, workspace_bytes, need)) != WLM_OK) return rc;
-    WLM_CUDA(cudaSetDevice(p->device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const longform::LongArgs a = long_args(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev,
-                                           gmax_dev, workspace);
-
-    // plain launches in stream order: pass 1 starts after everything before it, pass 2 after pass 1
-    WLM_CUDA(cudaMemsetAsync(workspace, 0, need, st));
-    long_kernel_for(p->variant, p->out_format)<<<(int)long_ctas(p, a), fused::kThreads, fused::kSmemBytes, st>>>(a, p->mel,
-                                                                                                            p->d_win_lane);
-    WLM_CUDA(cudaGetLastError());
-    launch_clamp(p, a, st);
-    p->launches += 2;
-    WLM_CUDA(cudaGetLastError());
-    return WLM_OK;
-}
-
-// ------------------------------------------------------------------------------------------
-// conditioned long-form features: do_normalize and dither (logmel_long.cuh)
-// ------------------------------------------------------------------------------------------
-// workspace: that of wlm_logmel_padded, then the per-clip moments [B] float2, then the moments partials [B][n_chunks] double2
+// conditioned calls (do_normalize, dither); workspace: that of wlm_logmel_padded, then the per-clip moments [B] float2,
+// then the moments partials [B][n_chunks] double2
 static int64_t moment_chunks(int64_t padded_len) { return (padded_len + longform::kMomChunk - 1) / longform::kMomChunk; }
 static size_t moments_bytes(int B) { return ((size_t)B * sizeof(float2) + 255) / 256 * 256; }
 
 extern "C" size_t wlm_conditioned_workspace_bytes(const wlm_plan* p, int B, int64_t padded_len) {
     if (!p || B <= 0 || padded_len <= kNfft / 2 || padded_len > INT32_MAX) return 0;
     return wlm_padded_workspace_bytes(p, B) + moments_bytes(B) + (size_t)B * moment_chunks(padded_len) * sizeof(double2);
+}
+
+// The launches of a checked long-form call, plain and in stream order: pass 1 starts after everything before it, pass 2
+// after pass 1.  With nothing to condition, pass 1 is logmel_long_kernel and only wlm_logmel_padded's workspace is used.
+static int launch_long(wlm_plan* p, const longform::LongArgs& a, int do_normalize, float dither, uint64_t seed,
+                       void* workspace, cudaStream_t st) {
+    const size_t padded_bytes = wlm_padded_workspace_bytes(p, a.B);
+    WLM_CUDA(cudaMemsetAsync(workspace, 0, padded_bytes, st));
+    int launches = 2;
+    longform::CondArgs c{};
+    if (do_normalize) {
+        char* ws = static_cast<char*>(workspace) + padded_bytes;
+        float2* moments = reinterpret_cast<float2*>(ws);
+        double2* partial = reinterpret_cast<double2*>(ws + moments_bytes(a.B));
+        const int n_chunks = (int)moment_chunks(a.padded_len);
+        longform::logmel_moments_kernel<<<dim3(n_chunks, std::min(a.B, 65535)), longform::kMomThreads, 0, st>>>(a, partial, n_chunks);
+        WLM_CUDA(cudaGetLastError());
+        const int blocks = (int)std::min<int64_t>(((int64_t)a.B * 32 + 255) / 256, (int64_t)p->sm_count * 8);
+        longform::logmel_moments_merge_kernel<<<blocks, 256, 0, st>>>(a, partial, n_chunks, moments);
+        WLM_CUDA(cudaGetLastError());
+        c.moments = moments;
+        launches += 2;
+    }
+    const int ctas = (int)long_ctas(p, a);
+    if (!do_normalize && dither == 0.0f) {
+        long_kernel_for(p->variant, p->out_format)<<<ctas, fused::kThreads, fused::kSmemBytes, st>>>(a, p->mel, p->d_win_lane);
+    } else {
+        c.dither = dither;
+        c.key0 = (uint32_t)seed;
+        c.key1 = (uint32_t)(seed >> 32);
+        cond_kernel_for(p->variant, p->out_format)<<<ctas, fused::kThreads, fused::kSmemBytes, st>>>(a, p->mel, p->d_win_lane, c);
+    }
+    WLM_CUDA(cudaGetLastError());
+    longform::LongArgs a2 = a;
+    if (dither != 0.0f) {
+        // pass 2 sees every clip as L samples long: every half-tile was written by pass 1
+        a2.offsets = nullptr;
+        a2.lengths = nullptr;
+        a2.row_stride = a.padded_len;
+    }
+    launch_clamp(p, a2, st);
+    p->launches += launches;
+    WLM_CUDA(cudaGetLastError());
+    return WLM_OK;
+}
+
+extern "C" int wlm_logmel_padded(wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
+                                 const int32_t* lengths_dev, int64_t row_stride, int64_t padded_len, int B, void* out_dev,
+                                 float* gmax_dev, void* workspace, size_t workspace_bytes, void* stream) {
+    int rc = check_padded_call(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev);
+    if (rc != WLM_OK || B == 0) return rc;
+    if ((rc = check_workspace(workspace, workspace_bytes, wlm_padded_workspace_bytes(p, B))) != WLM_OK) return rc;
+    WLM_CUDA(cudaSetDevice(p->device));
+    return launch_long(p, long_args(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev, gmax_dev,
+                                    workspace),
+                       0, 0.0f, 0, workspace, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int wlm_logmel_conditioned(wlm_plan* p, const void* pcm_dev, int pcm_format, const int64_t* offsets_dev,
@@ -682,48 +709,11 @@ extern "C" int wlm_logmel_conditioned(wlm_plan* p, const void* pcm_dev, int pcm_
     if (rc != WLM_OK) return rc;
     if (!std::isfinite(dither)) return fail(WLM_ERR_BAD_ARG, "dither=%g is not finite", (double)dither);
     if (B == 0) return WLM_OK;
-    const size_t need = wlm_conditioned_workspace_bytes(p, B, padded_len);
-    if ((rc = check_workspace(workspace, workspace_bytes, need)) != WLM_OK) return rc;
-    if (!do_normalize && dither == 0.0f)
-        return wlm_logmel_padded(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev, gmax_dev,
-                                 workspace, workspace_bytes, stream);
+    if ((rc = check_workspace(workspace, workspace_bytes, wlm_conditioned_workspace_bytes(p, B, padded_len))) != WLM_OK) return rc;
     WLM_CUDA(cudaSetDevice(p->device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const longform::LongArgs a = long_args(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev,
-                                           gmax_dev, workspace);
-    char* ws = static_cast<char*>(workspace);
-    float2* moments = reinterpret_cast<float2*>(ws + wlm_padded_workspace_bytes(p, B));
-    double2* partial = reinterpret_cast<double2*>(ws + wlm_padded_workspace_bytes(p, B) + moments_bytes(B));
-    const int n_chunks = (int)moment_chunks(padded_len);
-
-    WLM_CUDA(cudaMemsetAsync(workspace, 0, wlm_padded_workspace_bytes(p, B), st));
-    int launches = 2;
-    if (do_normalize) {
-        longform::logmel_moments_kernel<<<dim3(n_chunks, std::min(B, 65535)), longform::kMomThreads, 0, st>>>(a, partial, n_chunks);
-        WLM_CUDA(cudaGetLastError());
-        const int blocks = (int)std::min<int64_t>(((int64_t)B * 32 + 255) / 256, (int64_t)p->sm_count * 8);
-        longform::logmel_moments_merge_kernel<<<blocks, 256, 0, st>>>(a, partial, n_chunks, moments);
-        WLM_CUDA(cudaGetLastError());
-        launches += 2;
-    }
-    longform::CondArgs c{};
-    c.moments = do_normalize ? moments : nullptr;
-    c.dither = dither;
-    c.key0 = (uint32_t)seed;
-    c.key1 = (uint32_t)(seed >> 32);
-    cond_kernel_for(p->variant, p->out_format)<<<(int)long_ctas(p, a), fused::kThreads, fused::kSmemBytes, st>>>(a, p->mel, p->d_win_lane, c);
-    WLM_CUDA(cudaGetLastError());
-    longform::LongArgs a2 = a;
-    if (dither != 0.0f) {
-        // pass 2 sees every clip as L samples long: every half-tile was written by pass 1
-        a2.offsets = nullptr;
-        a2.lengths = nullptr;
-        a2.row_stride = padded_len;
-    }
-    launch_clamp(p, a2, st);
-    p->launches += launches;
-    WLM_CUDA(cudaGetLastError());
-    return WLM_OK;
+    return launch_long(p, long_args(p, pcm_dev, pcm_format, offsets_dev, lengths_dev, row_stride, padded_len, B, out_dev, gmax_dev,
+                                    workspace),
+                       do_normalize, dither, seed, workspace, static_cast<cudaStream_t>(stream));
 }
 
 // ------------------------------------------------------------------------------------------

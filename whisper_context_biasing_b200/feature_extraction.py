@@ -73,6 +73,28 @@ def padded_length(lengths, pad_to_multiple_of=None) -> int:
     return L
 
 
+def _pcm_format(dtype) -> int:
+    """WLM_PCM_* of a numpy or torch PCM dtype: float32, or int16 (scaled by 1/32768 on the GPU)."""
+    import torch
+
+    fmt = {np.dtype(np.float32): N.WLM_PCM_F32, torch.float32: N.WLM_PCM_F32,
+           np.dtype(np.int16): N.WLM_PCM_I16, torch.int16: N.WLM_PCM_I16}.get(dtype)
+    if fmt is None:
+        raise ValueError(f"PCM dtype {dtype} not supported (float32 or int16)")
+    return fmt
+
+
+def _feature_format(dtype):
+    """(WLM_OUT_*, numpy dtype of a host copy) of a feature dtype; bfloat16 features are copied as uint16 bit patterns."""
+    import torch
+
+    fmt = {torch.float32: (N.WLM_OUT_F32, np.float32), torch.bfloat16: (N.WLM_OUT_BF16, np.uint16),
+           torch.float16: (N.WLM_OUT_F16, np.float16)}.get(dtype)
+    if fmt is None:
+        raise ValueError(f"feature_dtype {dtype} not supported (float32, bfloat16, float16)")
+    return fmt
+
+
 class LogMelBatch(dict):
     """dict with attribute access, like `BatchFeature.__getattr__`
     (feature_extraction_utils.py:95-99): `out.input_features`, `out["input_features"]`, item
@@ -199,12 +221,7 @@ class B200WhisperFeatureExtractor:
 
     def set_feature_dtype(self, dtype):
         """Element type of the features the kernel stores: float32, bfloat16 or float16."""
-        import torch
-
-        fmt = {torch.float32: N.WLM_OUT_F32, torch.bfloat16: N.WLM_OUT_BF16, torch.float16: N.WLM_OUT_F16}.get(dtype)
-        if fmt is None:
-            raise ValueError(f"feature_dtype {dtype} not supported (float32, bfloat16, float16)")
-        N.check(N.LIB.wlm_plan_set_output_format(self._plan, fmt))
+        N.check(N.LIB.wlm_plan_set_output_format(self._plan, _feature_format(dtype)[0]))
         self.feature_dtype = dtype
 
     def set_flat_clips(self, n: int = -1):
@@ -224,13 +241,14 @@ class B200WhisperFeatureExtractor:
 
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
-    def _workspace(self, B, padded=False, conditioned_len=None):
+    def _workspace(self, B, padded_len=None):
+        """Workspace of a wlm_logmel call (padded_len None) or of a wlm_logmel_conditioned call."""
         import torch
 
-        if conditioned_len is not None:
-            need = int(N.LIB.wlm_conditioned_workspace_bytes(self._plan, B, conditioned_len))
+        if padded_len is None:
+            need = int(N.LIB.wlm_workspace_bytes(self._plan, B))
         else:
-            need = int((N.LIB.wlm_padded_workspace_bytes if padded else N.LIB.wlm_workspace_bytes)(self._plan, B))
+            need = int(N.LIB.wlm_conditioned_workspace_bytes(self._plan, B, padded_len))
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(max(need, 256), dtype=torch.uint8, device=self.device)
         return self._ws, need
@@ -271,12 +289,7 @@ class B200WhisperFeatureExtractor:
             raise ValueError("extract_device expects a CUDA tensor")
         if pcm.device != self.device:
             raise ValueError(f"pcm is on {pcm.device}, the extractor on {self.device}")
-        if pcm.dtype == torch.float32:
-            fmt = N.WLM_PCM_F32
-        elif pcm.dtype == torch.int16:
-            fmt = N.WLM_PCM_I16
-        else:
-            raise ValueError(f"pcm dtype {pcm.dtype} not supported (float32 or int16)")
+        fmt = _pcm_format(pcm.dtype)
         if not pcm.is_contiguous() or pcm.data_ptr() % 16:
             pcm = pcm.contiguous() if pcm.data_ptr() % 16 == 0 else pcm.clone(memory_format=torch.contiguous_format)
         if offsets is None:
@@ -295,33 +308,28 @@ class B200WhisperFeatureExtractor:
             raise ValueError("lengths must be a CUDA int32 tensor of shape [B]")
         if padded_len is not None:
             padded_len = int(padded_len)
-            if padded_len <= N_FFT // 2:
-                raise ValueError(f"padded_len={padded_len}: the reflect padding of the STFT needs more than "
-                                 f"{N_FFT // 2} samples")
-        n_frames = self.nb_max_frames if padded_len is None else padded_len // self.hop_length
+            self._check_padded_len(padded_len)
+        L = self.n_samples if padded_len is None else padded_len
         dither, seed = self._conditioning(dither, seed)
-        conditioned = bool(do_normalize) or dither != 0.0
+        plain = padded_len is None and not do_normalize and dither == 0.0
         if out is None:
-            out = torch.empty((B, self.feature_size, n_frames), dtype=self.feature_dtype, device=self.device)
+            out = torch.empty((B, self.feature_size, L // self.hop_length), dtype=self.feature_dtype, device=self.device)
         else:
-            self._check_out(out, B, n_frames)
+            self._check_out(out, B, L // self.hop_length)
         gmax = torch.empty((max(B, 1),), dtype=torch.float32, device=self.device) if return_gmax else None
-        L = self.n_samples if padded_len is None else padded_len       # the 30-s geometry of the conditioned call
-        ws, need = self._workspace(B, padded=padded_len is not None, conditioned_len=L if conditioned else None)
+        ws, need = self._workspace(B, None if plain else L)
         if B:
             args = (C.c_void_p(pcm.data_ptr()), fmt,
                     C.c_void_p(offsets.data_ptr()) if offsets is not None else None,
                     C.c_void_p(lengths.data_ptr()) if lengths is not None else None, stride)
-            tail = (B, C.c_void_p(out.data_ptr()), C.c_void_p(gmax.data_ptr()) if gmax is not None else None,
+            tail = (C.c_void_p(out.data_ptr()), C.c_void_p(gmax.data_ptr()) if gmax is not None else None,
                     C.c_void_p(ws.data_ptr()), need, self._stream())
             with torch.cuda.device(self.device):
-                if conditioned:
+                if plain:
+                    N.check(N.LIB.wlm_logmel(self._plan, *args, B, *tail))
+                else:       # with nothing to condition: the launches of wlm_logmel_padded
                     N.check(N.LIB.wlm_logmel_conditioned(self._plan, *args, L, B, int(bool(do_normalize)), dither, seed,
-                                                         *tail[1:]))
-                elif padded_len is None:
-                    N.check(N.LIB.wlm_logmel(self._plan, *args, *tail))
-                else:
-                    N.check(N.LIB.wlm_logmel_padded(self._plan, *args, padded_len, *tail))
+                                                         *tail))
         return (out, gmax[:B]) if return_gmax else out
 
     def frame_mask_device(self, lengths, padded_len=None):
@@ -330,16 +338,11 @@ class B200WhisperFeatureExtractor:
         import torch
 
         B = lengths.shape[0]
-        n_frames = self.nb_max_frames if padded_len is None else int(padded_len) // self.hop_length
-        mask = torch.empty((B, max(n_frames, 0)), dtype=torch.int32, device=self.device)
+        L = self.n_samples if padded_len is None else int(padded_len)
+        mask = torch.empty((B, max(L // self.hop_length, 0)), dtype=torch.int32, device=self.device)
         with torch.cuda.device(self.device):
-            if padded_len is None:
-                if B:
-                    N.check(N.LIB.wlm_frame_mask(self._plan, C.c_void_p(lengths.data_ptr()), B,
-                                                 C.c_void_p(mask.data_ptr()), self._stream()))
-            else:
-                N.check(N.LIB.wlm_frame_mask_padded(self._plan, C.c_void_p(lengths.data_ptr()), B, int(padded_len),
-                                                    C.c_void_p(mask.data_ptr()), self._stream()))
+            N.check(N.LIB.wlm_frame_mask_padded(self._plan, C.c_void_p(lengths.data_ptr()), B, L,
+                                                C.c_void_p(mask.data_ptr()), self._stream()))
         return mask
 
     def extract_host(self, clips, out=None, out_host=None, do_normalize=False, dither=None, seed=None):
@@ -356,18 +359,13 @@ class B200WhisperFeatureExtractor:
         dt, B, ptr_arr, lens_arr, keep = self._host_batch(clips)
         if B == 0:
             return torch.empty((0, self.feature_size, self.nb_max_frames), dtype=self.feature_dtype, device=self.device)
-        if dt == np.float32:
-            fmt = N.WLM_PCM_F32
-        elif dt == np.int16:
-            fmt = N.WLM_PCM_I16
-        else:
-            raise ValueError(f"host PCM dtype {dt} not supported (float32 or int16)")
+        fmt = _pcm_format(dt)
         if out is None:
             out = torch.empty((B, self.feature_size, self.nb_max_frames), dtype=self.feature_dtype, device=self.device)
         else:
             self._check_out(out, B)
         if out_host is not None:
-            want = np.float32 if self.feature_dtype == torch.float32 else (np.float16 if self.feature_dtype == torch.float16 else np.uint16)
+            want = _feature_format(self.feature_dtype)[1]
             if (not isinstance(out_host, np.ndarray) or out_host.dtype != want or not out_host.flags["C_CONTIGUOUS"]
                     or out_host.shape != (B, self.feature_size, self.nb_max_frames)):
                 raise ValueError(f"out_host must be a C-contiguous {np.dtype(want)} ndarray [B={B}, {self.feature_size}, "
@@ -430,8 +428,7 @@ class B200WhisperFeatureExtractor:
         device buffer and the int32 lengths and int64 offsets of the ragged batch, on the device."""
         import torch
 
-        if dt not in (np.float32, np.int16):
-            raise ValueError(f"host PCM dtype {dt} not supported (float32 or int16)")
+        fmt = _pcm_format(dt)
         esz = np.dtype(dt).itemsize
         gran = 16 // esz
         lens = lens_arr.astype(np.int64)
@@ -439,7 +436,7 @@ class B200WhisperFeatureExtractor:
             lens = np.minimum(lens, max_len)
         starts = (lens + gran - 1) // gran * gran
         offs = np.concatenate([[0], np.cumsum(starts)[:-1]]).astype(np.int64)
-        host = torch.empty(int(starts.sum()) + gran, dtype=torch.float32 if dt == np.float32 else torch.int16,
+        host = torch.empty(int(starts.sum()) + gran, dtype=torch.float32 if fmt == N.WLM_PCM_F32 else torch.int16,
                            pin_memory=True)
         base = host.data_ptr()
         for o, n, p in zip(offs.tolist(), lens.tolist(), ptr_arr.tolist()):
@@ -474,36 +471,34 @@ class B200WhisperFeatureExtractor:
         if device not in (None, "cpu") and torch.device(device).type != "cuda":
             raise NotImplementedError(f"device={device!r}: features are always computed on {self.device}")
 
-        lengths_np = None
-        n_samples = self.n_samples                                          # samples every clip is padded to
         do_normalize = bool(do_normalize)
-        if longform:
-            feats, lengths_np, n_samples = self._call_longform(raw_speech, pad_to_multiple_of, do_normalize)
-        elif isinstance(raw_speech, torch.Tensor):
-            if raw_speech.dim() > 2:
-                raise ValueError(f"Only mono-channel audio is supported for input to {self}")
-            x = raw_speech if raw_speech.dim() == 2 else raw_speech[None]
-            if x.dtype != torch.float32:
-                x = x.to(torch.float32)
-            if x.is_cuda:
-                n = x.shape[1]
-                if n % 4:                  # rows must start on 16-byte boundaries (extract_device clones unaligned views)
-                    x = torch.nn.functional.pad(x, (0, 4 - n % 4))
-                if do_normalize or self.dither != 0.0:
-                    # the row padding above is not part of the clip: the moments and the noise see n samples
-                    lens = torch.full((x.shape[0],), n, dtype=torch.int32, device=self.device)
-                    feats = self.extract_device(x, lengths=lens, do_normalize=do_normalize)
-                else:
-                    feats = self.extract_device(x)
-                lengths_np = np.full((x.shape[0],), min(raw_speech.shape[-1], self.n_samples), dtype=np.int32)
-            else:
-                clips = [r.numpy() for r in x]
-                feats = self.extract_host(clips, do_normalize=do_normalize)
-                lengths_np = np.array([min(c.shape[0], self.n_samples) for c in clips], dtype=np.int32)
+        x = self._speech(raw_speech)
+        if isinstance(x, torch.Tensor):
+            lengths = np.full((x.shape[0],), x.shape[1], dtype=np.int64)
         else:
-            clips = self._host_clips(raw_speech)
-            feats = self.extract_host(clips, do_normalize=do_normalize)
-            lengths_np = np.array([min(c.shape[0], self.n_samples) for c in clips], dtype=np.int32)
+            lengths = np.array([c.shape[0] for c in x], dtype=np.int64)
+        if longform:                                            # every clip is zero-padded to L samples
+            L = padded_length(lengths, pad_to_multiple_of)
+            self._check_padded_len(L)
+        else:                                                   # every clip is padded or trimmed to 30 s
+            L = self.n_samples
+        if isinstance(x, torch.Tensor):                         # CUDA rows go to the kernels as they are
+            B, n = x.shape
+            if n % 4:          # rows must start on 16-byte boundaries; the padding is zeros, as HF pads
+                x = torch.nn.functional.pad(x, (0, 4 - n % 4))
+            lens = None        # a plain call keeps the dense layout: the static cluster / flat split
+            if do_normalize or self.dither != 0.0:
+                # the row padding above is not part of the clip: the moments and the noise see n samples
+                lens = torch.full((B,), n, dtype=torch.int32, device=self.device)
+            feats = self.extract_device(x, lengths=lens, padded_len=L if longform else None, do_normalize=do_normalize)
+        elif not longform:
+            feats = self.extract_host(x, do_normalize=do_normalize)
+        else:
+            # one pinned buffer, clip starts 16-byte aligned, copied over in one transfer and run as a ragged batch
+            dt, _, ptr_arr, lens_arr, keep = self._host_batch(x)
+            pcm, lens_dev, offs_dev = self._pack_host(dt, ptr_arr, lens_arr)
+            del keep
+            feats = self.extract_device(pcm, lengths=lens_dev, offsets=offs_dev, padded_len=L, do_normalize=do_normalize)
 
         want = return_tensors
         if want is None:
@@ -516,24 +511,21 @@ class B200WhisperFeatureExtractor:
             out["input_features"] = feats
         else:
             raise NotImplementedError(f"return_tensors={return_tensors!r} (use None, 'pt' or 'np')")
-        if return_attention_mask:                                                              # TF-FE:328-337
-            lens_dev = torch.from_numpy(lengths_np).to(self.device)
-            mask = self.frame_mask_device(lens_dev, padded_len=n_samples if longform else None)
-            out["attention_mask"] = mask.cpu().numpy() if want == "np" else mask
-        elif do_normalize or (return_attention_mask is None and self.return_attention_mask):
-            # The reference's quirk, kept: pad() is asked for the mask (do_normalize needs it; otherwise it falls back
-            # to the ctor attribute, TF-SU:135-137) and returns the SAMPLE-level mask [B, 480000] (long-form: [B, L]),
-            # which TF-FE:328 then does not rescale because the call argument is not True.
-            lens_dev = torch.from_numpy(lengths_np).to(self.device)
-            mask = (torch.arange(n_samples, device=self.device, dtype=torch.int32)[None, :] < lens_dev[:, None]).to(torch.int32)
+        if return_attention_mask or do_normalize or (return_attention_mask is None and self.return_attention_mask):
+            lens_dev = torch.from_numpy(np.minimum(lengths, L).astype(np.int32)).to(self.device)
+            if return_attention_mask:                                                          # TF-FE:328-337
+                mask = self.frame_mask_device(lens_dev, padded_len=L)
+            else:
+                # The reference's quirk, kept: pad() is asked for the mask (do_normalize needs it; otherwise it falls
+                # back to the ctor attribute, TF-SU:135-137) and returns the SAMPLE-level mask [B, L], which TF-FE:328
+                # then does not rescale because the call argument is not True.
+                mask = (torch.arange(L, device=self.device, dtype=torch.int32)[None, :] < lens_dev[:, None]).to(torch.int32)
             out["attention_mask"] = mask.cpu().numpy() if want == "np" else mask
         return out
 
-    def _call_longform(self, raw_speech, pad_to_multiple_of, do_normalize=False):
-        """`truncation=False, padding="longest"`: every clip is zero-padded to L = padded_length(...) samples.
-        A CUDA tensor goes to the kernels as it is (dense rows); host input is packed into one pinned buffer, clip
-        starts 16-byte aligned, copied over in one transfer and run as a ragged batch.
-        Returns (features [B, M, L // 160], int32 lengths, L)."""
+    def _speech(self, raw_speech):
+        """The input forms of `__call__` -> a CUDA float32 tensor [B, n], or a list of contiguous float32 1-D host clips
+        (TF-FE:274-290)."""
         import torch
 
         if isinstance(raw_speech, torch.Tensor):
@@ -542,33 +534,7 @@ class B200WhisperFeatureExtractor:
             x = raw_speech if raw_speech.dim() == 2 else raw_speech[None]
             if x.dtype != torch.float32:
                 x = x.to(torch.float32)
-            if x.is_cuda:
-                B, n = x.shape
-                L = padded_length([n] * B, pad_to_multiple_of)
-                self._check_padded_len(L)
-                if n % 4:          # rows must start on 16-byte boundaries; the padding is zeros, as HF pads
-                    x = torch.nn.functional.pad(x, (0, 4 - n % 4))
-                if do_normalize or self.dither != 0.0:
-                    # the row padding above is not part of the clip: the moments and the noise see n samples
-                    lens = torch.full((B,), n, dtype=torch.int32, device=self.device)
-                    feats = self.extract_device(x, lengths=lens, padded_len=L, do_normalize=do_normalize)
-                else:
-                    feats = self.extract_device(x, padded_len=L)
-                return feats, np.full((B,), n, dtype=np.int32), L
-            clips = [r.numpy() for r in x]
-        else:
-            clips = self._host_clips(raw_speech)
-        lens = np.array([c.shape[0] for c in clips], dtype=np.int64)
-        L = padded_length(lens, pad_to_multiple_of)
-        self._check_padded_len(L)
-        dt, _, ptr_arr, lens_arr, keep = self._host_batch(clips)
-        pcm, lens_dev, offs_dev = self._pack_host(dt, ptr_arr, lens_arr)
-        del keep
-        feats = self.extract_device(pcm, lengths=lens_dev, offsets=offs_dev, padded_len=L, do_normalize=do_normalize)
-        return feats, lens.astype(np.int32), L
-
-    def _host_clips(self, raw_speech):
-        """numpy / list input -> list of contiguous float32 1-D clips"""
+            return x if x.is_cuda else [np.ascontiguousarray(r.numpy()) for r in x]
         is_batched_numpy = isinstance(raw_speech, np.ndarray) and raw_speech.ndim > 1          # TF-FE:274
         if is_batched_numpy and raw_speech.ndim > 2:
             raise ValueError(f"Only mono-channel audio is supported for input to {self}")      # TF-FE:275-276
@@ -581,9 +547,11 @@ class B200WhisperFeatureExtractor:
 
     @staticmethod
     def _check_padded_len(L):
+        """A padded length the long-form kernels take: torch.stft's reflect padding needs more than n_fft // 2 samples,
+        and the frame positions stay in 32 bits."""
         if L <= N_FFT // 2:
-            raise ValueError(f"the longest clip has {L} samples: the reflect padding of the STFT needs more than "
-                             f"{N_FFT // 2} (torch.stft refuses it too)")
+            raise ValueError(f"padded length {L}: the reflect padding of the STFT needs more than {N_FFT // 2} samples "
+                             "(torch.stft refuses it too)")
         if L >= 2 ** 31:
             raise ValueError(f"padded length {L} does not fit 32 bits")
 
