@@ -63,16 +63,63 @@ def collate_labels(features: List[Dict[str, Any]], pad_token_id: int, decoder_st
     return out
 
 
+class PendingFeatures:
+    """One batch of PCM, collated in a DataLoader worker, whose features `collator.finish` computes in the main process.
+
+    pcm       1-D float32 or int16 tensor (as the clips came): every clip trimmed to 480000 samples and starting on a
+              16-byte boundary (`feature_extraction.pack_pcm`, the layout the extractor's host packing builds)
+    offsets   int64 [B] clip starts in `pcm` (elements)
+    lengths   int32 [B] samples of each clip
+
+    It is picklable (a worker sends it to the main process), `pin_memory()` and `to(device)` return copies, so the
+    DataLoader's pin thread and a trainer's device placement can handle it like a tensor.  `shape` and `numel()` are those
+    of the features it stands for, which is what a trainer reads to count FLOPs.
+    """
+
+    def __init__(self, pcm, offsets, lengths, feature_size: int):
+        self.pcm, self.offsets, self.lengths = pcm, offsets, lengths
+        self.feature_size = int(feature_size)
+
+    def pin_memory(self):
+        return PendingFeatures(self.pcm.pin_memory(), self.offsets.pin_memory(), self.lengths.pin_memory(),
+                               self.feature_size)
+
+    def to(self, device, non_blocking=False):
+        return PendingFeatures(*(t.to(device, non_blocking=non_blocking) for t in (self.pcm, self.offsets, self.lengths)),
+                               self.feature_size)
+
+    @property
+    def shape(self):
+        from .feature_extraction import NB_MAX_FRAMES
+
+        return (len(self), self.feature_size, NB_MAX_FRAMES)
+
+    def numel(self) -> int:
+        return int(np.prod(self.shape))
+
+    def __len__(self):
+        return int(self.offsets.shape[0])
+
+    def __repr__(self):
+        return f"PendingFeatures(B={len(self)}, pcm={self.pcm.dtype}, device={self.pcm.device})"
+
+
 class B200DataCollatorSpeechSeq2SeqWithPadding:
     """Drop-in for the reference collator with the feature extraction moved onto the B200.
 
     Args mirror the reference dataclass (`processor`, `decoder_start_token_id`,
     `decoder_prev_token_id`); `processor.feature_extractor` must be a `B200WhisperFeatureExtractor`
     and `processor.tokenizer.pad_token_id` supplies the pad id (or pass `pad_token_id=`).
+
+    defer:  whether a batch of PCM items is featurised later, by `finish` in the main process.  None (default): inside
+            a DataLoader worker (`torch.utils.data.get_worker_info() is not None`), where CUDA cannot be used; True /
+            False force the choice.  A deferred call touches neither CUDA nor the extractor: the batch carries a
+            `PendingFeatures` under the features' key, and labels stay on the CPU until `finish`.
     """
 
     def __init__(self, processor: Any = None, decoder_start_token_id: int = None, decoder_prev_token_id: Optional[int] = None,
-                 feature_extractor: Any = None, pad_token_id: Optional[int] = None, labels_on_device: bool = False):
+                 feature_extractor: Any = None, pad_token_id: Optional[int] = None, labels_on_device: bool = False,
+                 defer: Optional[bool] = None):
         self.processor = processor
         self.feature_extractor = feature_extractor if feature_extractor is not None else processor.feature_extractor
         if pad_token_id is None:
@@ -83,23 +130,69 @@ class B200DataCollatorSpeechSeq2SeqWithPadding:
         self.decoder_start_token_id = int(decoder_start_token_id)
         self.decoder_prev_token_id = decoder_prev_token_id
         self.labels_on_device = labels_on_device
+        self.defer = defer
+
+    def __getstate__(self):
+        # a spawned worker needs the extractor (it pickles detached) and the token ids, not the processor
+        return {**self.__dict__, "processor": None}
 
     def __call__(self, features: List[Dict[str, Any]]):
-        from .feature_extraction import LogMelBatch
+        import torch
+
+        from .feature_extraction import N_SAMPLES, B200WhisperFeatureExtractor, LogMelBatch, pack_pcm
 
         fe = self.feature_extractor
         name = fe.model_input_names[0]
+        defer = self.defer if self.defer is not None else torch.utils.data.get_worker_info() is not None
         if features and "audio" in features[0]:
             clips = [np.ascontiguousarray(np.asarray(f["audio"]).reshape(-1)) for f in features]
             if clips[0].dtype not in (np.float32, np.int16):
                 clips = [c.astype(np.float32) for c in clips]
-            feats = fe.extract_host(clips)                       # one batched call; stays in HBM
-            batch = LogMelBatch({name: feats})
+            if defer:
+                dt, _, ptr_arr, lens_arr, keep = B200WhisperFeatureExtractor._host_batch(clips)
+                pcm, offsets, lengths = pack_pcm(dt, ptr_arr, lens_arr, N_SAMPLES)
+                del keep
+                batch = LogMelBatch({name: PendingFeatures(pcm, offsets, lengths, fe.feature_size)})
+            else:
+                feats = fe.extract_host(clips)                   # one batched call; stays in HBM
+                batch = LogMelBatch({name: feats})
         else:
             batch = fe.pad({name: [f[name] for f in features]}, padding="longest", return_tensors="pt")
         lab = collate_labels(features, self.pad_token_id, self.decoder_start_token_id, self.decoder_prev_token_id)
-        if self.labels_on_device:
+        if self.labels_on_device and not defer:
             lab = {k: v.to(fe.device, non_blocking=True) for k, v in lab.items()}
         for k, v in lab.items():
             batch[k] = v
         return batch
+
+    def finish(self, batch):
+        """Main-process half of a deferred batch: every `PendingFeatures` in `batch` is replaced, in place, by its features
+        in HBM -- one ragged launch of the extractor (`extract_device(pcm, offsets=, lengths=)`), the features the
+        collator computes in-process, bit for bit; a dithering extractor draws its seed here, from this process's torch
+        generator.  The pending tensors may be on the CPU, pinned, or on the device.  Then `labels_on_device` is applied.
+        A batch with nothing pending is returned as it is."""
+        fe = self.feature_extractor
+        pending = [k for k, v in batch.items() if isinstance(v, PendingFeatures)]
+        if not pending:
+            return batch
+        for k in pending:
+            p = batch[k].to(fe.device, non_blocking=True)
+            batch[k] = fe.extract_device(p.pcm, offsets=p.offsets, lengths=p.lengths)
+        if self.labels_on_device:
+            for k in ("labels", "decoder_input_ids", "bias_spans"):
+                if k in batch:
+                    batch[k] = batch[k].to(fe.device, non_blocking=True)
+        return batch
+
+
+class B200FeaturesTrainerMixin:
+    """Featurises deferred batches in a `transformers.Trainer`'s main process:
+
+        class Trainer(B200FeaturesTrainerMixin, Seq2SeqTrainer):
+            pass
+
+    with `data_collator=B200DataCollatorSpeechSeq2SeqWithPadding(...)`.  Training and prediction steps both prepare their
+    inputs through `_prepare_inputs`; `Trainer._prepare_input` passes the `PendingFeatures` through untouched."""
+
+    def _prepare_inputs(self, inputs):
+        return self.data_collator.finish(super()._prepare_inputs(inputs))

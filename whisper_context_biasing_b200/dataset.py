@@ -81,5 +81,15 @@ def pcm_dataset_class(ref_dataset_cls):
         def all_bias_spans(self) -> List[List[List[int]]]:
             return [self.bias_spans_only(i) for i in range(len(self))]
 
+        def __reduce__(self):
+            # this class is made at run time, so pickle (a spawned DataLoader worker) cannot find it by name: rebuild it
+            # from the reference class; `device_feature_extractor` pickles detached
+            return _pcm_dataset_instance, (ref_dataset_cls,), self.__getstate__()
+
     PcmPromptWhisperDataset.__qualname__ = "PcmPromptWhisperDataset"
     return PcmPromptWhisperDataset
+
+
+def _pcm_dataset_instance(ref_dataset_cls):
+    cls = pcm_dataset_class(ref_dataset_cls)
+    return cls.__new__(cls)

@@ -16,6 +16,7 @@ from __future__ import annotations
 import ctypes as C
 import logging
 import math
+import os
 import warnings
 from typing import Sequence
 
@@ -71,6 +72,29 @@ def padded_length(lengths, pad_to_multiple_of=None) -> int:
     if pad_to_multiple_of is not None and L % pad_to_multiple_of != 0:
         L = (L // pad_to_multiple_of + 1) * pad_to_multiple_of
     return L
+
+
+def pack_pcm(dt, ptr_arr, lens_arr, max_len=None, pin_memory=False):
+    """Host clips (float32 or int16; `ptr_arr` their addresses, `lens_arr` their lengths) -> one 1-D host tensor holding
+    every clip, trimmed to `max_len` samples and starting on a 16-byte boundary, plus the int64 offsets and int32 lengths
+    of that ragged batch (CPU tensors).  The gaps between clips are not initialised; nothing reads them."""
+    import torch
+
+    fmt = _pcm_format(dt)
+    esz = np.dtype(dt).itemsize
+    gran = 16 // esz
+    lens = lens_arr.astype(np.int64)
+    if max_len is not None:
+        lens = np.minimum(lens, max_len)
+    starts = (lens + gran - 1) // gran * gran
+    offs = np.concatenate([[0], np.cumsum(starts)[:-1]]).astype(np.int64)
+    host = torch.empty(int(starts.sum()) + gran, dtype=torch.float32 if fmt == N.WLM_PCM_F32 else torch.int16,
+                       pin_memory=pin_memory)
+    base = host.data_ptr()
+    for o, n, p in zip(offs.tolist(), lens.tolist(), ptr_arr.tolist()):
+        if n:
+            C.memmove(base + o * esz, p, n * esz)
+    return host, torch.from_numpy(offs), torch.from_numpy(lens.astype(np.int32))
 
 
 def _pcm_format(dtype) -> int:
@@ -132,7 +156,9 @@ class B200WhisperFeatureExtractor:
 
     Deviations from the reference class, on purpose: non-default geometry / padding arguments
     raise NotImplementedError; the object is bound to one CUDA device and (like every stateful
-    CUDA plan) is meant to be driven from one host thread and one stream at a time.
+    CUDA plan) is meant to be driven from one host thread and one stream at a time.  It is also
+    bound to the process that created it: in a forked child, or as an unpickled copy (a spawned
+    DataLoader worker's), its attributes work but featurising raises RuntimeError.
     """
 
     model_input_names = ["input_features"]          # TF-FE:67
@@ -184,6 +210,7 @@ class B200WhisperFeatureExtractor:
         handle = C.c_void_p()
         N.check(N.LIB.wlm_plan_create(dev.index, self.feature_size, table.ctypes.data, C.byref(handle)))
         self._plan = handle
+        self._owner_pid = os.getpid()
         self._ws = None
         self.feature_dtype = torch.float32
         if feature_dtype is not None:
@@ -192,8 +219,30 @@ class B200WhisperFeatureExtractor:
     # -- lifecycle ---------------------------------------------------------------------------
     def close(self):
         plan, self._plan = getattr(self, "_plan", None), None
-        if plan:
+        if plan and getattr(self, "_owner_pid", None) == os.getpid():     # a forked copy never frees the parent's plan
             N.LIB.wlm_plan_destroy(plan)
+
+    def __getstate__(self):
+        """The configuration and attributes, without the CUDA plan and workspace: these belong to the creating process."""
+        return {k: v for k, v in self.__dict__.items() if k not in ("_plan", "_owner_pid", "_ws")}
+
+    def __setstate__(self, state):
+        """An unpickled extractor is detached: its attributes work, featurising raises RuntimeError (see `_check_owner`).
+        This is what a spawned DataLoader worker receives with the collator or the PCM dataset."""
+        self.__dict__.update(state)
+        self._plan, self._owner_pid, self._ws = None, None, None
+
+    def _check_owner(self):
+        """Featurising needs the plan's CUDA state, which only the process that created the plan has."""
+        if self._owner_pid == os.getpid():
+            return
+        where = ("this is an unpickled copy, which has no CUDA plan" if self._owner_pid is None else
+                 f"this process (pid {os.getpid()}) is not the one that created its CUDA plan (pid {self._owner_pid}), "
+                 "e.g. a forked DataLoader worker")
+        raise RuntimeError(
+            f"B200WhisperFeatureExtractor cannot featurise here: {where}. Compute features in the main process: "
+            "collate PCM with B200DataCollatorSpeechSeq2SeqWithPadding (it defers inside DataLoader workers) and call "
+            "collator.finish(batch), or B200FeaturesTrainerMixin, in the main process; or use dataloader_num_workers=0.")
 
     def __del__(self):
         try:
@@ -285,6 +334,7 @@ class B200WhisperFeatureExtractor:
         """
         import torch
 
+        self._check_owner()
         if not (isinstance(pcm, torch.Tensor) and pcm.is_cuda):
             raise ValueError("extract_device expects a CUDA tensor")
         if pcm.device != self.device:
@@ -337,6 +387,7 @@ class B200WhisperFeatureExtractor:
         mask [B, L // 160]."""
         import torch
 
+        self._check_owner()
         B = lengths.shape[0]
         L = self.n_samples if padded_len is None else int(padded_len)
         mask = torch.empty((B, max(L // self.hop_length, 0)), dtype=torch.int32, device=self.device)
@@ -355,6 +406,7 @@ class B200WhisperFeatureExtractor:
                 and runs `extract_device` on it (wlm_logmel_host has no conditioning)."""
         import torch
 
+        self._check_owner()
         dither, seed = self._conditioning(dither, seed)
         dt, B, ptr_arr, lens_arr, keep = self._host_batch(clips)
         if B == 0:
@@ -426,25 +478,9 @@ class B200WhisperFeatureExtractor:
         """Host clips (`_host_batch`'s pointers and lengths, float32 or int16) -> one pinned buffer on the device, each
         clip trimmed to `max_len` samples and starting on a 16-byte boundary, copied over in one transfer.  Returns the
         device buffer and the int32 lengths and int64 offsets of the ragged batch, on the device."""
-        import torch
-
-        fmt = _pcm_format(dt)
-        esz = np.dtype(dt).itemsize
-        gran = 16 // esz
-        lens = lens_arr.astype(np.int64)
-        if max_len is not None:
-            lens = np.minimum(lens, max_len)
-        starts = (lens + gran - 1) // gran * gran
-        offs = np.concatenate([[0], np.cumsum(starts)[:-1]]).astype(np.int64)
-        host = torch.empty(int(starts.sum()) + gran, dtype=torch.float32 if fmt == N.WLM_PCM_F32 else torch.int16,
-                           pin_memory=True)
-        base = host.data_ptr()
-        for o, n, p in zip(offs.tolist(), lens.tolist(), ptr_arr.tolist()):
-            if n:
-                C.memmove(base + o * esz, p, n * esz)
+        host, offs, lens = pack_pcm(dt, ptr_arr, lens_arr, max_len, pin_memory=True)
         pcm = host.to(self.device, non_blocking=True)     # (the caching host allocator keeps `host` until the copy is done)
-        return (pcm, torch.from_numpy(lens.astype(np.int32)).to(self.device),
-                torch.from_numpy(offs).to(self.device))
+        return pcm, lens.to(self.device), offs.to(self.device)
 
     # -- the reference-facing call (TF-FE:189-342) ---------------------------------------------
     def __call__(self, raw_speech, truncation=True, pad_to_multiple_of=None, return_tensors=None,
@@ -452,6 +488,7 @@ class B200WhisperFeatureExtractor:
                  do_normalize=None, device=None, **kwargs):
         import torch
 
+        self._check_owner()
         if sampling_rate is not None:
             if sampling_rate != self.sampling_rate:                         # TF-FE:261-267
                 raise ValueError(
